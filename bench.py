@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (ours; N>1 under torchrun, one rank per GPU)
   python bench.py --impl reference --gpus N --steps K ...   (the reference's own CPU path, rank 0 only)
+  python bench.py ... --dump-outputs DIR                    (also save the last step's outputs: compare two builds)
 
 A step = one pass of the hot path (aes_to_lwe_trasnciphering, stage 7 of the reference) over one
 batch of synthetic AES blocks: BLOCKS_PER_GPU = 8 blocks per GPU = the block count of the small
@@ -38,6 +39,21 @@ RF_WORDS_PER_WARP_STEP = 10_555  # register source words per warp and step of k_
 NCU_BR_CSV = "r02_blind_rotate_ncu_full.csv"   # ncu --set full of k_blind_rotate_v4 on the 512-ciphertext lane shape the step launches
 METRIC = "AES-128 blocks transciphered/sec"
 UNIT = "blocks/s"
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, name, lwe, limit_bytes):
+    """Write u64 LWE ciphertexts [..., 2049] to out_dir/name.npy as float64 torus values in [-1/2, 1/2) (the top 53 of the
+    64 bits; noise sits at 2^58).  Above limit_bytes, a fixed seeded sample of whole ciphertexts in row order."""
+    import numpy as np
+    a = np.ascontiguousarray(lwe).view(np.int64)
+    budget = limit_bytes - 4096  # room for the .npy header
+    if a.nbytes > budget:
+        rows = a.reshape(-1, a.shape[-1])
+        keep = np.sort(np.random.default_rng(0).choice(rows.shape[0], budget // rows[0].nbytes, replace=False))
+        a = rows[keep]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64) * 2.0 ** -64)
 
 
 def read_ncu_traffic():
@@ -346,7 +362,7 @@ def main_ours(args):
     d_ctr = torch.frombuffer(bytearray(counters), dtype=torch.uint8).cuda()
     d_cct = torch.frombuffer(bytearray(ctr_ct), dtype=torch.uint8).cuda()
     d_cout = torch.empty((nblocks, 128, 2049), dtype=torch.int64, device="cuda")
-    ctr_steps = max(1, min(args.steps, 5))
+    ctr_steps = args.steps
     for _ in range(min(args.warmup, 3)):
         ctx.ctr_transcipher_dev(d_ctr.data_ptr(), d_cct.data_ptr(), nblocks, d_cout.data_ptr())
     barrier()
@@ -370,7 +386,7 @@ def main_ours(args):
     verified = np.packbits(bits).tobytes() == pt
 
     # --- end-to-end leg: host buffers through the C ABI, H2D + D2H inside the timed region ---
-    e2e_steps = max(1, min(args.steps, 5))
+    e2e_steps = args.steps
     for _ in range(min(args.warmup, 2)):
         e2e_call()
     barrier()
@@ -511,6 +527,10 @@ def main_ours(args):
         if cpu is not None:
             line["cpu_baseline"] = cpu
         print(json.dumps(line))
+    if args.dump_outputs:
+        # what the timed device-resident path returned in its last step (d_out is not written after the timed loop)
+        dump_outputs(args.dump_outputs, "transcipher_out" if world == 1 else f"transcipher_out_rank{rank}", out,
+                     DUMP_LIMIT_BYTES // world)
     ctx.close()
     if world > 1:
         dist.destroy_process_group()
@@ -525,7 +545,15 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--blocks", type=int, default=BLOCKS_PER_GPU, help="AES blocks per GPU per step")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's output ciphertexts to DIR/transcipher_out.npy "
+                         "(transcipher_out_rank<r>.npy per rank under torchrun; float64 torus values in [-1/2, 1/2); "
+                         "at most 64 MB in all, a seeded sample of ciphertexts beyond)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         return main_reference(args)
     return main_ours(args)

@@ -42,14 +42,15 @@ def available():
     return os.path.isfile(os.path.join(REF, "harness", "run_submission.py")) and os.path.isfile(os.path.join(REF, "client_key_generation"))
 
 
-def layout(workdir, size, servers="ours"):
-    """Create harness/, scripts/, submission/target/release/ under workdir.  servers = "ours" | "reference"."""
+def layout(workdir, size, servers="ours", ref=REF):
+    """Create harness/, scripts/, submission/target/release/ under workdir out of `ref` (a tree shaped like oracle/_ref)
+    and bin/.  servers = "ours" | "reference"."""
     os.makedirs(workdir, exist_ok=True)
     for d in ("harness", "scripts"):
         dst = os.path.join(workdir, d)
         if os.path.exists(dst):
             shutil.rmtree(dst)
-        shutil.copytree(os.path.join(REF, d), dst)
+        shutil.copytree(os.path.join(ref, d), dst)
     rel = os.path.join(workdir, "submission", "target", "release")
     if os.path.exists(rel):
         shutil.rmtree(rel)
@@ -57,7 +58,7 @@ def layout(workdir, size, servers="ours"):
     origin = {}
     for st in STAGES:
         ours = servers == "ours" and (st.startswith("server_encrypted") or (st == "client_encode_encrypt" and size >= 1))
-        src = os.path.join(BIN if ours else REF, st)
+        src = os.path.join(BIN if ours else ref, st)
         if not os.path.isfile(src):
             raise FileNotFoundError(src)
         os.symlink(src, os.path.join(rel, st))  # $ORIGIN of our executables resolves through the link to bin/
@@ -91,6 +92,66 @@ def run(workdir, size, mini_workload=0, seed=None, servers="ours", env_extra=Non
     rj = os.path.join(workdir, "measurements", name, "results.json")
     if os.path.isfile(rj):
         res["results_json"] = json.load(open(rj))
+    if os.path.isfile(timing_file):
+        res["stage_timing"] = [json.loads(l) for l in open(timing_file) if l.strip()]
+    return res
+
+
+VALUES = [8, 64, 512]  # u16 values of the toy / small / medium instance (harness/params.py:39)
+STAGE_LABEL = {"client_key_generation": "FHE Key Generation", "client_encode_encrypt": "AES key encoding and encryption",
+               "server_encrypted_aes_decryption": "Encrypted aes decryption",
+               "server_encrypted_compute": "Encrypted computation of mini workload"}
+
+
+def replay(workdir, size, mini_workload=0, seed=None, timeout=3600):
+    """Where oracle/_ref has no harness copy: the driver of harness/run_submission.py (SURVEY.md 3.1) replayed here with this
+    repository's ten stage executables.  Dataset as harness/generate_dataset.py + aes_keygen_and_encrypt.py make it (random
+    u16 values, AES key sha256("None")[:16], ECB for size 0 and CTR for sizes 1/2), the stages in the harness's order with
+    argv[1] = size in cwd = workdir, then the verifiers' exact list equality against harness/cleartext_impl.py:52-70.
+    Returns the same dict as run()."""
+    import numpy as np
+    sys.path.insert(0, os.path.join(ROOT, "oracle"))
+    import aes_clear
+    name = SIZE_NAME[size]
+    vals = np.random.default_rng(seed).integers(0, 65536, VALUES[size]).tolist()
+    key = aes_clear.harness_aes_key(None)
+    ds = os.path.join(workdir, "datasets", name)
+    os.makedirs(ds)
+    open(os.path.join(ds, "aes_key.hex"), "w").write(key.hex())
+    if size == 0:
+        ct = aes_clear.ecb_encrypt(key, aes_clear.pack_u16_be(vals))
+    else:
+        iv = aes_clear.harness_iv(None)
+        open(os.path.join(ds, "aes_iv.hex"), "w").write(iv.hex())
+        ct = aes_clear.ctr_crypt(key, iv, aes_clear.pack_u16_be(vals))
+    open(os.path.join(ds, "db.hex"), "w").write(ct.hex())
+    env = dict(os.environ)
+    env["CBS_MINI_WORKLOAD"] = str(mini_workload)
+    timing_file = os.path.join(workdir, "stage_timing.jsonl")
+    env.setdefault("CBS_STAGE_TIMING", timing_file)
+    per_stage, out, rc = {}, [], 0
+    t0 = time.time()
+    for st in STAGES:
+        t = time.time()
+        p = subprocess.run([os.path.join(BIN, st), str(size)], cwd=workdir, env=env, stdout=subprocess.PIPE,
+                           stderr=subprocess.STDOUT, text=True, timeout=timeout)
+        per_stage[STAGE_LABEL.get(st, st)] = "%.4fs" % (time.time() - t)
+        out.append(p.stdout)
+        if p.returncode != 0:
+            rc = p.returncode
+            break
+    wall = time.time() - t0
+
+    def ints(f):
+        path = os.path.join(workdir, "io", name, f)
+        return [int(x) for x in open(path).read().split()] if os.path.isfile(path) else None
+
+    h = len(vals) // 2
+    want = sum((x * y) % 65536 for x, y in zip(vals[:h], vals[h:])) % 65536 if mini_workload else max(vals)
+    res = {"size": size, "instance": name, "mini_workload": mini_workload, "servers": "ours", "rc": rc, "wall_s": round(wall, 3),
+           "stage_origin": {st: "ours" for st in STAGES}, "stdout": "".join(out), "values": vals,
+           "pass_aes": rc == 0 and ints("result_aes.txt") == vals, "pass_result": rc == 0 and ints("result.txt") == [want],
+           "results_json": {"per_stage": per_stage, "total_latency_s": round(wall, 4)}}
     if os.path.isfile(timing_file):
         res["stage_timing"] = [json.loads(l) for l in open(timing_file) if l.strip()]
     return res

@@ -29,22 +29,39 @@ def test_pyaes_shim_matches_fips197_and_oracle_aes():
         assert pyaes.AESModeOfOperationCTR(key, counter=pyaes.Counter(int.from_bytes(iv, "big"))).decrypt(out) == data
 
 
-@pytest.mark.skipif(not harness_run.available(), reason="oracle/_ref has no harness copy")
+HARNESS_FILES = ("run_submission.py", "utils.py", "params.py", "cleartext_impl.py", "verify_result.py")
+
+
+def _stand_in_reference(d):
+    """A tree shaped like oracle/_ref (the reference's harness, scripts and client executables, which this repository does
+    not contain) with placeholder files: enough to check what layout() builds where oracle/_ref is absent."""
+    (d / "harness").mkdir(parents=True)
+    (d / "scripts").mkdir()
+    for f in HARNESS_FILES:
+        (d / "harness" / f).write_text(f"# stand-in for the reference's harness/{f}\n")
+    for st in harness_run.STAGES:
+        (d / st).write_text("#!/bin/sh\nexit 0\n")
+        (d / st).chmod(0o755)
+    return str(d)
+
+
 @pytest.mark.parametrize("size", [0, 1])
 def test_layout_is_what_run_submission_expects(tmp_path, size):
-    origin = harness_run.layout(str(tmp_path), size)
-    rel = tmp_path / "submission" / "target" / "release"
+    ref = harness_run.REF if harness_run.available() else _stand_in_reference(tmp_path / "ref")
+    work = tmp_path / "work"
+    origin = harness_run.layout(str(work), size, ref=ref)
+    rel = work / "submission" / "target" / "release"
     for st in harness_run.STAGES:
         assert os.access(rel / st, os.X_OK), st
+        src = os.path.join(harness_run.BIN if origin[st] == "ours" else ref, st)
+        assert os.path.realpath(rel / st) == os.path.realpath(src), st
     assert origin["server_encrypted_aes_decryption"] == origin["server_encrypted_compute"] == "ours"
     assert origin["client_encode_encrypt"] == ("ours" if size >= 1 else "reference")
-    for f in ("run_submission.py", "utils.py", "params.py", "cleartext_impl.py", "verify_result.py"):
-        assert (tmp_path / "harness" / f).is_file()
-    assert (tmp_path / "scripts").is_dir()
-    # the harness copy is the reference's, byte for byte, wherever the reference is present
-    ref = "/root/reference/harness/run_submission.py"
-    if os.path.exists(ref):
-        assert open(ref, "rb").read() == (tmp_path / "harness" / "run_submission.py").read_bytes()
+    for f in HARNESS_FILES:
+        assert (work / "harness" / f).is_file()
+    assert (work / "scripts").is_dir()
+    # the harness is copied byte for byte
+    assert open(os.path.join(ref, "harness", "run_submission.py"), "rb").read() == (work / "harness" / "run_submission.py").read_bytes()
 
 
 @pytest.mark.parametrize("nblocks,cvd,gpus,want", [(1, "3,5,6", None, "3"), (64, "0,1,2,3,4,5,6,7", None, "0"),

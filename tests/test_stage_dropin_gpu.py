@@ -1,7 +1,7 @@
 """Drop-in test of the stage executables: the REFERENCE's own prebuilt client binaries (oracle/_ref,
-unmodified) generate the keys and decrypt the results; OUR server_encrypted_aes_decryption and
-server_encrypted_compute run in between, over the same io/ + datasets/ file contract that
-harness/run_submission.py drives (SURVEY.md 8(b)(1))."""
+unmodified; this repository's C++ twins where oracle/_ref is absent) generate the keys and decrypt the results; OUR
+server_encrypted_aes_decryption and server_encrypted_compute run in between, over the same io/ + datasets/ file contract
+that harness/run_submission.py drives (SURVEY.md 8(b)(1))."""
 import os
 import subprocess
 
@@ -14,13 +14,15 @@ pytestmark = pytest.mark.gpu
 
 REF = os.path.join(ROOT, "oracle", "_ref")
 BIN = os.path.join(ROOT, "temp_fhe_transciphering_b200", "bin")
+# key generation and decryption clients: the reference's own where oracle/_ref has them, else this repository's C++ twins
+# (same files, byte for byte: tests/test_oracle_cpu.py::test_client_stage_tools_match_reference_clients)
+CLIENTS = REF if os.path.exists(os.path.join(REF, "client_key_generation")) else BIN
 
 
 def _run(exe, cwd, *args):
     subprocess.run([exe, "0", *args], cwd=cwd, check=True, stdout=subprocess.DEVNULL, timeout=900)
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF, "client_key_generation")), reason="oracle/_ref not built")
 @pytest.mark.parametrize("nvals", [8, 24])
 def test_reference_clients_around_our_servers(tmp_path, nvals):
     retry_on_noise(lambda k: _reference_clients_around_our_servers(tmp_path / f"try{k}", nvals))
@@ -35,14 +37,14 @@ def _reference_clients_around_our_servers(d, nvals):
     os.makedirs(d / "datasets" / "toy")
     (d / "datasets" / "toy" / "aes_key.hex").write_text(key.hex())
     (d / "datasets" / "toy" / "db.hex").write_text(ct.hex())
-    _run(os.path.join(REF, "client_key_generation"), d)          # reference, unseeded
-    _run(os.path.join(REF, "client_encode_encrypt"), d)          # reference
+    _run(os.path.join(CLIENTS, "client_key_generation"), d)      # unseeded
+    _run(os.path.join(CLIENTS, "client_encode_encrypt"), d)
     _run(os.path.join(BIN, "server_encrypted_aes_decryption"), d)  # ours (all blocks, all visible GPUs)
     _run(os.path.join(BIN, "server_encrypted_compute"), d)         # ours
-    _run(os.path.join(REF, "client_decrypt_decode_aes_decryption"), d)
-    _run(os.path.join(REF, "client_postprocess_aes_decryption"), d)
-    _run(os.path.join(REF, "client_decrypt_decode"), d)
-    _run(os.path.join(REF, "client_postprocess"), d)
+    _run(os.path.join(CLIENTS, "client_decrypt_decode_aes_decryption"), d)
+    _run(os.path.join(CLIENTS, "client_postprocess_aes_decryption"), d)
+    _run(os.path.join(CLIENTS, "client_decrypt_decode"), d)
+    _run(os.path.join(CLIENTS, "client_postprocess"), d)
     got = [int(x) for x in (d / "io" / "toy" / "result_aes.txt").read_text().split()]
     got_max = [int(x) for x in (d / "io" / "toy" / "result.txt").read_text().split()]
     check_blocks(got, vals)
@@ -52,14 +54,13 @@ def _reference_clients_around_our_servers(d, nvals):
     assert os.path.getsize(d / "io" / "toy" / "ciphertexts_download" / "result.bin") == 262_312
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF, "client_key_generation")), reason="oracle/_ref not built")
 @pytest.mark.parametrize("size,nvals", [(1, 64), pytest.param(2, 8192, marks=pytest.mark.slow)])
 def test_ctr_instances_and_both_mini_workloads(tmp_path, size, nvals):
     retry_on_noise(lambda k: _ctr_instances_and_both_mini_workloads(tmp_path / f"try{k}", size, nvals))
 
 
 def _ctr_instances_and_both_mini_workloads(d, size, nvals):
-    """CTR-mode instances through the stage executables: reference key generation and decryption clients, OUR
+    """CTR-mode instances through the stage executables: key generation and decryption clients from CLIENTS, OUR
     client_encode_encrypt (forward keys; the reference's only emits ECB-decryption keys) and OUR two servers.
       * size 1, 64 values = the harness's "small" instance (8 blocks; harness/aes_keygen_and_encrypt.py:49-55);
       * size 2 directory with 8192 values = BASELINE.json config 5: "full-round AES-128 (10 rounds, 1024 blocks) with
@@ -85,14 +86,14 @@ def _ctr_instances_and_both_mini_workloads(d, size, nvals):
         subprocess.run([exe, str(size), *args], cwd=d, check=True, stdout=subprocess.DEVNULL, timeout=1800)
         wall[os.path.basename(exe) + "".join("_" + a for a in args)] = round(time.time() - t0, 3)
 
-    run(os.path.join(REF, "client_key_generation"))
+    run(os.path.join(CLIENTS, "client_key_generation"))
     run(os.path.join(BIN, "client_encode_encrypt"))
     run(os.path.join(BIN, "server_encrypted_aes_decryption"))
     run(os.path.join(BIN, "server_encrypted_compute"))
-    run(os.path.join(REF, "client_decrypt_decode_aes_decryption"))
-    run(os.path.join(REF, "client_postprocess_aes_decryption"))
-    run(os.path.join(REF, "client_decrypt_decode"))
-    run(os.path.join(REF, "client_postprocess"))
+    run(os.path.join(CLIENTS, "client_decrypt_decode_aes_decryption"))
+    run(os.path.join(CLIENTS, "client_postprocess_aes_decryption"))
+    run(os.path.join(CLIENTS, "client_decrypt_decode"))
+    run(os.path.join(CLIENTS, "client_postprocess"))
     got = [int(x) for x in (d / "io" / name / "result_aes.txt").read_text().split()]
     got_max = [int(x) for x in (d / "io" / name / "result.txt").read_text().split()]
     # AES_TIGHT leaves a measurable failure probability per block: the state bits entering a round are sums of four LUT
@@ -112,8 +113,8 @@ def _ctr_instances_and_both_mini_workloads(d, size, nvals):
     # the other mini-workload on the same transciphered values (second argument = harness --mini_workload 1), sharded
     # over the visible GPUs when there are several, combined with cbs_sum_u16
     run(os.path.join(BIN, "server_encrypted_compute"), "1")
-    run(os.path.join(REF, "client_decrypt_decode"))
-    run(os.path.join(REF, "client_postprocess"))
+    run(os.path.join(CLIENTS, "client_decrypt_decode"))
+    run(os.path.join(CLIENTS, "client_postprocess"))
     h = nvals // 2
     want = sum((x * y) % 65536 for x, y in zip(got[:h], got[h:])) % 65536
     assert [int(x) for x in (d / "io" / name / "result.txt").read_text().split()] == [want]
