@@ -181,7 +181,7 @@ int cbs_aes128_transcipher(cbs_ctx *ctx, const uint8_t *ct, int nblocks, const u
                            const uint64_t *k0, uint64_t *out);
 /* CTR-mode transciphering (forward AES on the public counter blocks IV+i, 128-bit big-endian counter as
  * pyaes.Counter; he_sub_bytes_8_to_24 / he_shift_rows / he_mix_columns_precomp, cbs_lib/src/aes_he.rs:285-474),
- * then XOR with the public AES-CTR ciphertext bits.  out as cbs_aes128_transcipher. */
+ * then XOR with the public AES-CTR ciphertext bits.  out, and the overlapped key upload, as cbs_aes128_transcipher. */
 int cbs_aes128_ctr_transcipher(cbs_ctx *ctx, const uint8_t *ct, int nblocks, const uint8_t iv[16], const uint64_t *kf_first,
                                const uint64_t *kf_mid, const uint64_t *kf_last, uint64_t *out);
 /* stage 8, src/bin/server_encrypted_compute.rs:99-359: encrypted max of nvals 16-bit values

@@ -21,6 +21,10 @@
 #include "host/ip_plan.h"
 
 using namespace cbs;
+using cbs_host::AesDir;
+using cbs_host::kAesDirs;
+using cbs_host::kAesFwd;
+using cbs_host::kAesInv;
 using cbs_host::set_error;
 
 namespace {
@@ -39,17 +43,15 @@ struct cbs_ctx {
     uint64_t launches = 0;
     DeviceKeys K{};
     std::vector<void *> key_allocs;
-    uint64_t *d_k10_9 = nullptr, *d_k8_1 = nullptr, *d_k0 = nullptr;
-    bool have_trans_key = false;
-    uint64_t *d_kf_first = nullptr, *d_kf_mid = nullptr, *d_kf_last = nullptr;
-    bool have_fwd_key = false;
-    // every mask word of the round 8..1 / round 0 LUTs is zero (always true for AllRdKeys written by the
-    // reference, src/data_struct.rs:145-151,258-263); checked at upload, enables the first-CMux shortcut
-    int inv_luts_trivial = 0, fwd_luts_trivial = 0;  // host-side promise (unused since the device flags below)
-    int *d_masks_nonzero = nullptr;                  // [0] round 8..0 LUTs, [1] forward (CTR) LUTs: 0 = every mask word is zero
-    int jobs24_nblocks[5] = {-1, -1, -1, -1, -1};
+    // transciphering keys per direction (AesDir): device LUTs of the first, middle and last rounds (host_common.h kAesDirs)
+    struct AesKeys {
+        uint64_t *first = nullptr, *mid = nullptr, *last = nullptr;
+        bool uploaded = false;
+    } aes[2];
+    // [dir]: 0 = every mask word of the direction's middle and last LUTs is zero (always true for AllRdKeys written by the
+    // reference, src/data_struct.rs:145-151,258-263); set by k_masks_nonzero at upload, enables the first-CMux shortcut
+    int *d_masks_nonzero = nullptr;
     std::map<std::string, DevBuf> ws;
-    // cached LUT job tables, keyed by block count
     int chunk_blocks = 64;
     // Lanes: a chunk is processed as up to kMaxLanes block-aligned parts on separate side streams so that
     // the second (partial) wave of one part's blind rotation overlaps the trace / scheme switch / LUT
@@ -59,9 +61,10 @@ struct cbs_ctx {
     int lane = -1;
     cudaStream_t side[kMaxLanes] = {nullptr, nullptr, nullptr, nullptr};
     cudaEvent_t ev_fork = nullptr, ev_join[kMaxLanes] = {nullptr, nullptr, nullptr, nullptr};
-    int jobs_nblocks[kMaxLanes + 1] = {-1, -1, -1, -1, -1};
-    // end-to-end calls upload the round 8..0 LUTs (26 MB) on a copy stream while the first rounds and the first blind
-    // rotation already run; the first LUT launch of every lane waits for ev_keys
+    // block count the LUT job tables of [lane + 1][nmult] were built for (0: none)
+    int jobs_nblocks[kMaxLanes + 1][5] = {};
+    // end-to-end calls upload the middle and last LUTs (ECB 26 MB) on a copy stream while the first rounds and the first
+    // blind rotation already run; the first middle-round LUT launch of every lane waits for ev_keys
     cudaStream_t copy_stream = nullptr;
     cudaEvent_t ev_keys = nullptr, ev_copy_after = nullptr;
     bool keys_in_flight = false;
@@ -208,125 +211,88 @@ int dev_circuit_bootstrap(cbs_ctx *ctx, const uint64_t *d_in, uint64_t *d_ggsw_s
     return check_launch("k_scheme_switch");
 }
 
-int ensure_job_tables(cbs_ctx *ctx, int nb, int **lut32, int **out32, int **lut8, int **out8)
+// 8-bit LUT ladders (a7); masks_nonzero = the device flag of the LUTs' direction, nullptr if not known
+int dev_lut8(cbs_ctx *ctx, const double *ggsw_f, const uint64_t *luts, const int *lut_index, const int *out_index, uint64_t *out,
+             int njobs, int accs_per_byte, const int *masks_nonzero)
 {
-    const int j32 = nb * 16 * 8, j8 = nb * 16 * 2;
-    TRY(ws_typed(ctx, "job_lut32", (size_t)j32, lut32));
-    TRY(ws_typed(ctx, "job_out32", (size_t)j32, out32));
-    TRY(ws_typed(ctx, "job_lut8", (size_t)j8, lut8));
-    TRY(ws_typed(ctx, "job_out8", (size_t)j8, out8));
-    if (ctx->jobs_nblocks[ctx->lane + 1] == nb) return CBS_OK;
-    std::vector<int> l32(j32), o32(j32), l8(j8), o8(j8);
+    if (launch_lut8(ctx->K, ggsw_f, luts, lut_index, out_index, out, njobs, accs_per_byte, masks_nonzero, S(ctx))) {
+        set_error("k_lut8_v2: " + std::to_string(njobs) + " jobs are not a whole number of bytes of " + std::to_string(accs_per_byte) +
+                  " accumulators");
+        return CBS_ERR_ARG;
+    }
+    ctx->launches++;
+    return check_launch("k_lut8_v2");
+}
+
+// LUT job tables of nb blocks with nmult LUTs per byte (4: inverse middle rounds, 3: forward middle rounds, 1: last round):
+// job (blk, byte, m, a) runs accumulator a of LUT (m, byte) and writes its 4 LWE to row (m, blk, byte*8 + 4a) of the
+// [nmult][nb][128] state.  Cached per lane and nmult, so repeated calls at one block count rebuild nothing.
+int job_tables(cbs_ctx *ctx, int nb, int nmult, int **lut, int **out)
+{
+    const int n = nb * 16 * nmult * 2;
+    const std::string jobs = std::to_string(nmult * 8);
+    TRY(ws_typed(ctx, ("job_lut" + jobs).c_str(), (size_t)n, lut));
+    TRY(ws_typed(ctx, ("job_out" + jobs).c_str(), (size_t)n, out));
+    int &built = ctx->jobs_nblocks[ctx->lane + 1][nmult];
+    if (built == nb) return CBS_OK;
+    std::vector<int> l(n), o(n);
     for (int blk = 0; blk < nb; blk++)
-        for (int byte = 0; byte < 16; byte++) {
-            for (int m = 0; m < 4; m++)
+        for (int byte = 0; byte < 16; byte++)
+            for (int m = 0; m < nmult; m++)
                 for (int a = 0; a < 2; a++) {
-                    const int job = (blk * 16 + byte) * 8 + m * 2 + a;
-                    l32[job] = (m * 16 + byte) * 2 + a;
-                    o32[job] = (m * nb + blk) * 128 + byte * 8 + 4 * a;
+                    const int job = ((blk * 16 + byte) * nmult + m) * 2 + a;
+                    l[job] = (m * 16 + byte) * 2 + a;
+                    o[job] = (m * nb + blk) * 128 + byte * 8 + 4 * a;
                 }
-            for (int a = 0; a < 2; a++) {
-                const int job = (blk * 16 + byte) * 2 + a;
-                l8[job] = byte * 2 + a;
-                o8[job] = blk * 128 + byte * 8 + 4 * a;
-            }
-        }
-    CUDA_TRY(cudaMemcpyAsync(*lut32, l32.data(), sizeof(int) * j32, cudaMemcpyHostToDevice, S(ctx)));
-    CUDA_TRY(cudaMemcpyAsync(*out32, o32.data(), sizeof(int) * j32, cudaMemcpyHostToDevice, S(ctx)));
-    CUDA_TRY(cudaMemcpyAsync(*lut8, l8.data(), sizeof(int) * j8, cudaMemcpyHostToDevice, S(ctx)));
-    CUDA_TRY(cudaMemcpyAsync(*out8, o8.data(), sizeof(int) * j8, cudaMemcpyHostToDevice, S(ctx)));
+    CUDA_TRY(cudaMemcpyAsync(*lut, l.data(), sizeof(int) * n, cudaMemcpyHostToDevice, S(ctx)));
+    CUDA_TRY(cudaMemcpyAsync(*out, o.data(), sizeof(int) * n, cudaMemcpyHostToDevice, S(ctx)));
     CUDA_TRY(cudaStreamSynchronize(S(ctx)));  // host vectors go out of scope
-    ctx->jobs_nblocks[ctx->lane + 1] = nb;
+    built = nb;
     return CBS_OK;
 }
 
-// aes_to_lwe_trasnciphering for one chunk of nb blocks
-int dev_transcipher_part(cbs_ctx *ctx, const uint8_t *d_ct, int nb, uint64_t *d_out)
+// One chunk of nb blocks through the AES rounds of direction `dir`.  Inverse (ECB, aes_to_lwe_trasnciphering,
+// server_encrypted_aes_decryption.rs:89-189): rounds 10 + 9 on the public ciphertext blocks d_in, rounds 8..1, the last
+// round and the per-byte bit reversal.  Forward (CTR, aes_he.rs:285-474): round 1 on the public counter blocks d_in,
+// rounds 2..9, the last round, then XOR with the public CTR ciphertext d_ct.
+int dev_aes_part(cbs_ctx *ctx, AesDir dir, const uint8_t *d_in, const uint8_t *d_ct, int nb, uint64_t *d_out)
 {
-    const int B = nb * 128;
-    uint64_t *d_t4, *d_st, *d_ks;
+    const int nmult = kAesDirs[dir].nmult, B = nb * 128;
+    const bool inv = dir == kAesInv;
+    const cbs_ctx::AesKeys &key = ctx->aes[dir];
+    const int *masks_nonzero = ctx->d_masks_nonzero + dir;
+    uint64_t *d_t, *d_st, *d_ks;
     double *d_ggsw_f;
-    int *lut32, *out32, *lut8, *out8;
-    TRY(ws_typed(ctx, "t4", (size_t)4 * B * kLweBig, &d_t4));
+    int *lut_m, *out_m, *lut_1, *out_1;
+    TRY(ws_typed(ctx, "t4", (size_t)4 * B * kLweBig, &d_t));
     TRY(ws_typed(ctx, "st", (size_t)B * kLweBig, &d_st));
     TRY(ws_typed(ctx, "ks", (size_t)B * kLweSmall, &d_ks));
     TRY(ws_typed(ctx, "ggsw_f", (size_t)B * kGgswWords, &d_ggsw_f));
-    TRY(ensure_job_tables(ctx, nb, &lut32, &out32, &lut8, &out8));
-    // rounds 10 + 9 (server_encrypted_aes_decryption.rs:89-128)
-    launch_known_rotate(d_ct, ctx->d_k10_9, d_t4, nb, 4, 1, S(ctx));
-    launch_inv_linear(d_t4, d_st, nb, S(ctx));
+    TRY(job_tables(ctx, nb, nmult, &lut_m, &out_m));
+    TRY(job_tables(ctx, nb, 1, &lut_1, &out_1));
+    auto linear = [&]() { inv ? launch_inv_linear(d_t, d_st, nb, S(ctx)) : launch_fwd_linear(d_t, d_st, nb, S(ctx)); };
+    // first round(s): the input block is public, so the keyed LUTs are "rotated" by sample extraction
+    launch_known_rotate(d_in, key.first, d_t, nb, nmult, inv, S(ctx));
+    linear();
     ctx->launches += 2;
     TRY(check_launch("first rounds"));
-    // rounds 8..1 (:130-163)
-    for (int round = 8; round >= 1; round--) {
+    for (int i = 0; i < 8; i++) {
         TRY(dev_keyswitch(ctx, d_st, d_ks, B));
         TRY(dev_circuit_bootstrap(ctx, d_ks, nullptr, d_ggsw_f, B));
-        const uint64_t *luts = ctx->d_k8_1 + (size_t)(round - 1) * 4 * 16 * 2 * kGlweWords;
-        if (ctx->keys_in_flight && round == 8) CUDA_TRY(cudaStreamWaitEvent(S(ctx), ctx->ev_keys, 0));
-        launch_lut8(ctx->K, d_ggsw_f, luts, lut32, out32, d_t4, nb * 16 * 8, 8, ctx->inv_luts_trivial, ctx->d_masks_nonzero, S(ctx));
-        launch_inv_linear(d_t4, d_st, nb, S(ctx));
-        ctx->launches += 2;
+        // middle block r is keyed with round key r + 1: decryption runs the blocks from the last one down
+        const uint64_t *luts = key.mid + (size_t)(inv ? 7 - i : i) * nmult * 16 * 2 * kGlweWords;
+        if (ctx->keys_in_flight && i == 0) CUDA_TRY(cudaStreamWaitEvent(S(ctx), ctx->ev_keys, 0));
+        TRY(dev_lut8(ctx, d_ggsw_f, luts, lut_m, out_m, d_t, nb * 16 * nmult * 2, nmult * 2, masks_nonzero));
+        linear();
+        ctx->launches++;
         TRY(check_launch("round"));
     }
-    // last round (:166-180) + per-byte bit reversal (:182-189)
     TRY(dev_keyswitch(ctx, d_st, d_ks, B));
     TRY(dev_circuit_bootstrap(ctx, d_ks, nullptr, d_ggsw_f, B));
-    launch_lut8(ctx->K, d_ggsw_f, ctx->d_k0, lut8, out8, d_st, nb * 16 * 2, 2, ctx->inv_luts_trivial, ctx->d_masks_nonzero, S(ctx));
-    launch_reverse_bits(d_st, d_out, nb, S(ctx));
-    ctx->launches += 2;
+    TRY(dev_lut8(ctx, d_ggsw_f, key.last, lut_1, out_1, d_st, nb * 16 * 2, 2, masks_nonzero));
+    inv ? launch_reverse_bits(d_st, d_out, nb, S(ctx)) : launch_ctr_finish(d_st, d_ct, d_out, nb, S(ctx));
+    ctx->launches++;
     return check_launch("last round");
-}
-
-// CTR mode: forward AES of the public counter blocks (aes_he.rs:285-474), one chunk of nb blocks
-int dev_ctr_part(cbs_ctx *ctx, const uint8_t *d_ctr, const uint8_t *d_ct, int nb, uint64_t *d_out)
-{
-    const int B = nb * 128;
-    uint64_t *d_t3, *d_st, *d_ks;
-    double *d_ggsw_f;
-    int *lut24, *out24, *lut8, *out8, *dummy_a, *dummy_b;
-    TRY(ws_typed(ctx, "t4", (size_t)4 * B * kLweBig, &d_t3));
-    TRY(ws_typed(ctx, "st", (size_t)B * kLweBig, &d_st));
-    TRY(ws_typed(ctx, "ks", (size_t)B * kLweSmall, &d_ks));
-    TRY(ws_typed(ctx, "ggsw_f", (size_t)B * kGgswWords, &d_ggsw_f));
-    TRY(ensure_job_tables(ctx, nb, &dummy_a, &dummy_b, &lut8, &out8));
-    const int j24 = nb * 16 * 6;
-    TRY(ws_typed(ctx, "job_lut24", (size_t)j24, &lut24));
-    TRY(ws_typed(ctx, "job_out24", (size_t)j24, &out24));
-    if (ctx->jobs24_nblocks[ctx->lane + 1] != nb) {
-        std::vector<int> l(j24), o(j24);
-        for (int blk = 0; blk < nb; blk++)
-            for (int byte = 0; byte < 16; byte++)
-                for (int m = 0; m < 3; m++)
-                    for (int a = 0; a < 2; a++) {
-                        const int job = (blk * 16 + byte) * 6 + m * 2 + a;
-                        l[job] = (m * 16 + byte) * 2 + a;
-                        o[job] = (m * nb + blk) * 128 + byte * 8 + 4 * a;
-                    }
-        CUDA_TRY(cudaMemcpyAsync(lut24, l.data(), sizeof(int) * j24, cudaMemcpyHostToDevice, S(ctx)));
-        CUDA_TRY(cudaMemcpyAsync(out24, o.data(), sizeof(int) * j24, cudaMemcpyHostToDevice, S(ctx)));
-        CUDA_TRY(cudaStreamSynchronize(S(ctx)));
-        ctx->jobs24_nblocks[ctx->lane + 1] = nb;
-    }
-    // round 1: the counter block is public -> keyed LUTs are "rotated" by sample extraction
-    launch_known_rotate(d_ctr, ctx->d_kf_first, d_t3, nb, 3, 0, S(ctx));
-    launch_fwd_linear(d_t3, d_st, nb, S(ctx));
-    ctx->launches += 2;
-    TRY(check_launch("ctr round 1"));
-    for (int round = 2; round <= 9; round++) {
-        TRY(dev_keyswitch(ctx, d_st, d_ks, B));
-        TRY(dev_circuit_bootstrap(ctx, d_ks, nullptr, d_ggsw_f, B));
-        const uint64_t *luts = ctx->d_kf_mid + (size_t)(round - 2) * 3 * 16 * 2 * kGlweWords;
-        launch_lut8(ctx->K, d_ggsw_f, luts, lut24, out24, d_t3, j24, 6, ctx->fwd_luts_trivial, ctx->d_masks_nonzero + 1, S(ctx));
-        launch_fwd_linear(d_t3, d_st, nb, S(ctx));
-        ctx->launches += 2;
-        TRY(check_launch("ctr round"));
-    }
-    TRY(dev_keyswitch(ctx, d_st, d_ks, B));
-    TRY(dev_circuit_bootstrap(ctx, d_ks, nullptr, d_ggsw_f, B));
-    launch_lut8(ctx->K, d_ggsw_f, ctx->d_kf_last, lut8, out8, d_st, nb * 16 * 2, 2, ctx->fwd_luts_trivial, ctx->d_masks_nonzero + 1, S(ctx));
-    launch_ctr_finish(d_st, d_ct, d_out, nb, S(ctx));
-    ctx->launches += 2;
-    return check_launch("ctr last round");
 }
 
 // Run `part(lane_index, first_block, block_count)` over a chunk split into block-aligned lanes on the side
@@ -351,44 +317,89 @@ int run_in_lanes(cbs_ctx *ctx, int nb, Fn part)
     return rc;
 }
 
-int dev_transcipher_chunk(cbs_ctx *ctx, const uint8_t *d_ct, int nb, uint64_t *d_out)
+// nblocks blocks in chunks of chunk_blocks, each split into lanes; d_ct is nullptr for the inverse direction
+int dev_aes(cbs_ctx *ctx, AesDir dir, const uint8_t *d_in, const uint8_t *d_ct, int nblocks, uint64_t *d_out)
 {
-    return run_in_lanes(ctx, nb, [&](int b0, int n) {
-        return dev_transcipher_part(ctx, d_ct + (size_t)b0 * 16, n, d_out + (size_t)b0 * 128 * kLweBig);
-    });
-}
-
-int dev_ctr_chunk(cbs_ctx *ctx, const uint8_t *d_ctr, const uint8_t *d_ct, int nb, uint64_t *d_out)
-{
-    return run_in_lanes(ctx, nb, [&](int b0, int n) {
-        return dev_ctr_part(ctx, d_ctr + (size_t)b0 * 16, d_ct + (size_t)b0 * 16, n, d_out + (size_t)b0 * 128 * kLweBig);
-    });
-}
-
-int dev_ctr(cbs_ctx *ctx, const uint8_t *d_ctr, const uint8_t *d_ct, int nblocks, uint64_t *d_out)
-{
-    if (!ctx->have_fwd_key) {
-        set_error("forward transciphering key not uploaded (cbs_fwd_trans_key_upload)");
+    if (!ctx->aes[dir].uploaded) {
+        set_error(dir == kAesInv ? "transciphering key not uploaded (cbs_trans_key_upload)"
+                                 : "forward transciphering key not uploaded (cbs_fwd_trans_key_upload)");
         return CBS_ERR_ARG;
     }
-    for (int b0 = 0; b0 < nblocks; b0 += ctx->chunk_blocks) {
-        const int nb = std::min(ctx->chunk_blocks, nblocks - b0);
-        TRY(dev_ctr_chunk(ctx, d_ctr + (size_t)b0 * 16, d_ct + (size_t)b0 * 16, nb, d_out + (size_t)b0 * 128 * kLweBig));
+    for (int c0 = 0; c0 < nblocks; c0 += ctx->chunk_blocks) {
+        auto part = [&](int b0, int n) {
+            const size_t b = (size_t)c0 + b0;
+            return dev_aes_part(ctx, dir, d_in + b * 16, d_ct ? d_ct + b * 16 : nullptr, n, d_out + b * 128 * kLweBig);
+        };
+        TRY(run_in_lanes(ctx, std::min(ctx->chunk_blocks, nblocks - c0), part));
     }
     return CBS_OK;
 }
 
-int dev_transcipher(cbs_ctx *ctx, const uint8_t *d_ct, int nblocks, uint64_t *d_out)
+// Uploads direction `dir`'s transciphering key and answers "are its middle and last LUTs trivial?" on the device, right behind
+// the copies (k_masks_nonzero; a host scan of them would sit on the critical path).  overlap = false: all on the compute stream,
+// synchronised before returning, so the caller owns the host buffers again.  overlap = true: the first-round LUTs go on the
+// compute stream; the middle and last LUTs, first read by the ladders of the first middle round (one keyswitch + blind rotation,
+// >= 2.4 ms, into the call), go with the check on the copy stream, and ev_keys marks their end.  The caller then sets
+// keys_in_flight for dev_aes_part and orders the compute stream after ev_keys before it releases the host buffers.
+int aes_key_upload(cbs_ctx *ctx, AesDir dir, const uint64_t *first, const uint64_t *mid, const uint64_t *last, bool overlap)
 {
-    if (!ctx->have_trans_key) {
-        set_error("transciphering key not uploaded (cbs_trans_key_upload)");
-        return CBS_ERR_ARG;
+    const cbs_host::AesDirDesc &d = kAesDirs[dir];
+    cbs_ctx::AesKeys &key = ctx->aes[dir];
+    // each buffer on its own: a failed allocation leaves its pointer null and the next call retries it
+    if (!key.first) CUDA_TRY(cudaMalloc(&key.first, (size_t)d.first_words * 8));
+    if (!key.mid) CUDA_TRY(cudaMalloc(&key.mid, (size_t)d.mid_words * 8));
+    if (!key.last) CUDA_TRY(cudaMalloc(&key.last, (size_t)d.last_words * 8));
+    cudaStream_t cs = ctx->stream;
+    if (overlap) {
+        if (!ctx->copy_stream) {
+            CUDA_TRY(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
+            CUDA_TRY(cudaEventCreateWithFlags(&ctx->ev_keys, cudaEventDisableTiming));
+            CUDA_TRY(cudaEventCreateWithFlags(&ctx->ev_copy_after, cudaEventDisableTiming));
+        }
+        // the copy must not overtake earlier work on the compute stream that may still read the old keys
+        CUDA_TRY(cudaEventRecord(ctx->ev_copy_after, ctx->stream));
+        CUDA_TRY(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_copy_after, 0));
+        cs = ctx->copy_stream;
     }
-    for (int b0 = 0; b0 < nblocks; b0 += ctx->chunk_blocks) {
-        const int nb = std::min(ctx->chunk_blocks, nblocks - b0);
-        TRY(dev_transcipher_chunk(ctx, d_ct + (size_t)b0 * 16, nb, d_out + (size_t)b0 * 128 * kLweBig));
-    }
+    int *flag = ctx->d_masks_nonzero + dir;
+    CUDA_TRY(cudaMemcpyAsync(key.mid, mid, (size_t)d.mid_words * 8, cudaMemcpyHostToDevice, cs));
+    CUDA_TRY(cudaMemcpyAsync(key.last, last, (size_t)d.last_words * 8, cudaMemcpyHostToDevice, cs));
+    CUDA_TRY(cudaMemsetAsync(flag, 0, sizeof(int), cs));
+    launch_masks_nonzero(key.mid, 8 * d.nmult * 16 * 2, flag, cs);
+    launch_masks_nonzero(key.last, 16 * 2, flag, cs);
+    if (overlap) CUDA_TRY(cudaEventRecord(ctx->ev_keys, cs));
+    TRY(upload(ctx, key.first, first, (size_t)d.first_words * 8));
+    if (!overlap) CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    key.uploaded = true;
     return CBS_OK;
+}
+
+// Host-buffer transciphering in direction `dir` with the key upload overlapped.  in = the public blocks of the first round
+// (ECB: the ciphertext; CTR: the counter blocks), ct = the CTR ciphertext (nullptr for ECB).  Synchronous for the caller.
+int aes_transcipher_host(cbs_ctx *ctx, AesDir dir, const uint8_t *in, const uint8_t *ct, int nblocks, const uint64_t *first,
+                         const uint64_t *mid, const uint64_t *last, uint64_t *out)
+{
+    TRY(aes_key_upload(ctx, dir, first, mid, last, true));
+    ctx->keys_in_flight = true;
+    uint64_t *d_out = nullptr;
+    auto run = [&]() {
+        uint8_t *d_in, *d_ct = nullptr;
+        TRY(ws_typed(ctx, ct ? "io_ctr" : "io_ct", (size_t)nblocks * 16, &d_in));
+        if (ct) TRY(ws_typed(ctx, "io_ct", (size_t)nblocks * 16, &d_ct));
+        TRY(ws_typed(ctx, "io_result", (size_t)nblocks * 128 * kLweBig, &d_out));
+        TRY(upload(ctx, d_in, in, (size_t)nblocks * 16));
+        if (ct) TRY(upload(ctx, d_ct, ct, (size_t)nblocks * 16));
+        return dev_aes(ctx, dir, d_in, d_ct, nblocks, d_out);
+    };
+    const int rc = run();
+    // whatever happened, the compute stream is ordered after the key copy before the call returns (host buffers, later calls)
+    cudaStreamWaitEvent(ctx->stream, ctx->ev_keys, 0);
+    ctx->keys_in_flight = false;
+    if (rc != CBS_OK) {
+        cudaStreamSynchronize(ctx->stream);
+        return rc;
+    }
+    return download(ctx, out, d_out, (size_t)nblocks * 128 * kLweBig * 8);
 }
 
 }  // namespace
@@ -584,15 +595,12 @@ void cbs_ctx_destroy(cbs_ctx *ctx)
     for (void *p : ctx->key_allocs) cudaFree(p);
     for (auto &kv : ctx->ws)
         if (kv.second.p) cudaFree(kv.second.p);
-    if (ctx->d_k10_9) cudaFree(ctx->d_k10_9);
-    if (ctx->d_k8_1) cudaFree(ctx->d_k8_1);
-    if (ctx->d_k0) cudaFree(ctx->d_k0);
+    for (const cbs_ctx::AesKeys &key : ctx->aes)
+        for (uint64_t *p : {key.first, key.mid, key.last})
+            if (p) cudaFree(p);
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
     if (ctx->ev_keys) cudaEventDestroy(ctx->ev_keys);
     if (ctx->ev_copy_after) cudaEventDestroy(ctx->ev_copy_after);
-    if (ctx->d_kf_first) cudaFree(ctx->d_kf_first);
-    if (ctx->d_kf_mid) cudaFree(ctx->d_kf_mid);
-    if (ctx->d_kf_last) cudaFree(ctx->d_kf_last);
     for (int l = 0; l < cbs_ctx::kMaxLanes; l++) {
         if (ctx->side[l]) cudaStreamDestroy(ctx->side[l]);
         if (ctx->ev_join[l]) cudaEventDestroy(ctx->ev_join[l]);
@@ -824,9 +832,8 @@ int cbs_lut8_eval(cbs_ctx *ctx, const uint64_t *ggsw_bits, int nbytes, const uin
     TRY(upload(ctx, d_li, li.data(), sizeof(int) * njobs));
     TRY(upload(ctx, d_oi, oi.data(), sizeof(int) * njobs));
     launch_ggsw_to_fourier(ctx->K, d_ggsw, d_ggsw_f, nbits, ctx->stream);
-    launch_lut8(ctx->K, d_ggsw_f, d_luts, d_li, d_oi, d_out, njobs, apb, 0, nullptr, ctx->stream);
-    ctx->launches += 2;
-    TRY(check_launch("k_lut8"));
+    ctx->launches++;
+    TRY(dev_lut8(ctx, d_ggsw_f, d_luts, d_li, d_oi, d_out, njobs, apb, nullptr));
     return download(ctx, out, d_out, (size_t)njobs * 4 * kLweBig * 8);
 }
 
@@ -869,28 +876,14 @@ int cbs_trans_key_upload(cbs_ctx *ctx, const uint64_t *k10_9, const uint64_t *k8
 {
     ENTER(ctx);
     if (!k10_9 || !k8_1 || !k0) return set_error("cbs_trans_key_upload: null argument"), CBS_ERR_ARG;
-    // each buffer on its own: a failed allocation leaves its pointer null and the next call retries it
-    if (!ctx->d_k10_9) CUDA_TRY(cudaMalloc(&ctx->d_k10_9, (size_t)CBS_K10_9_WORDS * 8));
-    if (!ctx->d_k8_1) CUDA_TRY(cudaMalloc(&ctx->d_k8_1, (size_t)CBS_K8_1_WORDS * 8));
-    if (!ctx->d_k0) CUDA_TRY(cudaMalloc(&ctx->d_k0, (size_t)CBS_K0_WORDS * 8));
-    TRY(upload(ctx, ctx->d_k10_9, k10_9, (size_t)CBS_K10_9_WORDS * 8));
-    TRY(upload(ctx, ctx->d_k8_1, k8_1, (size_t)CBS_K8_1_WORDS * 8));
-    TRY(upload(ctx, ctx->d_k0, k0, (size_t)CBS_K0_WORDS * 8));
-    // are the LUT accumulators trivial (zero masks)?  Answered on the device, right behind the copies
-    CUDA_TRY(cudaMemsetAsync(ctx->d_masks_nonzero, 0, sizeof(int), ctx->stream));
-    launch_masks_nonzero(ctx->d_k8_1, 8 * 4 * 16 * 2, ctx->d_masks_nonzero, ctx->stream);
-    launch_masks_nonzero(ctx->d_k0, 16 * 2, ctx->d_masks_nonzero, ctx->stream);
-    ctx->inv_luts_trivial = 0;
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));  // the caller owns the host buffers again
-    ctx->have_trans_key = true;
-    return CBS_OK;
+    return aes_key_upload(ctx, kAesInv, k10_9, k8_1, k0, false);
 }
 
 int cbs_aes128_transcipher_dev(cbs_ctx *ctx, const uint8_t *d_ct, int nblocks, uint64_t *d_out)
 {
     ENTER(ctx);
     if (nblocks <= 0 || !d_ct || !d_out) return set_error("cbs_aes128_transcipher_dev: bad argument"), CBS_ERR_ARG;
-    return dev_transcipher(ctx, d_ct, nblocks, d_out);
+    return dev_aes(ctx, kAesInv, d_ct, nullptr, nblocks, d_out);
 }
 
 int cbs_aes128_transcipher(cbs_ctx *ctx, const uint8_t *ct, int nblocks, const uint64_t *k10_9, const uint64_t *k8_1,
@@ -899,69 +892,21 @@ int cbs_aes128_transcipher(cbs_ctx *ctx, const uint8_t *ct, int nblocks, const u
     ENTER(ctx);
     if (nblocks < 0 || (nblocks && (!ct || !out)) || !k10_9 || !k8_1 || !k0) return set_error("cbs_aes128_transcipher: bad argument"), CBS_ERR_ARG;
     if (!nblocks) return CBS_OK;
-    // keys: rounds 10 + 9 need k10_9 (3 MB, on the compute stream); k8_1 and k0 (26 MB) are first read by the LUT ladders of
-    // round 8, one keyswitch + blind rotation (>= 2.4 ms) into the call, so they travel on the copy stream meanwhile
-    if (!ctx->d_k10_9) CUDA_TRY(cudaMalloc(&ctx->d_k10_9, (size_t)CBS_K10_9_WORDS * 8));
-    if (!ctx->d_k8_1) CUDA_TRY(cudaMalloc(&ctx->d_k8_1, (size_t)CBS_K8_1_WORDS * 8));
-    if (!ctx->d_k0) CUDA_TRY(cudaMalloc(&ctx->d_k0, (size_t)CBS_K0_WORDS * 8));
-    if (!ctx->copy_stream) {
-        CUDA_TRY(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
-        CUDA_TRY(cudaEventCreateWithFlags(&ctx->ev_keys, cudaEventDisableTiming));
-        CUDA_TRY(cudaEventCreateWithFlags(&ctx->ev_copy_after, cudaEventDisableTiming));
-    }
-    // the copy must not overtake earlier work on the compute stream that may still read the old keys
-    CUDA_TRY(cudaEventRecord(ctx->ev_copy_after, ctx->stream));
-    CUDA_TRY(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_copy_after, 0));
-    CUDA_TRY(cudaMemcpyAsync(ctx->d_k8_1, k8_1, (size_t)CBS_K8_1_WORDS * 8, cudaMemcpyHostToDevice, ctx->copy_stream));
-    CUDA_TRY(cudaMemcpyAsync(ctx->d_k0, k0, (size_t)CBS_K0_WORDS * 8, cudaMemcpyHostToDevice, ctx->copy_stream));
-    CUDA_TRY(cudaMemsetAsync(ctx->d_masks_nonzero, 0, sizeof(int), ctx->copy_stream));
-    launch_masks_nonzero(ctx->d_k8_1, 8 * 4 * 16 * 2, ctx->d_masks_nonzero, ctx->copy_stream);
-    launch_masks_nonzero(ctx->d_k0, 16 * 2, ctx->d_masks_nonzero, ctx->copy_stream);
-    CUDA_TRY(cudaEventRecord(ctx->ev_keys, ctx->copy_stream));
-    TRY(upload(ctx, ctx->d_k10_9, k10_9, (size_t)CBS_K10_9_WORDS * 8));
-    uint8_t *d_ct;
-    uint64_t *d_out;
-    TRY(ws_typed(ctx, "io_ct", (size_t)nblocks * 16, &d_ct));
-    TRY(ws_typed(ctx, "io_result", (size_t)nblocks * 128 * kLweBig, &d_out));
-    TRY(upload(ctx, d_ct, ct, (size_t)nblocks * 16));
-    ctx->inv_luts_trivial = 0;
-    ctx->have_trans_key = true;
-    ctx->keys_in_flight = true;
-    int rc = dev_transcipher(ctx, d_ct, nblocks, d_out);
-    // whatever happened, the compute stream is ordered after the key copy before the call returns (host buffers, later calls)
-    cudaStreamWaitEvent(ctx->stream, ctx->ev_keys, 0);
-    ctx->keys_in_flight = false;
-    if (rc != CBS_OK) {
-        cudaStreamSynchronize(ctx->stream);
-        return rc;
-    }
-    return download(ctx, out, d_out, (size_t)nblocks * 128 * kLweBig * 8);
+    return aes_transcipher_host(ctx, kAesInv, ct, nullptr, nblocks, k10_9, k8_1, k0, out);
 }
 
 int cbs_fwd_trans_key_upload(cbs_ctx *ctx, const uint64_t *kf_first, const uint64_t *kf_mid, const uint64_t *kf_last)
 {
     ENTER(ctx);
     if (!kf_first || !kf_mid || !kf_last) return set_error("cbs_fwd_trans_key_upload: null argument"), CBS_ERR_ARG;
-    if (!ctx->d_kf_first) CUDA_TRY(cudaMalloc(&ctx->d_kf_first, (size_t)CBS_KF_FIRST_WORDS * 8));
-    if (!ctx->d_kf_mid) CUDA_TRY(cudaMalloc(&ctx->d_kf_mid, (size_t)CBS_KF_MID_WORDS * 8));
-    if (!ctx->d_kf_last) CUDA_TRY(cudaMalloc(&ctx->d_kf_last, (size_t)CBS_KF_LAST_WORDS * 8));
-    TRY(upload(ctx, ctx->d_kf_first, kf_first, (size_t)CBS_KF_FIRST_WORDS * 8));
-    TRY(upload(ctx, ctx->d_kf_mid, kf_mid, (size_t)CBS_KF_MID_WORDS * 8));
-    TRY(upload(ctx, ctx->d_kf_last, kf_last, (size_t)CBS_KF_LAST_WORDS * 8));
-    CUDA_TRY(cudaMemsetAsync(ctx->d_masks_nonzero + 1, 0, sizeof(int), ctx->stream));
-    launch_masks_nonzero(ctx->d_kf_mid, 8 * 3 * 16 * 2, ctx->d_masks_nonzero + 1, ctx->stream);
-    launch_masks_nonzero(ctx->d_kf_last, 16 * 2, ctx->d_masks_nonzero + 1, ctx->stream);
-    ctx->fwd_luts_trivial = 0;
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-    ctx->have_fwd_key = true;
-    return CBS_OK;
+    return aes_key_upload(ctx, kAesFwd, kf_first, kf_mid, kf_last, false);
 }
 
 int cbs_aes128_ctr_transcipher_dev(cbs_ctx *ctx, const uint8_t *d_ctr, const uint8_t *d_ct, int nblocks, uint64_t *d_out)
 {
     ENTER(ctx);
     if (nblocks <= 0 || !d_ctr || !d_ct || !d_out) return set_error("cbs_aes128_ctr_transcipher_dev: bad argument"), CBS_ERR_ARG;
-    return dev_ctr(ctx, d_ctr, d_ct, nblocks, d_out);
+    return dev_aes(ctx, kAesFwd, d_ctr, d_ct, nblocks, d_out);
 }
 
 int cbs_aes128_ctr_transcipher(cbs_ctx *ctx, const uint8_t *ct, int nblocks, const uint8_t iv[16], const uint64_t *kf_first,
@@ -971,7 +916,6 @@ int cbs_aes128_ctr_transcipher(cbs_ctx *ctx, const uint8_t *ct, int nblocks, con
     if (nblocks < 0 || (nblocks && (!ct || !out)) || !iv || !kf_first || !kf_mid || !kf_last)
         return set_error("cbs_aes128_ctr_transcipher: bad argument"), CBS_ERR_ARG;
     if (!nblocks) return CBS_OK;
-    TRY(cbs_fwd_trans_key_upload(ctx, kf_first, kf_mid, kf_last));
     // counter blocks: 128-bit big-endian IV + block index (pyaes.Counter, harness/aes_keygen_and_encrypt.py:52)
     std::vector<uint8_t> ctr((size_t)nblocks * 16);
     uint8_t cur[16];
@@ -981,16 +925,7 @@ int cbs_aes128_ctr_transcipher(cbs_ctx *ctx, const uint8_t *ct, int nblocks, con
         for (int i = 15; i >= 0; i--)
             if (++cur[i] != 0) break;
     }
-    uint8_t *d_ctr, *d_ct;
-    uint64_t *d_out;
-    TRY(ws_typed(ctx, "io_ctr", (size_t)nblocks * 16, &d_ctr));
-    TRY(ws_typed(ctx, "io_ct", (size_t)nblocks * 16, &d_ct));
-    TRY(ws_typed(ctx, "io_result", (size_t)nblocks * 128 * kLweBig, &d_out));
-    TRY(upload(ctx, d_ctr, ctr.data(), (size_t)nblocks * 16));
-    TRY(upload(ctx, d_ct, ct, (size_t)nblocks * 16));
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));  // `ctr` is a local vector
-    TRY(dev_ctr(ctx, d_ctr, d_ct, nblocks, d_out));
-    return download(ctx, out, d_out, (size_t)nblocks * 128 * kLweBig * 8);
+    return aes_transcipher_host(ctx, kAesFwd, ctr.data(), ct, nblocks, kf_first, kf_mid, kf_last, out);
 }
 
 int cbs_max_u16(cbs_ctx *ctx, const uint64_t *in, int nvals, uint64_t *out)

@@ -1793,7 +1793,7 @@ void launch_glev_to_lwe(const uint64_t *glev, const int *pairs, uint64_t *pool, 
 // ---- LUT ladder v2: GGSW row tiles staged through the same 2-deep TMA ring as the blind rotation --------
 // All groups of a CTA evaluate accumulators of the SAME byte, i.e. against the same 8 GGSW bits, so each
 // (level, row) tile of 3 Fourier polynomials is fetched once per CTA.  `groups` = jobs per CTA must divide
-// accs_per_byte (8 -> 4, 6 -> 3, 2 -> 2).  `trivial` = the LUT accumulators are trivial GLWE (zero mask),
+// accs_per_byte (8 -> 4, 6 -> 3, 2 -> 2).  *masks_nonzero == 0: the LUT accumulators are trivial GLWE (zero mask),
 // as every keyed LUT of rounds 8..1 and 0 is (src/data_struct.rs:145-151,258-263): the first CMux then has
 // zero digits for both mask polynomials and 14 of its 21 forward transforms are skipped.
 constexpr int kLut2GroupSmem = kGlweWords * 8 + 2 * 512 * 16;  // 40 KB
@@ -1804,12 +1804,12 @@ __global__ void __launch_bounds__(64 * kLutGroups, 1) k_lut8_v2(const double *__
                                                                  const int *__restrict__ lut_index,
                                                                  const int *__restrict__ out_index,
                                                                  uint64_t *__restrict__ out, int njobs, int accs_per_byte,
-                                                                 const double *__restrict__ twtab, int groups, int trivial_arg,
+                                                                 const double *__restrict__ twtab, int groups,
                                                                  const int *__restrict__ masks_nonzero)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    // trivial accumulators: promised by the caller, or found by k_masks_nonzero right after the key upload (device flag)
-    const int trivial = trivial_arg || (masks_nonzero != nullptr && *masks_nonzero == 0);
+    // trivial accumulators: found by k_masks_nonzero right after the key upload (device flag)
+    const int trivial = masks_nonzero != nullptr && *masks_nonzero == 0;
     const int gi = threadIdx.x >> 6;
     const int job = (gi < groups) ? blockIdx.x * groups + gi : njobs;
     unsigned char *ring = smem_raw + (size_t)kLutGroups * kLut2GroupSmem;
@@ -1957,11 +1957,12 @@ void launch_masks_nonzero(const uint64_t *luts, int count, int *flag, cudaStream
     k_masks_nonzero<<<count < 592 ? count : 592, 256, 0, s>>>(luts, count, flag);
 }
 
-void launch_lut8(const DeviceKeys &K, const double *ggsw_f, const uint64_t *luts, const int *lut_index,
-                 const int *out_index, uint64_t *out, int njobs, int accs_per_byte, int trivial, const int *masks_nonzero,
-                 cudaStream_t s)
+int launch_lut8(const DeviceKeys &K, const double *ggsw_f, const uint64_t *luts, const int *lut_index,
+                const int *out_index, uint64_t *out, int njobs, int accs_per_byte, const int *masks_nonzero, cudaStream_t s)
 {
-    if (njobs <= 0) return;
+    if (njobs <= 0) return 0;
+    // a ragged tail would read another byte's selectors
+    if (njobs % accs_per_byte != 0) return -1;
     static bool attr_done[64] = {false};
     int attr_dev = 0;
     cudaGetDevice(&attr_dev);
@@ -1977,10 +1978,9 @@ void launch_lut8(const DeviceKeys &K, const double *ggsw_f, const uint64_t *luts
             groups = gsz;
             break;
         }
-    // njobs is a whole number of bytes for every caller (cbs_api.cu); a ragged tail would read another byte's selectors
-    if (njobs % accs_per_byte != 0) return;
     k_lut8_v2<<<njobs / groups, 64 * kLutGroups, kLut2SmemBytes, s>>>(ggsw_f, luts, lut_index, out_index, out, njobs, accs_per_byte, K.tw,
-                                                                      groups, trivial, masks_nonzero);
+                                                                      groups, masks_nonzero);
+    return 0;
 }
 
 // ------------------------------------------------------------------------------------------------

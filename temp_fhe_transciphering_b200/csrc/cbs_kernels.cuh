@@ -61,10 +61,10 @@ void launch_ggsw_to_fourier(const DeviceKeys &K, const uint64_t *ggsw_std, doubl
 
 // a7  8-bit LUT ladders.  job j: GGSW bits ggsw_f[(j / accs_per_byte) * 8 .. +8], accumulator
 //     lut[lut_index[j]] (GLWE), outputs 4 LWE(2048) written to out[out_index[j] + {0,1,2,3}].
-//     trivial = 1 promises that every accumulator is a trivial GLWE (zero mask polynomials).
-void launch_lut8(const DeviceKeys &K, const double *ggsw_f, const uint64_t *luts, const int *lut_index,
-                 const int *out_index, uint64_t *out, int njobs, int accs_per_byte, int trivial, const int *masks_nonzero,
-                 cudaStream_t s);
+//     *masks_nonzero == 0 (launch_masks_nonzero) marks every accumulator as a trivial GLWE (zero mask polynomials);
+//     nullptr = not known.  Returns non-zero, launching nothing, if njobs is not a multiple of accs_per_byte.
+int launch_lut8(const DeviceKeys &K, const double *ggsw_f, const uint64_t *luts, const int *lut_index,
+                const int *out_index, uint64_t *out, int njobs, int accs_per_byte, const int *masks_nonzero, cudaStream_t s);
 // *flag |= 1 if any mask word of the `count` GLWE accumulators at `luts` is non-zero (device-side "are these LUTs trivial?")
 void launch_masks_nonzero(const uint64_t *luts, int count, int *flag, cudaStream_t s);
 

@@ -448,6 +448,126 @@ static void lut_plaintext(uint64_t *pt, const uint8_t table[256], int acc_idx, u
 
 using namespace cbs_host;
 
+// Transciphering key of direction `dir` (host_common.h kAesDirs): the first-round LUTs encrypted, one Rng stream per LUT; the
+// middle and last rounds as trivial GLWE (zero mask, the table in the body), as src/data_struct.rs:140-151,258-263 writes them.
+// Keyed tables: inverse get_10_9_round_lut / get_round_lut / get_0_round_lut (aes_manager.rs:338-432), forward
+// S(x ^ rk0) / S(x ^ rk_i) / the last round (cbs_lib/src/aes_ref.rs:334-380).  Middle block i is keyed with round key i + 1.
+static int aes_key_generate(AesDir dir, const char *fn, const cbs_keyset *ks, const uint8_t aes_key[16], const RngSource &src,
+                            uint64_t *first, uint64_t *mid, uint64_t *last)
+{
+    if (!ks || ks->glwe_sk.empty() || !aes_key || !first || !mid || !last) {
+        set_error(std::string(fn) + ": needs a keyset with the GLWE secret key");
+        return CBS_ERR_ARG;
+    }
+    const AesDirDesc &d = kAesDirs[dir];
+    const bool inv = dir == kAesInv;
+    AesTables aes(aes_key);
+    uint8_t tab[16][256];
+    inv ? aes.lut_10_9(tab) : aes.lut_fwd(0, tab);
+    const uint64_t *S = ks->glwe_sk.data();
+    parallel_for(d.nmult * 16 * 2, [&](int id) {
+        const int a = id & 1, b = (id >> 1) & 15, m = id >> 5;
+        Rng rng(src, d.seed_base + (uint64_t)id);
+        std::vector<uint64_t> pt(1024);
+        lut_plaintext(pt.data(), tab[b], a, d.mults[m]);
+        glwe_encrypt(first + (size_t)id * 3072, pt.data(), S, 2, 1024, kStdGlwe, rng);
+    });
+    memset(mid, 0, sizeof(uint64_t) * d.mid_words);
+    for (int i = 0; i < 8; i++) {
+        inv ? aes.lut_round(i + 1, tab) : aes.lut_fwd(i + 1, tab);
+        for (int m = 0; m < d.nmult; m++)
+            for (int b = 0; b < 16; b++)
+                for (int a = 0; a < 2; a++)
+                    lut_plaintext(mid + ((((size_t)i * d.nmult + m) * 16 + b) * 2 + a) * 3072 + 2048, tab[b], a, d.mults[m]);
+    }
+    memset(last, 0, sizeof(uint64_t) * d.last_words);
+    inv ? aes.lut_round(0, tab) : aes.lut_fwd_last(tab);
+    for (int b = 0; b < 16; b++)
+        for (int a = 0; a < 2; a++) lut_plaintext(last + ((size_t)b * 2 + a) * 3072 + 2048, tab[b], a, 0);
+    return CBS_OK;
+}
+
+static int aes_key_generate_os_entropy(AesDir dir, const char *fn, const cbs_keyset *ks, const uint8_t aes_key[16],
+                                       uint64_t *first, uint64_t *mid, uint64_t *last)
+{
+    RngSource src(0);
+    if (!RngSource::os_entropy(src)) {
+        set_error("getrandom failed");
+        return CBS_ERR_IO;
+    }
+    return aes_key_generate(dir, fn, ks, aes_key, src, first, mid, last);
+}
+
+// The AllRdKeys bincode shape for `nmult` multiples: [nmult] x GlweCiphertextList of the 16 first-round LUT pairs, then
+// Vec of 8 rounds x [nmult] x Vec of 16 [GlweCiphertext; 2], then Vec of 16 [GlweCiphertext; 2].  shape(v) writes or checks
+// one word of the layout, data(p, n) moves the n key words at p (with their length prefix).
+template <typename P, typename Shape, typename Data>
+static void all_rd_keys_walk(int nmult, P first, P mid, P last, Shape shape, Data data)
+{
+    auto modulus = [&]() {  // CiphertextModulus<u64> native: u128 0, then scalar bits 64
+        shape(0);
+        shape(0);
+        shape(64);
+    };
+    for (int m = 0; m < nmult; m++) {
+        shape(16);
+        for (int b = 0; b < 16; b++) {  // GlweCiphertextList { data, glwe_size, poly, modulus }
+            data(first + ((size_t)m * 16 + b) * 2 * 3072, 2 * 3072);
+            shape(3);
+            shape(1024);
+            modulus();
+        }
+    }
+    auto pairs = [&](P base) {
+        shape(16);
+        for (int b = 0; b < 16; b++) {
+            shape(2);
+            for (int a = 0; a < 2; a++) {  // GlweCiphertext { data, poly, modulus }
+                data(base + ((size_t)b * 2 + a) * 3072, 3072);
+                shape(1024);
+                modulus();
+            }
+        }
+    };
+    shape(8);
+    for (int rd = 0; rd < 8; rd++)
+        for (int m = 0; m < nmult; m++) pairs(mid + ((size_t)rd * nmult + m) * 16 * 2 * 3072);
+    pairs(last);
+}
+
+static int aes_key_load(AesDir dir, const char *not_what, const char *path, uint64_t *first, uint64_t *mid, uint64_t *last)
+{
+    Reader r;
+    if (!path || !r.load(path)) {
+        set_error(std::string("cannot read ") + (path ? path : "(null)"));
+        return CBS_ERR_IO;
+    }
+    all_rd_keys_walk(kAesDirs[dir].nmult, first, mid, last, [&](uint64_t v) { r.expect(v); },
+                     [&](uint64_t *p, uint64_t n) { r.vec_into(p, n); });
+    if (!r.done()) {
+        set_error(std::string(path) + ": " + not_what);
+        return CBS_ERR_FORMAT;
+    }
+    return CBS_OK;
+}
+
+static int aes_key_save(AesDir dir, const char *path, const uint64_t *first, const uint64_t *mid, const uint64_t *last)
+{
+    if (!path) return CBS_ERR_ARG;
+    const AesDirDesc &d = kAesDirs[dir];
+    Writer w;
+    w.buf.reserve(((size_t)d.first_words + d.mid_words + d.last_words) * 8 + 65536);
+    all_rd_keys_walk(d.nmult, first, mid, last, [&](uint64_t v) { w.u64(v); }, [&](const uint64_t *p, uint64_t n) { w.vec(p, n); });
+    std::string p(path);
+    size_t slash = p.find_last_of('/');
+    if (slash != std::string::npos) mkdirs(p.substr(0, slash));
+    if (!w.save(p)) {
+        set_error("cannot write " + p);
+        return CBS_ERR_IO;
+    }
+    return CBS_OK;
+}
+
 extern "C" {
 
 const char *cbs_last_error(void) { return g_last_error.c_str(); }
@@ -777,291 +897,49 @@ int cbs_keyset_generate_os_entropy(cbs_keyset **out)
     return keyset_generate_impl(src, out);
 }
 
-static int trans_key_generate_impl(const cbs_keyset *ks, const uint8_t aes_key[16], const RngSource &src, uint64_t *k10_9,
-                                   uint64_t *k8_1, uint64_t *k0)
-{
-    if (!ks || ks->glwe_sk.empty() || !aes_key || !k10_9 || !k8_1 || !k0) {
-        set_error("cbs_trans_key_generate: needs a keyset with the GLWE secret key");
-        return CBS_ERR_ARG;
-    }
-    AesTables aes(aes_key);
-    static const uint8_t mults[4] = {9, 11, 13, 14};  // AllRdKeys tuple order, data_struct.rs:76-81
-    uint8_t tab[16][256];
-    aes.lut_10_9(tab);
-    const uint64_t *S = ks->glwe_sk.data();
-    parallel_for(4 * 16 * 2, [&](int id) {
-        const int a = id & 1, b = (id >> 1) & 15, m = id >> 5;
-        Rng rng(src, 9000 + (uint64_t)id);
-        std::vector<uint64_t> pt(1024);
-        lut_plaintext(pt.data(), tab[b], a, mults[m]);
-        glwe_encrypt(k10_9 + (size_t)id * 3072, pt.data(), S, 2, 1024, kStdGlwe, rng);
-    });
-    memset(k8_1, 0, sizeof(uint64_t) * CBS_K8_1_WORDS);
-    for (int r = 1; r <= 8; r++) {
-        aes.lut_round(r, tab);
-        for (int m = 0; m < 4; m++)
-            for (int b = 0; b < 16; b++)
-                for (int a = 0; a < 2; a++)
-                    lut_plaintext(k8_1 + ((((size_t)(r - 1) * 4 + m) * 16 + b) * 2 + a) * 3072 + 2048, tab[b], a, mults[m]);
-    }
-    memset(k0, 0, sizeof(uint64_t) * CBS_K0_WORDS);
-    aes.lut_round(0, tab);
-    for (int b = 0; b < 16; b++)
-        for (int a = 0; a < 2; a++) lut_plaintext(k0 + ((size_t)b * 2 + a) * 3072 + 2048, tab[b], a, 0);
-    return CBS_OK;
-}
-
 int cbs_trans_key_generate(const cbs_keyset *ks, const uint8_t aes_key[16], uint64_t seed, uint64_t *k10_9,
                            uint64_t *k8_1, uint64_t *k0)
 {
-    return trans_key_generate_impl(ks, aes_key, RngSource(seed), k10_9, k8_1, k0);
+    return aes_key_generate(kAesInv, "cbs_trans_key_generate", ks, aes_key, RngSource(seed), k10_9, k8_1, k0);
 }
 
 int cbs_trans_key_generate_os_entropy(const cbs_keyset *ks, const uint8_t aes_key[16], uint64_t *k10_9, uint64_t *k8_1,
                                       uint64_t *k0)
 {
-    RngSource src(0);
-    if (!RngSource::os_entropy(src)) {
-        set_error("getrandom failed");
-        return CBS_ERR_IO;
-    }
-    return trans_key_generate_impl(ks, aes_key, src, k10_9, k8_1, k0);
+    return aes_key_generate_os_entropy(kAesInv, "cbs_trans_key_generate", ks, aes_key, k10_9, k8_1, k0);
 }
 
 int cbs_trans_key_load(const char *path, uint64_t *k10_9, uint64_t *k8_1, uint64_t *k0)
 {
-    Reader r;
-    if (!path || !r.load(path)) {
-        set_error(std::string("cannot read ") + (path ? path : "(null)"));
-        return CBS_ERR_IO;
-    }
-    for (int m = 0; m < 4; m++) {
-        r.expect(16);
-        for (int b = 0; b < 16; b++) {  // GlweCiphertextList { data, glwe_size, poly, modulus }
-            r.vec_into(k10_9 + ((size_t)m * 16 + b) * 2 * 3072, 2 * 3072);
-            r.expect(3);
-            r.expect(1024);
-            r.modulus();
-        }
-    }
-    r.expect(8);
-    for (int rd = 0; rd < 8; rd++)
-        for (int m = 0; m < 4; m++) {
-            r.expect(16);
-            for (int b = 0; b < 16; b++) {
-                r.expect(2);
-                for (int a = 0; a < 2; a++) {  // GlweCiphertext { data, poly, modulus }
-                    r.vec_into(k8_1 + ((((size_t)rd * 4 + m) * 16 + b) * 2 + a) * 3072, 3072);
-                    r.expect(1024);
-                    r.modulus();
-                }
-            }
-        }
-    r.expect(16);
-    for (int b = 0; b < 16; b++) {
-        r.expect(2);
-        for (int a = 0; a < 2; a++) {
-            r.vec_into(k0 + ((size_t)b * 2 + a) * 3072, 3072);
-            r.expect(1024);
-            r.modulus();
-        }
-    }
-    if (!r.done()) {
-        set_error(std::string(path) + ": not an AllRdKeys file for AES_TIGHT");
-        return CBS_ERR_FORMAT;
-    }
-    return CBS_OK;
+    return aes_key_load(kAesInv, "not an AllRdKeys file for AES_TIGHT", path, k10_9, k8_1, k0);
 }
 
 int cbs_trans_key_save(const char *path, const uint64_t *k10_9, const uint64_t *k8_1, const uint64_t *k0)
 {
-    if (!path) return CBS_ERR_ARG;
-    Writer w;
-    w.buf.reserve(29200000);
-    for (int m = 0; m < 4; m++) {
-        w.u64(16);
-        for (int b = 0; b < 16; b++) {
-            w.vec(k10_9 + ((size_t)m * 16 + b) * 2 * 3072, 2 * 3072);
-            w.u64(3);
-            w.u64(1024);
-            w.modulus();
-        }
-    }
-    w.u64(8);
-    for (int rd = 0; rd < 8; rd++)
-        for (int m = 0; m < 4; m++) {
-            w.u64(16);
-            for (int b = 0; b < 16; b++) {
-                w.u64(2);
-                for (int a = 0; a < 2; a++) {
-                    w.vec(k8_1 + ((((size_t)rd * 4 + m) * 16 + b) * 2 + a) * 3072, 3072);
-                    w.u64(1024);
-                    w.modulus();
-                }
-            }
-        }
-    w.u64(16);
-    for (int b = 0; b < 16; b++) {
-        w.u64(2);
-        for (int a = 0; a < 2; a++) {
-            w.vec(k0 + ((size_t)b * 2 + a) * 3072, 3072);
-            w.u64(1024);
-            w.modulus();
-        }
-    }
-    std::string p(path);
-    size_t slash = p.find_last_of('/');
-    if (slash != std::string::npos) mkdirs(p.substr(0, slash));
-    if (!w.save(p)) {
-        set_error("cannot write " + p);
-        return CBS_ERR_IO;
-    }
-    return CBS_OK;
-}
-
-// ---- forward direction (CTR mode) ----
-static int fwd_trans_key_generate_impl(const cbs_keyset *ks, const uint8_t aes_key[16], const RngSource &src, uint64_t *kf_first,
-                               uint64_t *kf_mid, uint64_t *kf_last)
-{
-    if (!ks || ks->glwe_sk.empty() || !aes_key || !kf_first || !kf_mid || !kf_last) {
-        set_error("cbs_fwd_trans_key_generate: needs a keyset with the GLWE secret key");
-        return CBS_ERR_ARG;
-    }
-    AesTables aes(aes_key);
-    static const uint8_t mults[3] = {1, 2, 3};
-    uint8_t tab[16][256];
-    aes.lut_fwd(0, tab);
-    const uint64_t *S = ks->glwe_sk.data();
-    parallel_for(3 * 16 * 2, [&](int id) {
-        const int a = id & 1, b = (id >> 1) & 15, m = id >> 5;
-        Rng rng(src, 11000 + (uint64_t)id);
-        std::vector<uint64_t> pt(1024);
-        lut_plaintext(pt.data(), tab[b], a, mults[m] == 1 ? 0 : mults[m]);
-        glwe_encrypt(kf_first + (size_t)id * 3072, pt.data(), S, 2, 1024, kStdGlwe, rng);
-    });
-    memset(kf_mid, 0, sizeof(uint64_t) * CBS_KF_MID_WORDS);
-    for (int r = 2; r <= 9; r++) {
-        aes.lut_fwd(r - 1, tab);
-        for (int m = 0; m < 3; m++)
-            for (int b = 0; b < 16; b++)
-                for (int a = 0; a < 2; a++)
-                    lut_plaintext(kf_mid + ((((size_t)(r - 2) * 3 + m) * 16 + b) * 2 + a) * 3072 + 2048, tab[b], a,
-                                  mults[m] == 1 ? 0 : mults[m]);
-    }
-    memset(kf_last, 0, sizeof(uint64_t) * CBS_KF_LAST_WORDS);
-    aes.lut_fwd_last(tab);
-    for (int b = 0; b < 16; b++)
-        for (int a = 0; a < 2; a++) lut_plaintext(kf_last + ((size_t)b * 2 + a) * 3072 + 2048, tab[b], a, 0);
-    return CBS_OK;
+    return aes_key_save(kAesInv, path, k10_9, k8_1, k0);
 }
 
 // Forward keys use the AllRdKeys bincode shape with 3-tuples (x1, x2, x3) and 8 middle rounds.
 int cbs_fwd_trans_key_generate(const cbs_keyset *ks, const uint8_t aes_key[16], uint64_t seed, uint64_t *kf_first,
                                uint64_t *kf_mid, uint64_t *kf_last)
 {
-    return fwd_trans_key_generate_impl(ks, aes_key, RngSource(seed), kf_first, kf_mid, kf_last);
+    return aes_key_generate(kAesFwd, "cbs_fwd_trans_key_generate", ks, aes_key, RngSource(seed), kf_first, kf_mid, kf_last);
 }
 
 int cbs_fwd_trans_key_generate_os_entropy(const cbs_keyset *ks, const uint8_t aes_key[16], uint64_t *kf_first, uint64_t *kf_mid,
                                           uint64_t *kf_last)
 {
-    RngSource src(0);
-    if (!RngSource::os_entropy(src)) {
-        set_error("getrandom failed");
-        return CBS_ERR_IO;
-    }
-    return fwd_trans_key_generate_impl(ks, aes_key, src, kf_first, kf_mid, kf_last);
+    return aes_key_generate_os_entropy(kAesFwd, "cbs_fwd_trans_key_generate", ks, aes_key, kf_first, kf_mid, kf_last);
 }
 
 int cbs_fwd_trans_key_save(const char *path, const uint64_t *kf_first, const uint64_t *kf_mid, const uint64_t *kf_last)
 {
-    if (!path) return CBS_ERR_ARG;
-    Writer w;
-    w.buf.reserve(22000000);
-    for (int m = 0; m < 3; m++) {
-        w.u64(16);
-        for (int b = 0; b < 16; b++) {
-            w.vec(kf_first + ((size_t)m * 16 + b) * 2 * 3072, 2 * 3072);
-            w.u64(3);
-            w.u64(1024);
-            w.modulus();
-        }
-    }
-    w.u64(8);
-    for (int rd = 0; rd < 8; rd++)
-        for (int m = 0; m < 3; m++) {
-            w.u64(16);
-            for (int b = 0; b < 16; b++) {
-                w.u64(2);
-                for (int a = 0; a < 2; a++) {
-                    w.vec(kf_mid + ((((size_t)rd * 3 + m) * 16 + b) * 2 + a) * 3072, 3072);
-                    w.u64(1024);
-                    w.modulus();
-                }
-            }
-        }
-    w.u64(16);
-    for (int b = 0; b < 16; b++) {
-        w.u64(2);
-        for (int a = 0; a < 2; a++) {
-            w.vec(kf_last + ((size_t)b * 2 + a) * 3072, 3072);
-            w.u64(1024);
-            w.modulus();
-        }
-    }
-    std::string p(path);
-    size_t slash = p.find_last_of('/');
-    if (slash != std::string::npos) mkdirs(p.substr(0, slash));
-    if (!w.save(p)) {
-        set_error("cannot write " + p);
-        return CBS_ERR_IO;
-    }
-    return CBS_OK;
+    return aes_key_save(kAesFwd, path, kf_first, kf_mid, kf_last);
 }
 
 int cbs_fwd_trans_key_load(const char *path, uint64_t *kf_first, uint64_t *kf_mid, uint64_t *kf_last)
 {
-    Reader r;
-    if (!path || !r.load(path)) {
-        set_error(std::string("cannot read ") + (path ? path : "(null)"));
-        return CBS_ERR_IO;
-    }
-    for (int m = 0; m < 3; m++) {
-        r.expect(16);
-        for (int b = 0; b < 16; b++) {
-            r.vec_into(kf_first + ((size_t)m * 16 + b) * 2 * 3072, 2 * 3072);
-            r.expect(3);
-            r.expect(1024);
-            r.modulus();
-        }
-    }
-    r.expect(8);
-    for (int rd = 0; rd < 8; rd++)
-        for (int m = 0; m < 3; m++) {
-            r.expect(16);
-            for (int b = 0; b < 16; b++) {
-                r.expect(2);
-                for (int a = 0; a < 2; a++) {
-                    r.vec_into(kf_mid + ((((size_t)rd * 3 + m) * 16 + b) * 2 + a) * 3072, 3072);
-                    r.expect(1024);
-                    r.modulus();
-                }
-            }
-        }
-    r.expect(16);
-    for (int b = 0; b < 16; b++) {
-        r.expect(2);
-        for (int a = 0; a < 2; a++) {
-            r.vec_into(kf_last + ((size_t)b * 2 + a) * 3072, 3072);
-            r.expect(1024);
-            r.modulus();
-        }
-    }
-    if (!r.done()) {
-        set_error(std::string(path) + ": not a forward (CTR) transciphering key for AES_TIGHT");
-        return CBS_ERR_FORMAT;
-    }
-    return CBS_OK;
+    return aes_key_load(kAesFwd, "not a forward (CTR) transciphering key for AES_TIGHT", path, kf_first, kf_mid, kf_last);
 }
 
 int cbs_lwe_list_load(const char *path, uint64_t **data, uint64_t *count, uint64_t *lwe_words)

@@ -374,31 +374,49 @@ def test_golden_pin_b_on_gpu(cbs):
     assert np.abs(err).max() < 2.0 * np.abs(ref_err).max()
 
 
+def _check_non_trivial_luts(keyset, gen, key, run, pt):
+    """Adds a GLWE encryption of zero (difference of two encryptions of the same first-round table, from `gen` with another
+    seed) to one middle-round accumulator of every round of `key`; run(key) must still decrypt to pt."""
+    import ref_io
+    first, mid, last = key
+    other = gen(424242)[0]
+    if (other == first).all():  # same seed as the key: take another one
+        other = gen(424243)[0]
+    zero = (first[0, 0, 0].astype(np.uint64) - other[0, 0, 0].astype(np.uint64))
+    assert zero[:2048].any()
+    mid = mid.copy()
+    with np.errstate(over="ignore"):
+        for r in range(8):
+            mid[r, 0, 0, 0] = mid[r, 0, 0, 0] + zero
+    assert mid[0, 0, 0, 0, :2048].any()
+    got = run((first, mid, last))
+    bits, std, mx = ref_io.noise_stats(got.reshape(-1, 2049), keyset.glwe_sk)
+    assert np.packbits(bits).tobytes() == pt
+    assert std < 58.6 and mx < 61.2, (std, mx)
+    # and back to the trivial LUTs of the key (later tests share the context)
+    got = run(key)
+    bits, _, _ = ref_io.noise_stats(got.reshape(-1, 2049), keyset.glwe_sk)
+    assert np.packbits(bits).tobytes() == pt
+
+
 def test_aes_transcipher_with_non_trivial_luts(ctx, keyset, aes_key, trans_key):
     """The reference always writes the round 8..0 LUTs as trivial GLWE (zero masks, data_struct.rs:145-151) and the ladder
     skips the mask transforms of its first CMux when the device-side check (k_masks_nonzero) says so.  Here one accumulator
     gets a real mask: a GLWE encryption of zero (difference of two encryptions of the same table) is added to it, which
     leaves every decryption unchanged - provided the check notices and the full first CMux runs."""
     import aes_clear
-    import ref_io
-    k10_9, k8_1, k0 = trans_key
-    other = keyset.gen_transciphering_keys(aes_key, 424242)[0]
-    if (other == k10_9).all():  # same seed as the fixture: take another one
-        other = keyset.gen_transciphering_keys(aes_key, 424243)[0]
-    zero = (k10_9[0, 0, 0].astype(np.uint64) - other[0, 0, 0].astype(np.uint64))
-    assert zero[:2048].any()
-    k8_1 = k8_1.copy()
-    with np.errstate(over="ignore"):
-        for r in range(8):
-            k8_1[r, 0, 0, 0] = k8_1[r, 0, 0, 0] + zero
-    assert k8_1[0, 0, 0, 0, :2048].any()
     pt = bytes(np.random.default_rng(11).integers(0, 256, 16, dtype=np.uint8))
     ct = aes_clear.ecb_encrypt(aes_key, pt)
-    got = ctx.aes_to_lwe_transciphering(ct, k10_9, k8_1, k0)
-    bits, std, mx = ref_io.noise_stats(got.reshape(-1, 2049), keyset.glwe_sk)
-    assert np.packbits(bits).tobytes() == pt
-    assert std < 58.6 and mx < 61.2, (std, mx)
-    # and back to the trivial LUTs of the fixture (later tests share the context)
-    got = ctx.aes_to_lwe_transciphering(ct, *trans_key)
-    bits, _, _ = ref_io.noise_stats(got.reshape(-1, 2049), keyset.glwe_sk)
-    assert np.packbits(bits).tobytes() == pt
+    _check_non_trivial_luts(keyset, lambda seed: keyset.gen_transciphering_keys(aes_key, seed), trans_key,
+                            lambda k: ctx.aes_to_lwe_transciphering(ct, *k), pt)
+
+
+def test_aes_ctr_transcipher_with_non_trivial_luts(ctx, keyset, aes_key):
+    """The same for CTR mode, whose forward LUTs have their own device-side mask flag."""
+    import aes_clear
+    pt = bytes(np.random.default_rng(11).integers(0, 256, 16, dtype=np.uint8))
+    iv = bytes(range(16))
+    ct = aes_clear.ctr_crypt(aes_key, iv, pt)
+    _check_non_trivial_luts(keyset, lambda seed: keyset.gen_forward_transciphering_keys(aes_key, seed),
+                            keyset.gen_forward_transciphering_keys(aes_key, 55),
+                            lambda k: ctx.aes_ctr_to_lwe_transciphering(ct, iv, *k), pt)
