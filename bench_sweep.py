@@ -8,6 +8,7 @@ CUDA-event times, max over ranks, and rank 0 prints.
 
   python bench_sweep.py                      # CBS sweep 1..16384 + AES 64/256/1024 blocks
   python bench_sweep.py --cbs-only / --aes-only
+  torchrun --nproc_per_node 8 bench_sweep.py --config5 1024 --config5-dev 1024   # configs[4], host-buffer and HBM-resident
 Each CBS point = LWE keyswitch-free circuit bootstrap (blind rotation -> GLEV extraction + trace ->
 scheme switch to a Fourier GGSW), inputs resident in HBM, CUDA events on the launching stream, 3
 warm-up + 5 timed launches; the first batch sizes are verified by decrypting the GGSW rows.
@@ -33,6 +34,10 @@ def main():
     ap.add_argument("--config5", type=int, nargs="?", const=1024, default=0, metavar="BLOCKS",
                     help="BASELINE.json configs[4] only: BLOCKS (default 1024) AES-128-CTR blocks, then max and inner product "
                          "mod 2^16 over all transciphered u16 values")
+    ap.add_argument("--config5-dev", type=int, nargs="?", const=1024, default=0, metavar="BLOCKS",
+                    help="the same job with every ciphertext kept in HBM: device-resident CTR transciphering per rank, the max "
+                         "on each rank's own values, the inner product after a point-to-point exchange of the rows each rank's "
+                         "pairs need (sharding.max_u16_sharded_dev / inner_product_u16_sharded_dev); combinable with --config5")
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     import numpy as np
@@ -98,6 +103,9 @@ def main():
 
     if args.config5:
         config5(args.config5, ks, ctx, stream, world, rank, local, dist, emit, sync_all, max_over_ranks)
+    if args.config5_dev:
+        config5_dev(args.config5_dev, ks, ctx, world, rank, local, dist, emit, sync_all, max_over_ranks)
+    if args.config5 or args.config5_dev:
         args.aes_only = args.cbs_only = True  # nothing else
         args.aes_blocks = []
     if not args.aes_only:
@@ -258,6 +266,76 @@ def config5(nb, ks, ctx, stream, world, rank, local, dist, emit, sync_all, max_o
               "verified": bool(len(wrong) <= 2 * (1 + nb // 1024) and gmax == max(got) and gip == want_ip),
               "note": "host buffers through the C ABI on every rank; wall clock, max over ranks; mini-workloads are checked against "
                       "the values stage 7 actually produced"})
+
+
+def config5_dev(nb, ks, ctx, world, rank, local, dist, emit, sync_all, max_over_ranks):
+    """configs[4] with every ciphertext kept in HBM: each rank transciphers its blocks with cbs_aes128_ctr_transcipher_dev
+    (counters and ciphertext device-resident, as bench.py's ctr leg), the max reduces each rank's own values and the inner
+    product exchanges only the rows each rank's pairs need (sharding.inner_product_exchange_plan), point to point; the
+    16-ciphertext partials are gathered on the device and rank 0 combines them.  Same timing rule as config5 (wall clock
+    ending in a device synchronise, max over ranks) and the same verification against the values stage 7 decrypted to,
+    done on rank 0 after the timed region."""
+    import numpy as np
+    import torch
+    import aes_clear
+    import ref_io
+    from temp_fhe_transciphering_b200 import sharding
+    key, iv = aes_clear.harness_aes_key(None), aes_clear.harness_iv(None)
+    vals = np.random.default_rng(nb).integers(0, 65536, 8 * nb).tolist()
+    ct = aes_clear.ctr_crypt(key, iv, aes_clear.pack_u16_be(vals))
+    ctx.upload_fwd_trans_key(*ks.gen_forward_transciphering_keys(key, 424242))
+    b0, b1 = sharding.block_range(nb, rank, world)
+    mine = b1 - b0
+    counters = b"".join(((int.from_bytes(iv, "big") + b) % (1 << 128)).to_bytes(16, "big") for b in range(b0, b1))
+    d_ctr = torch.frombuffer(bytearray(counters), dtype=torch.uint8).cuda()
+    d_ct = torch.frombuffer(bytearray(ct[16 * b0:16 * b1]), dtype=torch.uint8).cuda()
+    out = torch.empty((mine, 128, 2049), dtype=torch.int64, device="cuda")
+    if mine:
+        ctx.ctr_transcipher_dev(d_ctr.data_ptr(), d_ct.data_ptr(), 1, out.data_ptr())  # warm-up, as config5: one block
+    sync_all()
+
+    def phase(fn):
+        t0 = time.perf_counter()
+        r = fn()
+        torch.cuda.synchronize()
+        t = max_over_ranks((time.perf_counter() - t0) * 1e3) * 1e-3
+        sync_all()
+        return r, t
+
+    _, t_tr = phase(lambda: ctx.ctr_transcipher_dev(d_ctr.data_ptr(), d_ct.data_ptr(), mine, out.data_ptr()) if mine else None)
+    rows, t_ex = phase(lambda: sharding.exchange_inner_product_rows(out, nb, rank, world, dist))
+    res_max, t_max = phase(lambda: sharding.max_u16_sharded_dev(ctx, out, nb, rank, world, dist))
+    res_ip, t_ip = phase(lambda: sharding.inner_product_u16_sharded_dev(ctx, out, nb, rank, world, dist, rows=rows))
+    del rows
+    # verification, after the timed region: rank 0 collects the stage-7 output and decrypts it
+    sizes = [sharding.block_range(nb, r, world) for r in range(world)]
+    full = out
+    if world > 1:
+        buf = torch.zeros((max(e - b for b, e in sizes), 128, 2049), dtype=torch.int64, device="cuda")
+        buf[:mine] = out
+        parts = [torch.empty_like(buf) for _ in range(world)] if rank == 0 else None
+        dist.gather(buf, parts, dst=0)
+        full = torch.cat([p[: e - b] for p, (b, e) in zip(parts, sizes)]) if rank == 0 else None
+        del buf, parts
+
+    def dec(t):
+        return ref_io.bits_to_u16(ref_io.decode_bit(ref_io.lwe_phase(t.cpu().numpy().view(np.uint64).reshape(-1, 2049), ks.glwe_sk)))
+
+    if rank == 0:
+        nvals = 8 * nb
+        got = dec(full)
+        wrong = sorted({i // 8 for i in range(nvals) if got[i] != vals[i]})
+        gmax, gip = dec(res_max)[0], dec(res_ip)[0]
+        h = nvals // 2
+        want_ip = sum((x * y) % 65536 for x, y in zip(got[:h], got[h:])) % 65536
+        emit({"bench": "config5_dev_ctr_blocks_then_max_and_inner_product", "blocks": nb, "values": nvals, "n_gpus": world,
+              "transcipher_s": t_tr, "blocks_per_s": nb / t_tr, "exchange_s": t_ex, "max_s": t_max, "inner_product_s": t_ip,
+              "total_s": t_tr + t_ex + t_max + t_ip, "blocks_differing_from_cleartext": wrong,
+              "max_verified": bool(gmax == max(got)), "inner_product_verified": bool(gip == want_ip),
+              "verified": bool(len(wrong) <= 2 * (1 + nb // 1024) and gmax == max(got) and gip == want_ip),
+              "note": "ciphertexts stay in HBM: *_dev calls on every rank, point-to-point row exchange for the inner product, "
+                      "device-side gather of the 16-ciphertext partials; wall clock ending in a device synchronise, max over "
+                      "ranks; mini-workloads are checked against the values stage 7 actually produced"})
 
 
 if __name__ == "__main__":

@@ -213,12 +213,30 @@ int cbs_inner_product_plan_check(const uint16_t *vals, int nvals, uint16_t *resu
 
 /* ---------------------------------------------------------------------------------------------
  * Device-resident variants (inputs/outputs already in HBM, asynchronous on the context's stream).
- * Used by bench.py's `value` leg and by callers that keep state on the GPU. */
+ * Used by bench.py's `value` leg and by callers that keep state on the GPU: stage 7 and stage 8 both have one, so
+ * transciphered ciphertexts can go on to the mini-workloads without leaving HBM. */
 int cbs_trans_key_upload(cbs_ctx *ctx, const uint64_t *k10_9, const uint64_t *k8_1, const uint64_t *k0);
 int cbs_aes128_transcipher_dev(cbs_ctx *ctx, const uint8_t *d_ct, int nblocks, uint64_t *d_out);
 int cbs_fwd_trans_key_upload(cbs_ctx *ctx, const uint64_t *kf_first, const uint64_t *kf_mid, const uint64_t *kf_last);
 /* d_ctr = the nblocks counter blocks (16 bytes each), d_ct = the AES-CTR ciphertext bytes */
 int cbs_aes128_ctr_transcipher_dev(cbs_ctx *ctx, const uint8_t *d_ctr, const uint8_t *d_ct, int nblocks, uint64_t *d_out);
+
+/* Stage 8 on device buffers: the same computations and results as cbs_max_u16, cbs_max_u16_lut, cbs_sum_u16 and
+ * cbs_inner_product_u16, bit for bit.
+ *   Layout: d_in [nvals][16] big LWE (MSB first), d_out [16] big LWE.  The transcipher output [nblocks][128] big LWE is
+ *   [8*nblocks][16], so a *_transcipher_dev output buffer can be passed as it is.
+ *   cbs_max_u16_dev picks the ladder or the LUT circuit by the same rule as cbs_max_u16, CBS_MAX_VARIANT included.
+ *   The inner product takes x and y from separate buffers, d_x [npairs][16] and d_y [npairs][16] big LWE, so npairs may be
+ *   odd; cbs_inner_product_u16_dev(ctx, X, X + npairs*16*2049, npairs, out) equals cbs_inner_product_u16(ctx, X, 2*npairs, out).
+ *   Asynchronous: the work is queued on the context's stream (cbs_ctx_set_stream) behind earlier work of the context,
+ *   lanes of a *_transcipher_dev call included, so its output can be passed on without synchronising; the call
+ *   synchronises neither the stream nor the device, and once it returns the queued work reads no host memory.
+ *   Counts <= 0, null pointers and a d_out that overlaps an input range return CBS_ERR_ARG. */
+int cbs_max_u16_dev(cbs_ctx *ctx, const uint64_t *d_in, int nvals, uint64_t *d_out);
+int cbs_max_u16_lut_dev(cbs_ctx *ctx, const uint64_t *d_in, int nvals, uint64_t *d_out);
+int cbs_sum_u16_dev(cbs_ctx *ctx, const uint64_t *d_in, int nvals, uint64_t *d_out);
+int cbs_inner_product_u16_dev(cbs_ctx *ctx, const uint64_t *d_x, const uint64_t *d_y, int npairs, uint64_t *d_out);
+
 int cbs_circuit_bootstrap_dev(cbs_ctx *ctx, const uint64_t *d_in_small, int count);  /* GGSW stays in the workspace */
 int cbs_blind_rotate_dev(cbs_ctx *ctx, const uint64_t *d_in_small, uint64_t *d_acc_out, int count);
 /* measured FP64 FMA throughput of the device (roofline denominator of the FFT kernels) */

@@ -278,6 +278,7 @@ class Context:
         _check(lib().cbs_ctx_create(keyset._h, int(device), ctypes.byref(h)), "cbs_ctx_create")
         self._h = h
         self._keyset = keyset
+        self._stream = None  # the cudaStream_t handle last given to set_stream; None: the context's own stream
 
     def close(self):
         if getattr(self, "_h", None) and _lib is not None:
@@ -293,6 +294,12 @@ class Context:
 
     def set_stream(self, cuda_stream):
         _check(lib().cbs_ctx_set_stream(self._h, ctypes.c_void_p(cuda_stream)), "cbs_ctx_set_stream")
+        self._stream = int(cuda_stream) if cuda_stream else None
+
+    @property
+    def stream(self):
+        """The cudaStream_t handle (an int) the context issues its work on, as given to set_stream; None: its own stream."""
+        return self._stream
 
     def synchronize(self):
         _check(lib().cbs_ctx_synchronize(self._h), "cbs_ctx_synchronize")
@@ -460,6 +467,23 @@ class Context:
     def transcipher_dev(self, d_ct_ptr, nblocks, d_out_ptr):
         _check(lib().cbs_aes128_transcipher_dev(self._h, ctypes.c_void_p(d_ct_ptr), int(nblocks), ctypes.c_void_p(d_out_ptr)),
                "cbs_aes128_transcipher_dev")
+
+    # stage 8 on device buffers: raw device pointers, same results as the host-buffer calls, queued on the context stream
+    def max_u16_dev(self, d_in_ptr, nvals, d_out_ptr):
+        """d_in [nvals][16][2049] -> d_out [16][2049]; ladder or LUT circuit by the rule of max_u16."""
+        _check(lib().cbs_max_u16_dev(self._h, ctypes.c_void_p(d_in_ptr), int(nvals), ctypes.c_void_p(d_out_ptr)), "cbs_max_u16_dev")
+
+    def max_u16_lut_dev(self, d_in_ptr, nvals, d_out_ptr):
+        _check(lib().cbs_max_u16_lut_dev(self._h, ctypes.c_void_p(d_in_ptr), int(nvals), ctypes.c_void_p(d_out_ptr)),
+               "cbs_max_u16_lut_dev")
+
+    def sum_u16_dev(self, d_in_ptr, nvals, d_out_ptr):
+        _check(lib().cbs_sum_u16_dev(self._h, ctypes.c_void_p(d_in_ptr), int(nvals), ctypes.c_void_p(d_out_ptr)), "cbs_sum_u16_dev")
+
+    def inner_product_u16_dev(self, d_x_ptr, d_y_ptr, npairs, d_out_ptr):
+        """d_x, d_y [npairs][16][2049] -> d_out [16][2049] encrypting sum_i (x_i * y_i mod 2^16) mod 2^16."""
+        _check(lib().cbs_inner_product_u16_dev(self._h, ctypes.c_void_p(d_x_ptr), ctypes.c_void_p(d_y_ptr), int(npairs),
+                                               ctypes.c_void_p(d_out_ptr)), "cbs_inner_product_u16_dev")
 
     def circuit_bootstrap_dev(self, d_in_ptr, count):
         _check(lib().cbs_circuit_bootstrap_dev(self._h, ctypes.c_void_p(d_in_ptr), int(count)), "cbs_circuit_bootstrap_dev")

@@ -10,6 +10,7 @@
 #include "fft_tables.h"
 #include "host/host_common.h"
 
+#include <climits>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -33,6 +34,25 @@ struct DevBuf {
     void *p = nullptr;
     size_t bytes = 0;
 };
+
+// A host-planned LUT circuit (host/ip_plan.h) compiled for one value count by lut_plan_get and executed by run_lut_plan:
+// the launch schedule stays on the host, the index tables live on the device.
+struct PlanBatch {
+    int idx_off, m, job_off, njobs, ref_off, nref;
+};
+struct PlanLayer {
+    int pre_off, npre, post_off, npost;
+    std::vector<PlanBatch> batches;
+};
+struct LutPlanExec {
+    int nvals = 0;  // value count the entry was built for (0: none)
+    int nin_bits = 0, pool_size = 0, max_m = 1;
+    std::vector<PlanLayer> layers;
+    int *d_tab = nullptr;  // one allocation holding the tables below, in this order
+    const int *idx = nullptr, *sel = nullptr, *lut = nullptr, *out = nullptr, *add = nullptr, *ref = nullptr;
+    int final_idx = 0;  // offset in idx of the 16 result rows, MSB first
+};
+enum PlanKind { kPlanInnerProduct, kPlanSum, kPlanMax, kNumPlanKinds };
 
 }  // namespace
 
@@ -68,6 +88,12 @@ struct cbs_ctx {
     cudaStream_t copy_stream = nullptr;
     cudaEvent_t ev_keys = nullptr, ev_copy_after = nullptr;
     bool keys_in_flight = false;
+    // stage-8 circuits: one compiled plan per kind (rebuilt when the count changes, so a repeated call uploads nothing),
+    // the trivial LUT accumulators of ip_plan.h's tables (uploaded once), and the ladder max's pair tables, which hold
+    // (2i, 2i+1) for i < ladder_pairs in the "max_a" / "max_b" workspaces
+    LutPlanExec plans[kNumPlanKinds];
+    uint64_t *d_plan_luts = nullptr;
+    int ladder_pairs = 0;
 };
 
 namespace {
@@ -404,8 +430,6 @@ int aes_transcipher_host(cbs_ctx *ctx, AesDir dir, const uint8_t *in, const uint
 
 }  // namespace
 
-static int run_lut_plan(cbs_ctx *ctx, const cbs_host::IpPlan &plan, const uint64_t *in, uint64_t *out);
-
 extern "C" {
 
 int cbs_device_count(int *count)
@@ -595,6 +619,9 @@ void cbs_ctx_destroy(cbs_ctx *ctx)
     for (void *p : ctx->key_allocs) cudaFree(p);
     for (auto &kv : ctx->ws)
         if (kv.second.p) cudaFree(kv.second.p);
+    for (const LutPlanExec &E : ctx->plans)
+        if (E.d_tab) cudaFree(E.d_tab);
+    if (ctx->d_plan_luts) cudaFree(ctx->d_plan_luts);
     for (const cbs_ctx::AesKeys &key : ctx->aes)
         for (uint64_t *p : {key.first, key.mid, key.last})
             if (p) cudaFree(p);
@@ -928,108 +955,68 @@ int cbs_aes128_ctr_transcipher(cbs_ctx *ctx, const uint8_t *ct, int nblocks, con
     return aes_transcipher_host(ctx, kAesFwd, ctr.data(), ct, nblocks, kf_first, kf_mid, kf_last, out);
 }
 
-int cbs_max_u16(cbs_ctx *ctx, const uint64_t *in, int nvals, uint64_t *out)
-{
-    ENTER(ctx);
-    if (nvals <= 0 || !in || !out) return set_error("cbs_max_u16: bad argument"), CBS_ERR_ARG;
-    if (nvals == 1) {
-        memcpy(out, in, (size_t)16 * kLweBig * 8);
-        return CBS_OK;
-    }
-    // up to the reference's own 8 values: its max_of_two CMux ladder; above (where the reference cannot run and the
-    // ladder's data-dependent noise becomes a real failure probability): the LUT circuit.  CBS_MAX_VARIANT=ladder|lut overrides.
-    {
-        const char *e = getenv("CBS_MAX_VARIANT");
-        const bool lut = e ? (strcmp(e, "lut") == 0) : nvals > 8;
-        if (lut) return run_lut_plan(ctx, cbs_host::max_make_plan(nvals), in, out);
-    }
-    // balanced tree: level buffers A (current) and B (next)
-    uint64_t *d_lwe[2], *d_op[2], *d_ks, *d_glev;
-    double *d_ggsw[2];
-    int *d_a, *d_b;
-    const size_t vals_lwe = (size_t)16 * kLweBig, vals_ggsw = (size_t)16 * kGgswWords, vals_op = (size_t)16 * kGlweWords;
-    TRY(ws_typed(ctx, "max_lwe0", (size_t)nvals * vals_lwe, &d_lwe[0]));
-    TRY(ws_typed(ctx, "max_lwe1", (size_t)((nvals + 1) / 2) * vals_lwe, &d_lwe[1]));
-    TRY(ws_typed(ctx, "max_ggsw0", (size_t)nvals * vals_ggsw, &d_ggsw[0]));
-    TRY(ws_typed(ctx, "max_ggsw1", (size_t)((nvals + 1) / 2) * vals_ggsw, &d_ggsw[1]));
-    TRY(ws_typed(ctx, "max_op0", (size_t)nvals * vals_op, &d_op[0]));
-    TRY(ws_typed(ctx, "max_op1", (size_t)((nvals + 1) / 2) * vals_op, &d_op[1]));
-    TRY(ws_typed(ctx, "ks", (size_t)nvals * 16 * kLweSmall, &d_ks));
-    TRY(ws_typed(ctx, "glev", (size_t)nvals * 16 * kGlevWords, &d_glev));  // the circuit bootstrap's own GLEV workspace
-    TRY(ws_typed(ctx, "max_a", (size_t)nvals, &d_a));
-    TRY(ws_typed(ctx, "max_b", (size_t)nvals, &d_b));
-    std::vector<int> ha(nvals / 2), hb(nvals / 2);
-    for (int i = 0; i < nvals / 2; i++) {
-        ha[i] = 2 * i;
-        hb[i] = 2 * i + 1;
-    }
-    TRY(upload(ctx, d_a, ha.data(), sizeof(int) * ha.size()));
-    TRY(upload(ctx, d_b, hb.data(), sizeof(int) * hb.size()));
-    TRY(upload(ctx, d_lwe[0], in, (size_t)nvals * vals_lwe * 8));
-    int cnt = nvals, cur = 0, fresh = nvals;  // `fresh` leading values of the current level still need a CBS
-    while (cnt > 1) {
-        // keyswitch + circuit bootstrap the values produced by the previous level (server_encrypted_compute.rs:213-263,314-342);
-        // the level-1 GLEV of the same bootstrap, doubled, is the refreshed data operand of the ladder
-        TRY(dev_keyswitch(ctx, d_lwe[cur], d_ks, fresh * 16));
-        TRY(dev_circuit_bootstrap(ctx, d_ks, nullptr, d_ggsw[cur], fresh * 16));
-        launch_glev_to_operand(d_glev, d_op[cur], fresh * 16, ctx->stream);
-        ctx->launches++;
-        TRY(check_launch("k_glev_to_operand"));
-        const int npairs = cnt / 2;
-        launch_max_ladder(ctx->K, d_ggsw[cur], d_op[cur], d_a, d_b, d_lwe[cur ^ 1], npairs, ctx->stream);
-        ctx->launches++;
-        TRY(check_launch("k_max_ladder"));
-        int next = npairs;
-        if (cnt & 1) {  // odd one out is carried with its GGSW and operand (no new bootstrap needed)
-            CUDA_TRY(cudaMemcpyAsync(d_lwe[cur ^ 1] + (size_t)npairs * vals_lwe, d_lwe[cur] + (size_t)(cnt - 1) * vals_lwe,
-                                     vals_lwe * 8, cudaMemcpyDeviceToDevice, ctx->stream));
-            CUDA_TRY(cudaMemcpyAsync(d_ggsw[cur ^ 1] + (size_t)npairs * vals_ggsw, d_ggsw[cur] + (size_t)(cnt - 1) * vals_ggsw,
-                                     vals_ggsw * 8, cudaMemcpyDeviceToDevice, ctx->stream));
-            CUDA_TRY(cudaMemcpyAsync(d_op[cur ^ 1] + (size_t)npairs * vals_op, d_op[cur] + (size_t)(cnt - 1) * vals_op,
-                                     vals_op * 8, cudaMemcpyDeviceToDevice, ctx->stream));
-            next++;
-        }
-        fresh = npairs;
-        cnt = next;
-        cur ^= 1;
-    }
-    return download(ctx, out, d_lwe[cur], vals_lwe * 8);
-}
-
 }  // extern "C"
 
-// Executes a host-planned LUT circuit (host/ip_plan.h) on `nin` input bit ciphertexts: every layer is
-// [LWE additions] -> [gather -> LWE keyswitch -> circuit bootstrap] -> [fresh operands from the bootstrap's GLEV] ->
-// [gathered LUT ladders] -> [LWE additions]; layers whose bootstraps exceed the workspace cap run in sub-batches.
-static int run_lut_plan(cbs_ctx *ctx, const cbs_host::IpPlan &plan, const uint64_t *in, uint64_t *out)
+// ---- stage 8: one core per computation, shared by the host-buffer and the device-resident entry points ----
+
+namespace {
+
+constexpr size_t kValueWords = (size_t)16 * kLweBig;  // one u16 value: 16 big LWE, MSB first
+
+// `bytes` of input into the workspace `d`, from the caller's host memory (host = true) or HBM, on the context stream
+int copy_in(cbs_ctx *ctx, void *d, const void *src, size_t bytes, bool host)
+{
+    CUDA_TRY(cudaMemcpyAsync(d, src, bytes, host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, ctx->stream));
+    return CBS_OK;
+}
+
+// The plan of `kind` for nvals values, compiled into ctx->plans[kind] unless it is there already: host-side planning and
+// the table upload run once per count, and a replaced table is freed in stream order behind the work that still reads it.
+// The tables come from pageable vectors, which cudaMemcpyAsync has staged by the time it returns, so nothing here waits.
+int lut_plan_get(cbs_ctx *ctx, PlanKind kind, int nvals, const LutPlanExec **out)
 {
     using namespace cbs_host;
     constexpr int kCap = 8192;  // circuit bootstraps per sub-batch (bounds the Fourier GGSW workspace to 4.2 GB)
-    struct Batch {
-        int idx_off, m, job_off, njobs, ref_off, nref;
-    };
-    struct LayerExec {
-        int pre_off, npre, post_off, npost;
-        std::vector<Batch> batches;
-    };
-    std::vector<LayerExec> layers;
+    LutPlanExec &E = ctx->plans[kind];
+    *out = &E;
+    if (E.nvals == nvals) return CBS_OK;
+    if (!ctx->d_plan_luts) {
+        // trivial LUT accumulators: coefficient i carries bit (4*acc + i/256) of table[i % 256] at 2^63
+        // (same layout as generate_vec_keyed_lut_accumulator, cbs_lib/src/aes_he.rs:835-875)
+        std::vector<uint64_t> h_luts((size_t)kIpNumLuts * 2 * kGlweWords, 0);
+        for (int l = 0; l < kIpNumLuts; l++)
+            for (int a = 0; a < 2; a++) {
+                uint64_t *body = h_luts.data() + (size_t)(l * 2 + a) * kGlweWords + 2048;
+                for (int i = 0; i < 1024; i++) body[i] = (uint64_t)((ip_lut_value(l, (unsigned)(i % 256)) >> (4 * a + i / 256)) & 1u) << 63;
+            }
+        uint64_t *d = nullptr;
+        CUDA_TRY(cudaMallocAsync(&d, h_luts.size() * 8, ctx->stream));
+        if (cudaMemcpyAsync(d, h_luts.data(), h_luts.size() * 8, cudaMemcpyHostToDevice, ctx->stream) != cudaSuccess) {
+            cudaFreeAsync(d, ctx->stream);
+            set_error("cudaMemcpyAsync(LUT accumulators) failed");
+            return CBS_ERR_CUDA;
+        }
+        ctx->d_plan_luts = d;
+    }
+    const IpPlan plan = kind == kPlanInnerProduct ? ip_make_plan(nvals) : kind == kPlanSum ? sum_make_plan(nvals) : max_make_plan(nvals);
+    std::vector<PlanLayer> layers;
     std::vector<int> h_idx, h_sel, h_lut, h_out, h_add, h_ref;
     for (const IpLayer &L : plan.layers) {
-        LayerExec E;
-        E.pre_off = (int)h_add.size() / 3;
-        E.npre = (int)L.pre.size();
+        PlanLayer P;
+        P.pre_off = (int)h_add.size() / 3;
+        P.npre = (int)L.pre.size();
         for (const IpAdd &a : L.pre) h_add.insert(h_add.end(), {a.dst, a.a, a.b});
-        E.post_off = (int)h_add.size() / 3;
-        E.npost = (int)L.post.size();
+        P.post_off = (int)h_add.size() / 3;
+        P.npost = (int)L.post.size();
         for (const IpAdd &a : L.post) h_add.insert(h_add.end(), {a.dst, a.a, a.b});
         std::vector<int> remap(L.cbs.size(), -1), ref_dst(L.cbs.size(), -1), touched;
         for (const IpRefresh &r : L.refresh) ref_dst[(size_t)r.pos] = r.dst;
-        Batch b{(int)h_idx.size(), 0, (int)h_lut.size(), 0, (int)h_ref.size() / 2, 0};
+        PlanBatch b{(int)h_idx.size(), 0, (int)h_lut.size(), 0, (int)h_ref.size() / 2, 0};
         auto flush = [&]() {
-            if (b.njobs) E.batches.push_back(b);
+            if (b.njobs) P.batches.push_back(b);
             for (int pos : touched) remap[(size_t)pos] = -1;
             touched.clear();
-            b = Batch{(int)h_idx.size(), 0, (int)h_lut.size(), 0, (int)h_ref.size() / 2, 0};
+            b = PlanBatch{(int)h_idx.size(), 0, (int)h_lut.size(), 0, (int)h_ref.size() / 2, 0};
         };
         for (const IpJob &j : L.jobs) {
             int fresh = 0;
@@ -1058,83 +1045,195 @@ static int run_lut_plan(cbs_ctx *ctx, const cbs_host::IpPlan &plan, const uint64
             b.njobs++;
         }
         flush();
-        layers.push_back(std::move(E));
+        layers.push_back(std::move(P));
     }
     int max_m = 1;
-    for (const LayerExec &E : layers)
-        for (const Batch &b : E.batches) max_m = b.m > max_m ? b.m : max_m;
+    for (const PlanLayer &P : layers)
+        for (const PlanBatch &b : P.batches) max_m = b.m > max_m ? b.m : max_m;
     for (int i = 0; i < 16; i++) h_idx.push_back(plan.result[15 - i]);  // final gather, MSB first
 
-    // trivial LUT accumulators: coefficient i carries bit (4*acc + i/256) of table[i % 256] at 2^63
-    // (same layout as generate_vec_keyed_lut_accumulator, cbs_lib/src/aes_he.rs:835-875)
-    std::vector<uint64_t> h_luts((size_t)kIpNumLuts * 2 * kGlweWords, 0);
-    for (int l = 0; l < kIpNumLuts; l++)
-        for (int a = 0; a < 2; a++) {
-            uint64_t *body = h_luts.data() + (size_t)(l * 2 + a) * kGlweWords + 2048;
-            for (int i = 0; i < 1024; i++) body[i] = (uint64_t)((ip_lut_value(l, (unsigned)(i % 256)) >> (4 * a + i / 256)) & 1u) << 63;
-        }
-
-    uint64_t *d_pool, *d_rows, *d_ks, *d_luts, *d_glev;
-    double *d_ggsw_f;
-    int *d_idx, *d_sel, *d_lut, *d_out, *d_add, *d_ref;
-    TRY(ws_typed(ctx, "ip_pool", (size_t)plan.pool_size * kLweBig, &d_pool));
-    TRY(ws_typed(ctx, "ip_rows", (size_t)max_m * kLweBig, &d_rows));
-    TRY(ws_typed(ctx, "ks", (size_t)max_m * kLweSmall, &d_ks));
-    TRY(ws_typed(ctx, "ggsw_f", (size_t)max_m * kGgswWords, &d_ggsw_f));
-    TRY(ws_typed(ctx, "glev", (size_t)max_m * kGlevWords, &d_glev));  // the circuit bootstrap's own GLEV workspace
-    TRY(ws_typed(ctx, "ip_luts", h_luts.size(), &d_luts));
-    TRY(ws_typed(ctx, "ip_idx", h_idx.size(), &d_idx));
-    TRY(ws_typed(ctx, "ip_sel", h_sel.size() + 1, &d_sel));
-    TRY(ws_typed(ctx, "ip_lut", h_lut.size() + 1, &d_lut));
-    TRY(ws_typed(ctx, "ip_out", h_out.size() + 1, &d_out));
-    TRY(ws_typed(ctx, "ip_add", h_add.size() + 1, &d_add));
-    TRY(ws_typed(ctx, "ip_ref", h_ref.size() + 1, &d_ref));
-    TRY(upload(ctx, d_pool, in, (size_t)plan.nin_bits * kLweBig * 8));
-    TRY(upload(ctx, d_luts, h_luts.data(), h_luts.size() * 8));
-    TRY(upload(ctx, d_idx, h_idx.data(), h_idx.size() * sizeof(int)));
-    if (!h_lut.empty()) {
-        TRY(upload(ctx, d_sel, h_sel.data(), h_sel.size() * sizeof(int)));
-        TRY(upload(ctx, d_lut, h_lut.data(), h_lut.size() * sizeof(int)));
-        TRY(upload(ctx, d_out, h_out.data(), h_out.size() * sizeof(int)));
+    std::vector<int> tab;
+    size_t off[6];
+    const std::vector<int> *parts[6] = {&h_idx, &h_sel, &h_lut, &h_out, &h_add, &h_ref};
+    for (int k = 0; k < 6; k++) {
+        off[k] = tab.size();
+        tab.insert(tab.end(), parts[k]->begin(), parts[k]->end());
     }
-    if (!h_add.empty()) TRY(upload(ctx, d_add, h_add.data(), h_add.size() * sizeof(int)));
-    if (!h_ref.empty()) TRY(upload(ctx, d_ref, h_ref.data(), h_ref.size() * sizeof(int)));
-    for (const LayerExec &E : layers) {
-        if (E.npre) {
-            launch_lwe_add_rows(d_pool, d_add + (size_t)E.pre_off * 3, E.npre, ctx->stream);
+    E.nvals = 0;
+    if (E.d_tab) {
+        CUDA_TRY(cudaFreeAsync(E.d_tab, ctx->stream));
+        E.d_tab = nullptr;
+    }
+    CUDA_TRY(cudaMallocAsync(&E.d_tab, tab.size() * sizeof(int), ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(E.d_tab, tab.data(), tab.size() * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+    E.idx = E.d_tab + off[0];
+    E.sel = E.d_tab + off[1];
+    E.lut = E.d_tab + off[2];
+    E.out = E.d_tab + off[3];
+    E.add = E.d_tab + off[4];
+    E.ref = E.d_tab + off[5];
+    E.final_idx = (int)h_idx.size() - 16;
+    E.nin_bits = plan.nin_bits;
+    E.pool_size = plan.pool_size;
+    E.max_m = max_m;
+    E.layers = std::move(layers);
+    E.nvals = nvals;
+    return CBS_OK;
+}
+
+// Executes the LUT circuit `kind` (host/ip_plan.h) on nvals values: every layer is
+// [LWE additions] -> [gather -> LWE keyswitch -> circuit bootstrap] -> [fresh operands from the bootstrap's GLEV] ->
+// [gathered LUT ladders] -> [LWE additions]; layers whose bootstraps exceed the workspace cap run in sub-batches.
+// The input rows are x, then y (y = nullptr: x holds them all).  host: x, y and out are host buffers and the call returns
+// with the result downloaded; otherwise they are device pointers and the work is only queued.
+int run_lut_plan(cbs_ctx *ctx, PlanKind kind, int nvals, const uint64_t *x, const uint64_t *y, bool host, uint64_t *out)
+{
+    const LutPlanExec *E;
+    TRY(lut_plan_get(ctx, kind, nvals, &E));
+    uint64_t *d_pool, *d_rows, *d_ks, *d_glev;
+    double *d_ggsw_f;
+    TRY(ws_typed(ctx, "ip_pool", (size_t)E->pool_size * kLweBig, &d_pool));
+    TRY(ws_typed(ctx, "ip_rows", (size_t)std::max(E->max_m, 16) * kLweBig, &d_rows));  // also holds the 16 result rows
+    TRY(ws_typed(ctx, "ks", (size_t)E->max_m * kLweSmall, &d_ks));
+    TRY(ws_typed(ctx, "ggsw_f", (size_t)E->max_m * kGgswWords, &d_ggsw_f));
+    TRY(ws_typed(ctx, "glev", (size_t)E->max_m * kGlevWords, &d_glev));  // the circuit bootstrap's own GLEV workspace
+    const size_t x_words = (size_t)(y ? E->nin_bits / 2 : E->nin_bits) * kLweBig;
+    TRY(copy_in(ctx, d_pool, x, x_words * 8, host));
+    if (y) TRY(copy_in(ctx, d_pool + x_words, y, x_words * 8, host));
+    for (const PlanLayer &P : E->layers) {
+        if (P.npre) {
+            launch_lwe_add_rows(d_pool, E->add + (size_t)P.pre_off * 3, P.npre, ctx->stream);
             ctx->launches++;
             TRY(check_launch("k_lwe_add_rows"));
         }
-        for (const Batch &b : E.batches) {
-            launch_gather_lwe(d_pool, d_idx + b.idx_off, d_rows, b.m, ctx->stream);
+        for (const PlanBatch &b : P.batches) {
+            launch_gather_lwe(d_pool, E->idx + b.idx_off, d_rows, b.m, ctx->stream);
             ctx->launches++;
             TRY(check_launch("k_gather_lwe"));
             TRY(dev_keyswitch(ctx, d_rows, d_ks, b.m));
             TRY(dev_circuit_bootstrap(ctx, d_ks, nullptr, d_ggsw_f, b.m));
             if (b.nref) {
-                launch_glev_to_lwe(d_glev, d_ref + (size_t)b.ref_off * 2, d_pool, b.nref, ctx->stream);
+                launch_glev_to_lwe(d_glev, E->ref + (size_t)b.ref_off * 2, d_pool, b.nref, ctx->stream);
                 ctx->launches++;
                 TRY(check_launch("k_glev_to_lwe"));
             }
-            launch_lut8_gather(ctx->K, d_ggsw_f, d_sel + (size_t)b.job_off * 8, d_luts, d_lut + b.job_off, d_out + b.job_off, d_pool,
-                               b.njobs, ctx->stream);
+            launch_lut8_gather(ctx->K, d_ggsw_f, E->sel + (size_t)b.job_off * 8, ctx->d_plan_luts, E->lut + b.job_off,
+                               E->out + b.job_off, d_pool, b.njobs, ctx->stream);
             ctx->launches++;
             TRY(check_launch("k_lut8_gather"));
         }
-        if (E.npost) {
-            launch_lwe_add_rows(d_pool, d_add + (size_t)E.post_off * 3, E.npost, ctx->stream);
+        if (P.npost) {
+            launch_lwe_add_rows(d_pool, E->add + (size_t)P.post_off * 3, P.npost, ctx->stream);
             ctx->launches++;
             TRY(check_launch("k_lwe_add_rows"));
         }
     }
-    launch_gather_lwe(d_pool, d_idx + (h_idx.size() - 16), d_rows, 16, ctx->stream);
+    launch_gather_lwe(d_pool, E->idx + E->final_idx, host ? d_rows : out, 16, ctx->stream);
     ctx->launches++;
     TRY(check_launch("k_gather_lwe"));
-    // download() synchronises the stream, so the host tables above outlive every asynchronous copy
-    return download(ctx, out, d_rows, (size_t)16 * kLweBig * 8);
+    return host ? download(ctx, out, d_rows, kValueWords * 8) : CBS_OK;
 }
 
+// The reference's max_of_two CMux ladder over a balanced tree, nvals >= 2; host / device buffers as run_lut_plan.
+int max_ladder(cbs_ctx *ctx, const uint64_t *in, int nvals, bool host, uint64_t *out)
+{
+    // balanced tree: level buffers A (current) and B (next)
+    uint64_t *d_lwe[2], *d_op[2], *d_ks, *d_glev;
+    double *d_ggsw[2];
+    int *d_a, *d_b;
+    const size_t vals_lwe = kValueWords, vals_ggsw = (size_t)16 * kGgswWords, vals_op = (size_t)16 * kGlweWords;
+    TRY(ws_typed(ctx, "max_lwe0", (size_t)nvals * vals_lwe, &d_lwe[0]));
+    TRY(ws_typed(ctx, "max_lwe1", (size_t)((nvals + 1) / 2) * vals_lwe, &d_lwe[1]));
+    TRY(ws_typed(ctx, "max_ggsw0", (size_t)nvals * vals_ggsw, &d_ggsw[0]));
+    TRY(ws_typed(ctx, "max_ggsw1", (size_t)((nvals + 1) / 2) * vals_ggsw, &d_ggsw[1]));
+    TRY(ws_typed(ctx, "max_op0", (size_t)nvals * vals_op, &d_op[0]));
+    TRY(ws_typed(ctx, "max_op1", (size_t)((nvals + 1) / 2) * vals_op, &d_op[1]));
+    TRY(ws_typed(ctx, "ks", (size_t)nvals * 16 * kLweSmall, &d_ks));
+    TRY(ws_typed(ctx, "glev", (size_t)nvals * 16 * kGlevWords, &d_glev));  // the circuit bootstrap's own GLEV workspace
+    // pair tables (2i, 2i+1) do not depend on the count: one table sized to the largest count seen serves every call
+    const int pairs = std::max(nvals / 2, ctx->ladder_pairs);
+    TRY(ws_typed(ctx, "max_a", (size_t)pairs, &d_a));
+    TRY(ws_typed(ctx, "max_b", (size_t)pairs, &d_b));
+    if (pairs > ctx->ladder_pairs) {
+        std::vector<int> ha(pairs), hb(pairs);
+        for (int i = 0; i < pairs; i++) {
+            ha[i] = 2 * i;
+            hb[i] = 2 * i + 1;
+        }
+        TRY(upload(ctx, d_a, ha.data(), sizeof(int) * ha.size()));
+        TRY(upload(ctx, d_b, hb.data(), sizeof(int) * hb.size()));
+        ctx->ladder_pairs = pairs;
+    }
+    TRY(copy_in(ctx, d_lwe[0], in, (size_t)nvals * vals_lwe * 8, host));
+    int cnt = nvals, cur = 0, fresh = nvals;  // `fresh` leading values of the current level still need a CBS
+    while (cnt > 1) {
+        // keyswitch + circuit bootstrap the values produced by the previous level (server_encrypted_compute.rs:213-263,314-342);
+        // the level-1 GLEV of the same bootstrap, doubled, is the refreshed data operand of the ladder
+        TRY(dev_keyswitch(ctx, d_lwe[cur], d_ks, fresh * 16));
+        TRY(dev_circuit_bootstrap(ctx, d_ks, nullptr, d_ggsw[cur], fresh * 16));
+        launch_glev_to_operand(d_glev, d_op[cur], fresh * 16, ctx->stream);
+        ctx->launches++;
+        TRY(check_launch("k_glev_to_operand"));
+        const int npairs = cnt / 2;
+        launch_max_ladder(ctx->K, d_ggsw[cur], d_op[cur], d_a, d_b, d_lwe[cur ^ 1], npairs, ctx->stream);
+        ctx->launches++;
+        TRY(check_launch("k_max_ladder"));
+        int next = npairs;
+        if (cnt & 1) {  // odd one out is carried with its GGSW and operand (no new bootstrap needed)
+            CUDA_TRY(cudaMemcpyAsync(d_lwe[cur ^ 1] + (size_t)npairs * vals_lwe, d_lwe[cur] + (size_t)(cnt - 1) * vals_lwe,
+                                     vals_lwe * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+            CUDA_TRY(cudaMemcpyAsync(d_ggsw[cur ^ 1] + (size_t)npairs * vals_ggsw, d_ggsw[cur] + (size_t)(cnt - 1) * vals_ggsw,
+                                     vals_ggsw * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+            CUDA_TRY(cudaMemcpyAsync(d_op[cur ^ 1] + (size_t)npairs * vals_op, d_op[cur] + (size_t)(cnt - 1) * vals_op,
+                                     vals_op * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+            next++;
+        }
+        fresh = npairs;
+        cnt = next;
+        cur ^= 1;
+    }
+    if (host) return download(ctx, out, d_lwe[cur], vals_lwe * 8);
+    CUDA_TRY(cudaMemcpyAsync(out, d_lwe[cur], vals_lwe * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+    return CBS_OK;
+}
+
+int max_u16(cbs_ctx *ctx, const uint64_t *in, int nvals, bool host, uint64_t *out)
+{
+    if (nvals == 1) {
+        if (host) memcpy(out, in, kValueWords * 8);
+        else CUDA_TRY(cudaMemcpyAsync(out, in, kValueWords * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+        return CBS_OK;
+    }
+    // up to the reference's own 8 values: its max_of_two CMux ladder; above (where the reference cannot run and the
+    // ladder's data-dependent noise becomes a real failure probability): the LUT circuit.  CBS_MAX_VARIANT=ladder|lut overrides.
+    const char *e = getenv("CBS_MAX_VARIANT");
+    const bool lut = e ? (strcmp(e, "lut") == 0) : nvals > 8;
+    return lut ? run_lut_plan(ctx, kPlanMax, nvals, in, nullptr, host, out) : max_ladder(ctx, in, nvals, host, out);
+}
+
+// Arguments of the device-resident calls: count values in d_x (and as many in d_y when given), 16 result rows in d_out,
+// which must not overlap either input.  Counts stay where count * 16 bit ciphertexts (both halves) fit an int.
+int check_dev_args(const char *what, int count, const uint64_t *d_x, const uint64_t *d_y, bool need_y, const uint64_t *d_out)
+{
+    auto overlaps = [](const uint64_t *a, size_t a_words, const uint64_t *b, size_t b_words) { return a < b + b_words && b < a + a_words; };
+    const bool ok = count > 0 && count <= (INT_MAX >> 5) && d_x && d_out && (d_y || !need_y) &&
+                    !overlaps(d_out, kValueWords, d_x, (size_t)count * kValueWords) &&
+                    !(d_y && overlaps(d_out, kValueWords, d_y, (size_t)count * kValueWords));
+    if (ok) return CBS_OK;
+    set_error(std::string(what) + ": bad argument (need a positive count, non-null pointers and a d_out apart from the inputs)");
+    return CBS_ERR_ARG;
+}
+
+}  // namespace
+
 extern "C" {
+
+int cbs_max_u16(cbs_ctx *ctx, const uint64_t *in, int nvals, uint64_t *out)
+{
+    ENTER(ctx);
+    if (nvals <= 0 || !in || !out) return set_error("cbs_max_u16: bad argument"), CBS_ERR_ARG;
+    return max_u16(ctx, in, nvals, true, out);
+}
 
 // Mini-workload #2 of the harness (harness/cleartext_impl.py:65-70; no reference implementation exists, SURVEY.md
 // 8(f)2): sum_i (x_i * y_i mod 2^16) mod 2^16 with x = first half, y = second half of the values.  The circuit
@@ -1144,7 +1243,7 @@ int cbs_inner_product_u16(cbs_ctx *ctx, const uint64_t *in, int nvals, uint64_t 
 {
     ENTER(ctx);
     if (nvals <= 0 || (nvals & 1) || !in || !out) return set_error("cbs_inner_product_u16: bad argument (need an even number of values)"), CBS_ERR_ARG;
-    return run_lut_plan(ctx, cbs_host::ip_make_plan(nvals), in, out);
+    return run_lut_plan(ctx, kPlanInnerProduct, nvals, in, nullptr, true, out);
 }
 
 // Sum of nvals 16-bit values mod 2^16 (the column-compression stage of the inner product alone): combines per-GPU
@@ -1153,7 +1252,7 @@ int cbs_sum_u16(cbs_ctx *ctx, const uint64_t *in, int nvals, uint64_t *out)
 {
     ENTER(ctx);
     if (nvals <= 0 || !in || !out) return set_error("cbs_sum_u16: bad argument"), CBS_ERR_ARG;
-    return run_lut_plan(ctx, cbs_host::sum_make_plan(nvals), in, out);
+    return run_lut_plan(ctx, kPlanSum, nvals, in, nullptr, true, out);
 }
 
 // Maximum as a LUT circuit (host/ip_plan.h max_make_plan): noise independent of the data and of the tree depth.
@@ -1161,7 +1260,35 @@ int cbs_max_u16_lut(cbs_ctx *ctx, const uint64_t *in, int nvals, uint64_t *out)
 {
     ENTER(ctx);
     if (nvals <= 0 || !in || !out) return set_error("cbs_max_u16_lut: bad argument"), CBS_ERR_ARG;
-    return run_lut_plan(ctx, cbs_host::max_make_plan(nvals), in, out);
+    return run_lut_plan(ctx, kPlanMax, nvals, in, nullptr, true, out);
+}
+
+int cbs_max_u16_dev(cbs_ctx *ctx, const uint64_t *d_in, int nvals, uint64_t *d_out)
+{
+    ENTER(ctx);
+    TRY(check_dev_args("cbs_max_u16_dev", nvals, d_in, nullptr, false, d_out));
+    return max_u16(ctx, d_in, nvals, false, d_out);
+}
+
+int cbs_max_u16_lut_dev(cbs_ctx *ctx, const uint64_t *d_in, int nvals, uint64_t *d_out)
+{
+    ENTER(ctx);
+    TRY(check_dev_args("cbs_max_u16_lut_dev", nvals, d_in, nullptr, false, d_out));
+    return run_lut_plan(ctx, kPlanMax, nvals, d_in, nullptr, false, d_out);
+}
+
+int cbs_sum_u16_dev(cbs_ctx *ctx, const uint64_t *d_in, int nvals, uint64_t *d_out)
+{
+    ENTER(ctx);
+    TRY(check_dev_args("cbs_sum_u16_dev", nvals, d_in, nullptr, false, d_out));
+    return run_lut_plan(ctx, kPlanSum, nvals, d_in, nullptr, false, d_out);
+}
+
+int cbs_inner_product_u16_dev(cbs_ctx *ctx, const uint64_t *d_x, const uint64_t *d_y, int npairs, uint64_t *d_out)
+{
+    ENTER(ctx);
+    TRY(check_dev_args("cbs_inner_product_u16_dev", npairs, d_x, d_y, true, d_out));
+    return run_lut_plan(ctx, kPlanInnerProduct, 2 * npairs, d_x, d_y, false, d_out);
 }
 
 }  // extern "C"
