@@ -73,6 +73,9 @@ struct cbs_ctx {
     int *d_masks_nonzero = nullptr;
     std::map<std::string, DevBuf> ws;
     int chunk_blocks = 64;
+    // circuit bootstraps per sub-batch of a stage-8 LUT-circuit layer (bounds the Fourier GGSW workspace to 4.2 GB at
+    // the default; CBS_PLAN_CAP lowers it so that small inputs take the sub-batch path too)
+    int plan_cap = 8192;
     // Lanes: a chunk is processed as up to kMaxLanes block-aligned parts on separate side streams so that
     // the second (partial) wave of one part's blind rotation overlaps the trace / scheme switch / LUT
     // kernels of another part.  lane = -1: work is issued on `stream` with un-prefixed workspaces.
@@ -488,6 +491,8 @@ int cbs_ctx_create(const cbs_keyset *ks, int device, cbs_ctx **out)
     ctx->device = device;
     if (const char *e = getenv("CBS_CHUNK_BLOCKS")) ctx->chunk_blocks = std::max(1, atoi(e));
     if (const char *e = getenv("CBS_LANES")) ctx->lanes = std::max(1, std::min((int)cbs_ctx::kMaxLanes, atoi(e)));
+    // at least 8: one job of a layer can bring 8 new bits into a sub-batch
+    if (const char *e = getenv("CBS_PLAN_CAP")) ctx->plan_cap = std::max(8, atoi(e));
     Activate act(ctx);
     keep_pool_memory(device);
     cudaError_t e = cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking);
@@ -976,7 +981,7 @@ int copy_in(cbs_ctx *ctx, void *d, const void *src, size_t bytes, bool host)
 int lut_plan_get(cbs_ctx *ctx, PlanKind kind, int nvals, const LutPlanExec **out)
 {
     using namespace cbs_host;
-    constexpr int kCap = 8192;  // circuit bootstraps per sub-batch (bounds the Fourier GGSW workspace to 4.2 GB)
+    const int kCap = ctx->plan_cap;  // circuit bootstraps per sub-batch
     LutPlanExec &E = ctx->plans[kind];
     *out = &E;
     if (E.nvals == nvals) return CBS_OK;
