@@ -288,7 +288,10 @@ CBS_HD double i32_to_double(int32_t x)
 
 // Inverse-FFT output -> torus word.  `r` already carries the 2^64 scale (folded into the key's
 // Fourier data), so: reduce modulo 2^64 to the nearest multiple (magic add, exact), then one
-// round-to-nearest conversion.  Same value as tfhe's from_torus(frac) * 2^64 rounding.
+// round-to-nearest conversion.  Same value as tfhe's from_torus(frac) * 2^64 rounding, except at
+// r = 2^63 mod 2^65: the tie of the reduction goes to the even multiple, f = +2^63, and the
+// conversion saturates to 2^63 - 1 where tfhe gives 2^63 (one unit of 2^-64, DESIGN.md section 2;
+// the exact fix costs 123 instructions per blind-rotation step).  The host branch does the same.
 CBS_HD uint64_t torus_from_scaled(double r)
 {
     const double M = 124615124604835863084731911901282304.0;  // 1.5 * 2^116: ulp = 2^64
@@ -297,7 +300,7 @@ CBS_HD uint64_t torus_from_scaled(double r)
 #ifdef __CUDA_ARCH__
     return (uint64_t)__double2ll_rn(f);
 #else
-    if (f >= 9223372036854775808.0) return 0x8000000000000000ull;
+    if (f >= 9223372036854775808.0) return 0x7FFFFFFFFFFFFFFFull;
     double rr = __builtin_nearbyint(f);
     return (uint64_t)(int64_t)rr;
 #endif

@@ -209,7 +209,7 @@ int main()
         long double fr = (long double)r / 18446744073709551616.0L;
         fr -= roundl(fr);
         long double want = roundl(fr * 18446744073709551616.0L);
-        uint64_t w = (want >= 9223372036854775808.0L) ? 0x8000000000000000ull : (uint64_t)(int64_t)want;
+        uint64_t w = (want >= 9223372036854775808.0L) ? 0x7FFFFFFFFFFFFFFFull : (uint64_t)(int64_t)want;  // saturates like the device
         if (got != w) bad_tor++;
     }
     printf("roundtrip_err=%.3e conv_err=%.3e bin_err=%.3e x_roundtrip_err=%.3e x_conv_err=%.3e bank_conflicts=%d bad_decomp=%d bad_torus=%d\n",
