@@ -9,6 +9,7 @@ CUDA-event times, max over ranks, and rank 0 prints.
   python bench_sweep.py                      # CBS sweep 1..16384 + AES 64/256/1024 blocks
   python bench_sweep.py --cbs-only / --aes-only
   torchrun --nproc_per_node 8 bench_sweep.py --config5 1024 --config5-dev 1024   # configs[4], host-buffer and HBM-resident
+  python bench_sweep.py --pack 8 64 1024     # LWE-to-GLWE packing of the CTR transcipher output (1 GPU)
 Each CBS point = LWE keyswitch-free circuit bootstrap (blind rotation -> GLEV extraction + trace ->
 scheme switch to a Fourier GGSW), inputs resident in HBM, CUDA events on the launching stream, 3
 warm-up + 5 timed launches; the first batch sizes are verified by decrypting the GGSW rows.
@@ -38,6 +39,9 @@ def main():
                     help="the same job with every ciphertext kept in HBM: device-resident CTR transciphering per rank, the max "
                          "on each rank's own values, the inner product after a point-to-point exchange of the rows each rank's "
                          "pairs need (sharding.max_u16_sharded_dev / inner_product_u16_sharded_dev); combinable with --config5")
+    ap.add_argument("--pack", type=int, nargs="*", default=None, metavar="BLOCKS",
+                    help="LWE-to-GLWE packing only: transcipher BLOCKS (default 8 64 1024) CTR blocks in HBM, time "
+                         "cbs_pack_lwes_dev and the download of the packed GLWEs against that of the LWE rows (1 GPU)")
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     import numpy as np
@@ -101,6 +105,11 @@ def main():
         sync_all()
         return max_over_ranks(e0.elapsed_time(e1) / reps)
 
+    if args.pack is not None:
+        assert world == 1, "--pack runs on one GPU"
+        pack_bench(args.pack or [8, 64, 1024], ks, ctx, stream, local, emit)
+        args.aes_only = args.cbs_only = True  # nothing else
+        args.aes_blocks = []
     if args.config5:
         config5(args.config5, ks, ctx, stream, world, rank, local, dist, emit, sync_all, max_over_ranks)
     if args.config5_dev:
@@ -336,6 +345,71 @@ def config5_dev(nb, ks, ctx, world, rank, local, dist, emit, sync_all, max_over_
               "note": "ciphertexts stay in HBM: *_dev calls on every rank, point-to-point row exchange for the inner product, "
                       "device-side gather of the 16-ciphertext partials; wall clock ending in a device synchronise, max over "
                       "ranks; mini-workloads are checked against the values stage 7 actually produced"})
+
+
+def pack_bench(blocks, ks, ctx, stream, local, emit):
+    """LWE-to-GLWE packing of the device-resident CTR transcipher output.  Per block count: the blocks are transciphered in
+    HBM, cbs_pack_lwes_dev is timed with CUDA events on the launching stream (2 warm-up calls, then the mean of 5 calls; at
+    8 blocks the 8.4 MB of input stays in L2 between calls, from 64 blocks on it does not), and the download of the packed
+    GLWEs is timed against the download of the LWE rows it replaces (pinned host buffers, best of 3 each).  Verified by
+    decrypting both: every packed bit must equal the bit of its row.  The card's name, power limit and max SM clock are
+    read in the same run."""
+    import subprocess
+    import numpy as np
+    import torch
+    import aes_clear
+    import ref_io
+    import temp_fhe_transciphering_b200 as cbs
+    try:
+        card = subprocess.run(["nvidia-smi", f"--id={local}", "--query-gpu=name,power.limit,clocks.max.sm",
+                               "--format=csv,noheader"], capture_output=True, text=True, timeout=30).stdout.strip()
+    except (OSError, subprocess.TimeoutExpired):
+        card = "nvidia-smi unavailable"
+    key, iv = aes_clear.harness_aes_key(None), aes_clear.harness_iv(None)
+    ctx.upload_fwd_trans_key(*ks.gen_forward_transciphering_keys(key, 424242))
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+
+    def events_ms(fn, reps):
+        torch.cuda.synchronize()
+        e0.record(stream)
+        for _ in range(reps):
+            fn()
+        e1.record(stream)
+        torch.cuda.synchronize()
+        return e0.elapsed_time(e1) / reps
+
+    for nb in blocks:
+        pt = bytes(np.random.default_rng(nb).integers(0, 256, 16 * nb, dtype=np.uint8))
+        ct = aes_clear.ctr_crypt(key, iv, pt)
+        counters = b"".join(((int.from_bytes(iv, "big") + b) % (1 << 128)).to_bytes(16, "big") for b in range(nb))
+        d_ctr = torch.frombuffer(bytearray(counters), dtype=torch.uint8).cuda()
+        d_ct = torch.frombuffer(bytearray(ct), dtype=torch.uint8).cuda()
+        rows = torch.empty((nb, 128, 2049), dtype=torch.int64, device="cuda")
+        ctx.ctr_transcipher_dev(d_ctr.data_ptr(), d_ct.data_ptr(), nb, rows.data_ptr())
+        count = 128 * nb
+        packed = torch.empty(((count + 1023) // 1024, 3072), dtype=torch.int64, device="cuda")
+
+        def run():
+            ctx.pack_lwes_dev(rows.data_ptr(), count, packed.data_ptr())
+
+        for _ in range(2):
+            run()
+        ms_pack = events_ms(run, 5)
+        h_rows = torch.empty(rows.shape, dtype=torch.int64, pin_memory=True)
+        h_packed = torch.empty(packed.shape, dtype=torch.int64, pin_memory=True)
+        ms_rows = min(events_ms(lambda: h_rows.copy_(rows, non_blocking=True), 1) for _ in range(3))
+        ms_packed = min(events_ms(lambda: h_packed.copy_(packed, non_blocking=True), 1) for _ in range(3))
+        lwe = h_rows.numpy().view(np.uint64).reshape(-1, 2049)
+        bits_rows = ref_io.decode_bit(ref_io.lwe_phase(lwe, ks.glwe_sk)).astype(np.uint64)
+        bits_packed = cbs.glwe_decrypt_bits(ks.glwe_sk, h_packed.numpy().view(np.uint64), count)
+        groups = [1024] * (count // 1024) + ([count % 1024] if count % 1024 else [])  # inputs per packed GLWE
+        wrong = np.flatnonzero((bits_rows != np.unpackbits(np.frombuffer(pt, dtype=np.uint8))).reshape(nb, 128).any(axis=1))
+        emit({"bench": "pack_lwes", "blocks": nb, "lwe_rows": count, "glwes": int(packed.shape[0]), "pack_ms": ms_pack,
+              "rows_per_s": count / (ms_pack * 1e-3), "keyswitches": sum(min(c, 1024 >> lv) for c in groups for lv in range(1, 11)),
+              "rows_bytes": rows.numel() * 8, "packed_bytes": packed.numel() * 8,
+              "download_rows_ms": ms_rows, "download_packed_ms": ms_packed,
+              "verified": bool((bits_packed == bits_rows).all()), "blocks_differing_from_cleartext": wrong.tolist(),
+              "card": card, "n_gpus": 1})
 
 
 if __name__ == "__main__":

@@ -120,6 +120,13 @@ int cbs_lwe_list_save(const char *path, const uint64_t *data, uint64_t count, ui
 void cbs_free(void *p);
 /* client side: decrypt_decode_lwe_list (submission/src/help_fun.rs:12-42), delta = 2^63; sk has n words */
 int cbs_lwe_decrypt_bits(const uint64_t *sk, int n, const uint64_t *lwe, uint64_t count, uint64_t *bits_out);
+/* client side, packed results (cbs_pack_lwes): glwe [nglwe][3072] under glwe_sk [2][1024] (the big LWE key); coefficient j
+ * of GLWE g decrypts to bits_out[g * 1024 + j], delta = 2^63, for the first nbits <= nglwe * 1024 bits */
+int cbs_glwe_decrypt_bits(const uint64_t *glwe_sk, const uint64_t *glwe, uint64_t nglwe, uint64_t nbits, uint64_t *bits_out);
+/* GlweCiphertextList<Vec<u64>> {data, glwe_size = 3, polynomial_size = 1024, modulus} of nglwe GLWE (the packed result);
+ * load malloc's *data (free with cbs_free) and rejects any other glwe_size or polynomial size */
+int cbs_glwe_list_save(const char *path, const uint64_t *glwe, uint64_t nglwe);
+int cbs_glwe_list_load(const char *path, uint64_t **data, uint64_t *nglwe);
 /* bincode Vec<u64>: io/<s>/intermediate/decoded_result{,_aes}.txt */
 int cbs_u64_vec_save(const char *path, const uint64_t *data, uint64_t n);
 int cbs_u64_vec_load(const char *path, uint64_t **data /* free with cbs_free */, uint64_t *n);
@@ -236,6 +243,21 @@ int cbs_max_u16_dev(cbs_ctx *ctx, const uint64_t *d_in, int nvals, uint64_t *d_o
 int cbs_max_u16_lut_dev(cbs_ctx *ctx, const uint64_t *d_in, int nvals, uint64_t *d_out);
 int cbs_sum_u16_dev(cbs_ctx *ctx, const uint64_t *d_in, int nvals, uint64_t *d_out);
 int cbs_inner_product_u16_dev(cbs_ctx *ctx, const uint64_t *d_x, const uint64_t *d_y, int npairs, uint64_t *d_out);
+
+/* LWE-to-GLWE packing (Chen-Dai-Kim-Song 2020; cbs_lib glwe_conv.rs pack_lwes): count big LWE bits at delta = 2^63
+ * -> ceil(count / 1024) GLWE, 3072 words each instead of 1024 x 2049.  Input i goes to GLWE i / 1024, where coefficient
+ * i % 1024 decrypts to its bit (cbs_glwe_decrypt_bits); the coefficients past count in the last GLWE decrypt to 0.
+ *   Tree of 10 levels, stride s = 1024 >> L, kappa = 2^L + 1 (the trace's automorphism keys, nothing new from the client):
+ *   p[j] = const_embed(lwe_j >> 10), then q[t] = (p[t] + X^s p[t+s]) + keyswitch(auto, (p[t] - X^s p[t+s])(X^kappa)) for
+ *   t < s.  A group of c inputs costs sum_L min(c, s) keyswitches (10 for one input, 1023 for 1024) and gives the same
+ *   words as the same inputs padded with zero rows.  Packed bits decrypt with the input's noise plus at most about 2^41.
+ *   cbs_pack_lwes: host buffers in_big [count][2049], glwe_out [ceil(count/1024)][3072]; synchronous; count 0 does nothing.
+ *   cbs_pack_lwes_dev: device buffers of the same layouts, so a *_transcipher_dev output ([nblocks][128] big LWE,
+ *   count = 128 nblocks) can be passed as it is; queued on the context's stream behind earlier work (lanes of a
+ *   *_transcipher_dev call included), never synchronises; count <= 0, null pointers and a d_out that overlaps d_in
+ *   return CBS_ERR_ARG. */
+int cbs_pack_lwes(cbs_ctx *ctx, const uint64_t *in_big, int count, uint64_t *glwe_out);
+int cbs_pack_lwes_dev(cbs_ctx *ctx, const uint64_t *d_in, int count, uint64_t *d_out);
 
 int cbs_circuit_bootstrap_dev(cbs_ctx *ctx, const uint64_t *d_in_small, int count);  /* GGSW stays in the workspace */
 int cbs_blind_rotate_dev(cbs_ctx *ctx, const uint64_t *d_in_small, uint64_t *d_acc_out, int count);

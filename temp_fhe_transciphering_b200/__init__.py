@@ -269,6 +269,35 @@ def save_lwe_list(path, arr):
            "cbs_lwe_list_save")
 
 
+def glwe_decrypt_bits(glwe_sk, glwe, nbits=None):
+    """Client side of Context.pack_lwes: coefficient j of GLWE g -> bit g*1024 + j (delta = 2^63) under glwe_sk [2048] (the
+    big LWE key); glwe [nglwe][3072]; the first nbits bits (default all nglwe*1024) as uint64 0/1."""
+    g, pg = _u64(np.reshape(glwe, (-1, GLWE_WORDS)))
+    s, ps = _u64(np.reshape(glwe_sk, (2048,)))
+    nbits = g.shape[0] * 1024 if nbits is None else int(nbits)
+    out, po = _out((nbits,))
+    _check(lib().cbs_glwe_decrypt_bits(ps, pg, ctypes.c_uint64(g.shape[0]), ctypes.c_uint64(nbits), po), "cbs_glwe_decrypt_bits")
+    return out
+
+
+def load_glwe_list(path):
+    """bincode GlweCiphertextList {data, glwe_size = 3, polynomial_size = 1024, modulus} -> [nglwe][3072]."""
+    data = ctypes.POINTER(ctypes.c_uint64)()
+    n = ctypes.c_uint64()
+    _check(lib().cbs_glwe_list_load(str(path).encode(), ctypes.byref(data), ctypes.byref(n)), "cbs_glwe_list_load")
+    try:
+        if n.value == 0:
+            return np.zeros((0, GLWE_WORDS), dtype=np.uint64)
+        return np.ctypeslib.as_array(data, shape=(n.value * GLWE_WORDS,)).reshape(n.value, GLWE_WORDS).copy()
+    finally:
+        lib().cbs_free(data)
+
+
+def save_glwe_list(path, glwe):
+    g, p = _u64(np.reshape(glwe, (-1, GLWE_WORDS)))
+    _check(lib().cbs_glwe_list_save(str(path).encode(), p, ctypes.c_uint64(g.shape[0])), "cbs_glwe_list_save")
+
+
 class Context:
     """One B200: Fourier-domain keys + workspaces (cbs_ctx).  Creation uploads the standard-domain
     keys and converts them on the GPU, replacing server_encrypted_aes_decryption.rs:645-687."""
@@ -442,6 +471,14 @@ class Context:
         _check(lib().cbs_inner_product_u16(self._h, pi, nvals, po), "cbs_inner_product_u16")
         return out
 
+    def pack_lwes(self, lwe_bits):
+        """LWE-to-GLWE packing (cbs_lib glwe_conv.rs pack_lwes): [count][2049] big LWE bits -> [ceil(count/1024)][3072] GLWE;
+        coefficient i % 1024 of GLWE i // 1024 decrypts to bit i (glwe_decrypt_bits)."""
+        a, pi = _u64(np.reshape(lwe_bits, (-1, LWE_BIG)))
+        out, po = _out(((a.shape[0] + 1023) // 1024, GLWE_WORDS))
+        _check(lib().cbs_pack_lwes(self._h, pi, a.shape[0], po), "cbs_pack_lwes")
+        return out
+
     def measure_fp64_tflops(self):
         v = ctypes.c_double()
         _check(lib().cbs_measure_fp64_tflops(self._h, ctypes.byref(v)), "cbs_measure_fp64_tflops")
@@ -484,6 +521,12 @@ class Context:
         """d_x, d_y [npairs][16][2049] -> d_out [16][2049] encrypting sum_i (x_i * y_i mod 2^16) mod 2^16."""
         _check(lib().cbs_inner_product_u16_dev(self._h, ctypes.c_void_p(d_x_ptr), ctypes.c_void_p(d_y_ptr), int(npairs),
                                                ctypes.c_void_p(d_out_ptr)), "cbs_inner_product_u16_dev")
+
+    def pack_lwes_dev(self, d_in_ptr, count, d_out_ptr):
+        """d_in [count][2049] big LWE (a transcipher_dev output as it is) -> d_out [ceil(count/1024)][3072] GLWE, queued on
+        the context stream."""
+        _check(lib().cbs_pack_lwes_dev(self._h, ctypes.c_void_p(d_in_ptr), int(count), ctypes.c_void_p(d_out_ptr)),
+               "cbs_pack_lwes_dev")
 
     def circuit_bootstrap_dev(self, d_in_ptr, count):
         _check(lib().cbs_circuit_bootstrap_dev(self._h, ctypes.c_void_p(d_in_ptr), int(count)), "cbs_circuit_bootstrap_dev")

@@ -1297,3 +1297,49 @@ int cbs_inner_product_u16_dev(cbs_ctx *ctx, const uint64_t *d_x, const uint64_t 
 }
 
 }  // extern "C"
+
+// ---- LWE-to-GLWE packing: one core for the host-buffer and the device-resident call ----
+
+namespace {
+
+// count big LWE at `in` -> ceil(count / 1024) GLWE at `out` (host = true: host buffers, uploaded and downloaded around the
+// kernels; otherwise device buffers and the work is only queued).  The tree levels live in the "pack_ws" workspace.
+int pack_lwes(cbs_ctx *ctx, const uint64_t *in, int count, bool host, uint64_t *out)
+{
+    const size_t nglwe = ((size_t)count + 1023) / 1024;
+    uint64_t *d_ws, *d_in = nullptr, *d_out = nullptr;
+    TRY(ws_typed(ctx, "pack_ws", nglwe * std::min(count, 512) * kGlweWords, &d_ws));
+    if (host) {
+        TRY(ws_typed(ctx, "pack_in", (size_t)count * kLweBig, &d_in));
+        TRY(ws_typed(ctx, "pack_out", nglwe * kGlweWords, &d_out));
+        TRY(copy_in(ctx, d_in, in, (size_t)count * kLweBig * 8, true));
+    }
+    launch_pack_lwes(ctx->K, host ? d_in : in, d_ws, host ? d_out : out, count, ctx->stream);
+    ctx->launches += 10;
+    TRY(check_launch("k_pack_level"));
+    return host ? download(ctx, out, d_out, nglwe * kGlweWords * 8) : CBS_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int cbs_pack_lwes(cbs_ctx *ctx, const uint64_t *in_big, int count, uint64_t *glwe_out)
+{
+    ENTER(ctx);
+    if (count < 0 || count > INT_MAX - 1023 || (count && (!in_big || !glwe_out))) return set_error("cbs_pack_lwes: bad argument"), CBS_ERR_ARG;
+    if (count == 0) return CBS_OK;
+    return pack_lwes(ctx, in_big, count, true, glwe_out);
+}
+
+int cbs_pack_lwes_dev(cbs_ctx *ctx, const uint64_t *d_in, int count, uint64_t *d_out)
+{
+    ENTER(ctx);
+    const size_t in_words = (size_t)count * kLweBig, out_words = ((size_t)count + 1023) / 1024 * kGlweWords;
+    if (count <= 0 || count > INT_MAX - 1023 || !d_in || !d_out || (d_out < d_in + in_words && d_in < d_out + out_words))
+        return set_error("cbs_pack_lwes_dev: bad argument (need a positive count, non-null pointers and a d_out apart from d_in)"),
+               CBS_ERR_ARG;
+    return pack_lwes(ctx, d_in, count, false, d_out);
+}
+
+}  // extern "C"

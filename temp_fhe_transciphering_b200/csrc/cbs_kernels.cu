@@ -1364,27 +1364,300 @@ __global__ void __launch_bounds__(128 * kTr2Glwe, 1) k_trace_v3(const uint64_t *
 // more sub-group barrier per level, the packed digits of a step parked in tensor memory, 124 B of spills): parity-green,
 // trace + scheme switch of 512 ciphertexts 1.88 ms against 1.80 ms (2.12 ms without the digits in tensor memory); the
 // aliasing alone costs 0.5 % at two units (profiles/r02_brbench_variants.txt).  More resident warps do not help here either.
-void launch_trace(const DeviceKeys &K, const uint64_t *in, uint64_t *out, int count, int from_acc, cudaStream_t s)
+
+// ------------------------------------------------------------------------------------------------
+// LWE-to-GLWE packing (Chen-Dai-Kim-Song 2020, cbs_lib glwe_conv.rs pack_lwes): big LWE i -> coefficient i % 1024 of
+// GLWE i / 1024, through a tree of automorphism keyswitches, one launch per level L = 1..10 covering every group.
+// Item t < s = 1024 >> L of a group is
+//   q[t] = (e + X^s o) + keyswitch(auto[10 - L], (e - X^s o)(X^kappa)),   kappa = 2^L + 1,  e = p[t],  o = p[t + s],
+// the keyswitch being one step of k_trace_v3 (the same Split(41) two-limb products, key ring and transforms) with the X^s
+// multiply-add/subtract fused into the load.  Level 1 reads the LWE rows: p[j] = const_embed(lwe_j >> 10) (glev_pre_word's
+// arithmetic).  A group of c inputs has min(c, s) non-zero items at level L and only those run: a zero item stays exactly
+// zero (its digits, spectra and products are 0), and an o past the previous level's min(c, 2s) items is read as zero.
+// Levels 2..9 work in place on ws [group][gs][3072]: item t reads slots t and t + s and writes slot t, and no other item
+// touches either.  Every CTA of a launch reads the same 295 KB key, which stays in L2.  The keyswitch is written out here
+// rather than shared with k_trace_v3 through an inline helper: ptxas then schedules the trace differently.
+__device__ __forceinline__ uint64_t pack_in_word(const uint64_t *item, bool lwe, int p, int j)
 {
-    if (count <= 0) return;
+    if (!lwe) return item[p * 1024 + j];
+    if (p == 2) return j == 0 ? item[2048] >> 10 : 0;
+    return j == 0 ? item[p * 1024] >> 10 : 0ull - (item[p * 1024 + 1024 - j] >> 10);
+}
+
+__global__ void __launch_bounds__(128 * kTr2Glwe, 1) k_pack_level(const uint64_t *src, uint64_t *dst, int count, int level,
+                                                                   int gs, const double *__restrict__ auto_f,
+                                                                   const double *__restrict__ twtab)
+{
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int gl = threadIdx.x >> 7;
+    const int sub = (threadIdx.x >> 6) & 1;
+    const int t = threadIdx.x & 63;
+    const int stride = 1024 >> level;
+    const int items = (count >> 10) * stride + min(count & 1023, stride);
+    const int idx = blockIdx.x * kTr2Glwe + gl;
+    unsigned char *ring = smem_raw + (size_t)kTr2Glwe * kTr3UnitSmem;
+    uint64_t *full = reinterpret_cast<uint64_t *>(ring + 4 * kBrTileBytes + 1024);
+    uint64_t *empty = full + 4;
+    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(empty + 4);
+    const int warp = threadIdx.x >> 5;
+    const int active_units = min(kTr2Glwe, items - blockIdx.x * kTr2Glwe);
+    if (threadIdx.x == 0) {
+        for (int b = 0; b < 4; b++) {
+            mbar_init(full + b, 1);
+            mbar_init(empty + b, 64 * active_units);
+        }
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    if (warp == 0) tmem_alloc_cols(tmem_slot, 128);
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    const uint32_t tm = *tmem_slot + ((uint32_t)(32 * (warp & 3)) << 16) + (uint32_t)(64 * (warp >> 2));
+    {
+        Twiddles tw;
+        load_twiddles_x(tw, twtab, t);
+        tmem_st_c4(tm, tw.t1);
+        tmem_st_c4(tm + 16, tw.t1 + 4);
+        tmem_st_c4(tm + 32, tw.t2);
+        tmem_st_c4(tm + 48, tw.t2 + 4);
+        asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+    }
+    if (idx < items) {
+        const int g = idx / stride, it = idx % stride;
+        const int nprev = min(min(1024, count - g * 1024), 2 * stride);  // non-zero items of the previous level
+        const bool lwe = (level == 1);
+        const size_t item_words = lwe ? kLweBig : kGlweWords;
+        const uint64_t *e_src = src + (lwe ? (size_t)(g * 1024 + it) : (size_t)g * gs + it) * item_words;
+        const uint64_t *o_src = (it + stride < nprev) ? e_src + (size_t)stride * item_words : nullptr;
+        uint64_t *dptr = dst + ((size_t)g * (level == 10 ? 1 : gs) + it) * kGlweWords;
+        const int ks = 10 - level;  // automorphism key X -> X^((1024 >> ks) + 1)
+
+        const bool producer = (threadIdx.x == 0);
+        const char *key_bytes = reinterpret_cast<const char *>(auto_f);
+        // tile of use n (digit level lev = 2 - n), lane (i, sp): Fourier polys [ks][i][sp][lev][0..2]; ring as k_trace_v3
+        auto tile_src = [&](int n, int i, int sp) {
+            return key_bytes + (size_t)((((ks * 2 + i) * 2 + sp) * 3 + (2 - n)) * 3) * kFourierPolyDoubles * 8;
+        };
+        int issued = 0;
+        auto produce = [&](int n, bool early) {
+            if (n >= 3) return;
+    #pragma unroll
+            for (int L = 0; L < 4; L++) {
+                if (issued & (1 << L)) continue;
+                if (n > 0) {
+                    if (early) {
+                        if (!mbar_test(empty + L, (n - 1) & 1)) continue;
+                    } else {
+                        mbar_wait(empty + L, (n - 1) & 1);
+                    }
+                }
+                tma_load_tile(ring + L * kBrTileBytes, tile_src(n, L & 1, L >> 1), kBrTileBytes, full + L);
+                issued |= 1 << L;
+            }
+            if (!early) issued = 0;
+        };
+        if (producer) produce(0, false);
+        __syncwarp();
+        int want = -1;
+
+        unsigned char *base = smem_raw + (size_t)gl * kTr3UnitSmem;
+        u64x2 *cur = reinterpret_cast<u64x2 *>(base);
+        cplx *scr = reinterpret_cast<cplx *>(base + kGlweWords * 8 + sub * 8192);
+        cplx *X = reinterpret_cast<cplx *>(base + kGlweWords * 8 + 16384);
+        const int sbar = 1 + gl * 2 + sub;
+        const int ubar = 5 + gl;
+        const int u = threadIdx.x & 127;
+        // cur = e - X^s o (the keyswitch input), sum = e + X^s o (kept in registers until the input has been read)
+        u64x2 sum[12];
+#pragma unroll
+        for (int k = 0; k < 12; k++) {
+            const int w = u + 128 * k;
+            const int p = k >> 2, jj = w & 511;
+            uint64_t ev[2], xo[2];
+#pragma unroll
+            for (int h = 0; h < 2; h++) {
+                const int j = jj + 512 * h, js = j - stride;
+                ev[h] = pack_in_word(e_src, lwe, p, j);
+                xo[h] = !o_src ? 0ull : js >= 0 ? pack_in_word(o_src, lwe, p, js) : 0ull - pack_in_word(o_src, lwe, p, js + 1024);
+            }
+            cur[w] = u64x2{ev[0] - xo[0], ev[1] - xo[1]};
+            sum[k] = u64x2{ev[0] + xo[0], ev[1] + xo[1]};
+        }
+        unit_sync(ubar);
+
+        const int kinv = c_kappa_inv[ks];
+        uint64_t pk[16];
+        {
+            const u64x2 *p = cur + sub * 512;
+    #pragma unroll
+            for (int m = 0; m < 8; m++) {
+                const int jj = t + 64 * m;
+                const int e = (jj * kinv) & 2047;
+                const u64x2 A = p[e & 511];
+                const int h = e >> 9;
+                pk[2 * m] = pack_digits<13, 3, uint64_t>(pair_pick(A, h));
+                pk[2 * m + 1] = pack_digits<13, 3, uint64_t>(pair_pick(A, (h + kinv) & 3));
+            }
+        }
+        u64x2 pb[4];  // body of the automorphism image, pairs u + 128 q
+    #pragma unroll
+        for (int q = 0; q < 4; q++) {
+            const int e = ((u + 128 * q) * kinv) & 2047;
+            const u64x2 A = cur[1024 + (e & 511)];
+            const int h = e >> 9;
+            pb[q] = u64x2{pair_pick(A, h), pair_pick(A, (h + kinv) & 3)};
+        }
+        unit_sync(ubar);
+    #pragma unroll
+        for (int k = 0; k < 12; k++) {
+            u64x2 x = sum[k];
+            if (k >= 8) {
+                x.lo += pb[k - 8].lo;
+                x.hi += pb[k - 8].hi;
+            }
+            cur[u + 128 * k] = x;
+        }
+
+        cplx acc[3][8];
+    #pragma unroll
+        for (int c = 0; c < 3; c++)
+    #pragma unroll
+            for (int k = 0; k < 8; k++) acc[c][k] = cplx{0.0, 0.0};
+    #pragma unroll 1
+        for (int n = 0; n < 3; n++) {
+            cplx v[8];
+    #pragma unroll
+            for (int m = 0; m < 8; m++)
+                v[m] = cplx{i32_to_double(unpack_digit<13, uint64_t>(pk[2 * m], n)),
+                            i32_to_double(unpack_digit<13, uint64_t>(pk[2 * m + 1], n))};
+            fwd_p1_tm(v, scr, tm, t);
+            group_sync(sbar);
+            if (producer && want >= 0) {
+                produce(want, false);
+                want = -1;
+            }
+            __syncwarp();
+            fwd_p2x_tm(v, scr, tm, t);
+            exchange8<-1>(v, t & 7);
+            fwd_p3x(v);
+            cplx *Xw = X + sub * 512 + t;
+            const cplx *Xr = X + (1 - sub) * 512 + t;
+    #pragma unroll
+            for (int k3 = 0; k3 < 8; k3++) Xw[k3 * 64] = v[k3];
+            unit_sync(ubar);
+            const int Lown = sub * 2 + sub, Loth = sub * 2 + (1 - sub);
+            mbar_wait(full + Lown, n & 1);
+            {
+                const cplx *key = reinterpret_cast<const cplx *>(ring + Lown * kBrTileBytes) + t;
+    #pragma unroll
+                for (int c = 0; c < 3; c++)
+    #pragma unroll
+                    for (int k3 = 0; k3 < 8; k3++) cfma(acc[c][k3], v[k3], key[c * 512 + k3 * 64]);
+            }
+            mbar_arrive(empty + Lown);
+            mbar_wait(full + Loth, n & 1);
+            {
+                const cplx *key = reinterpret_cast<const cplx *>(ring + Loth * kBrTileBytes) + t;
+    #pragma unroll
+                for (int k3 = 0; k3 < 8; k3++) {
+                    const cplx o = Xr[k3 * 64];
+    #pragma unroll
+                    for (int c = 0; c < 3; c++) cfma(acc[c][k3], o, key[c * 512 + k3 * 64]);
+                }
+            }
+            mbar_arrive(empty + Loth);
+            want = n + 1;
+            unit_sync(ubar);
+            if (producer) produce(want, true);
+            __syncwarp();
+        }
+        const int shift = sub ? 41 : 0;
+    #pragma unroll
+        for (int c = 0; c < 3; c++) {
+            inv_p3x(acc[c]);
+            exchange8<1>(acc[c], t & 7);
+            if (producer && want >= 0) {
+                produce(want, false);
+                want = -1;
+            }
+            __syncwarp();
+            inv_p2x_tm(acc[c], scr, tm, t);
+            group_sync(sbar);
+            inv_p1_tm(acc[c], scr, tm, t);
+            u64x2 *p = cur + c * 512;
+            if (sub == 0) {
+    #pragma unroll
+                for (int m = 0; m < 8; m++) {
+                    u64x2 w = p[t + 64 * m];
+                    w.lo += torus_from_scaled(acc[c][m].x);
+                    w.hi += torus_from_scaled(acc[c][m].y);
+                    p[t + 64 * m] = w;
+                }
+            }
+            unit_sync(ubar);
+            if (sub == 1) {
+    #pragma unroll
+                for (int m = 0; m < 8; m++) {
+                    u64x2 w = p[t + 64 * m];
+                    w.lo += torus_from_scaled(acc[c][m].x) << shift;
+                    w.hi += torus_from_scaled(acc[c][m].y) << shift;
+                    p[t + 64 * m] = w;
+                }
+            }
+        }
+        unit_sync(ubar);
+        for (int w = u; w < 3 * 512; w += 128) {
+            const u64x2 x = cur[w];
+            const int c = w >> 9, jj = w & 511;
+            dptr[c * 1024 + jj] = x.lo;
+            dptr[c * 1024 + jj + 512] = x.hi;
+        }
+    }
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    if (warp == 0) tmem_dealloc_cols(*tmem_slot, 128);
+}
+
+// once per device: the automorphism inverses of the trace and packing kernels, and their shared-memory opt-in
+static void auto_kernels_init()
+{
     static bool init_done[64] = {false};
     int init_dev = 0;
     cudaGetDevice(&init_dev);
     bool &init = init_done[init_dev & 63];
-    if (!init) {
-        int kinv[10];
-        for (int i = 0; i < 10; i++) {
-            const int kappa = (1024 >> i) + 1;
-            int x = 1;
-            for (int c = 1; c < 2048; c += 2)
-                if ((c * kappa) % 2048 == 1) x = c;
-            kinv[i] = x;
-        }
-        cudaMemcpyToSymbol(c_kappa_inv, kinv, sizeof(kinv));
-        cudaFuncSetAttribute(k_trace_v3, cudaFuncAttributeMaxDynamicSharedMemorySize, kTr3SmemBytes);
-        init = true;
+    if (init) return;
+    int kinv[10];
+    for (int i = 0; i < 10; i++) {
+        const int kappa = (1024 >> i) + 1;
+        int x = 1;
+        for (int c = 1; c < 2048; c += 2)
+            if ((c * kappa) % 2048 == 1) x = c;
+        kinv[i] = x;
     }
+    cudaMemcpyToSymbol(c_kappa_inv, kinv, sizeof(kinv));
+    cudaFuncSetAttribute(k_trace_v3, cudaFuncAttributeMaxDynamicSharedMemorySize, kTr3SmemBytes);
+    cudaFuncSetAttribute(k_pack_level, cudaFuncAttributeMaxDynamicSharedMemorySize, kTr3SmemBytes);
+    init = true;
+}
+
+void launch_trace(const DeviceKeys &K, const uint64_t *in, uint64_t *out, int count, int from_acc, cudaStream_t s)
+{
+    if (count <= 0) return;
+    auto_kernels_init();
     k_trace_v3<<<(count + kTr2Glwe - 1) / kTr2Glwe, 128 * kTr2Glwe, kTr3SmemBytes, s>>>(in, out, count, from_acc, K.auto_f, K.tw);
+}
+
+void launch_pack_lwes(const DeviceKeys &K, const uint64_t *in, uint64_t *ws, uint64_t *out, int count, cudaStream_t s)
+{
+    if (count <= 0) return;
+    auto_kernels_init();
+    const int gs = std::min(count, 512);
+    for (int level = 1; level <= 10; level++) {
+        const int st = 1024 >> level;
+        const int items = (count >> 10) * st + std::min(count & 1023, st);
+        k_pack_level<<<(items + kTr2Glwe - 1) / kTr2Glwe, 128 * kTr2Glwe, kTr3SmemBytes, s>>>(
+            level == 1 ? in : ws, level == 10 ? out : ws, count, level, gs, K.auto_f, K.tw);
+    }
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -53,6 +53,9 @@ void launch_blind_rotate(const DeviceKeys &K, const uint64_t *lwe, uint64_t *acc
 void launch_glev_from_acc(const uint64_t *acc, uint64_t *glev, int count, cudaStream_t s);
 // a3  trace on `count` GLWE.  from_acc = 1: `in` is acc[count/7][3072] and a2 is fused in.
 void launch_trace(const DeviceKeys &K, const uint64_t *in, uint64_t *out, int count, int from_acc, cudaStream_t s);
+// LWE-to-GLWE packing: in[count][2049] big LWE -> out[ceil(count/1024)][3072], coefficient i % 1024 of GLWE i / 1024
+//     decrypts to bit i; 10 launches (one per tree level), ws[ceil(count/1024)][min(count, 512)][3072] holds the levels
+void launch_pack_lwes(const DeviceKeys &K, const uint64_t *in, uint64_t *ws, uint64_t *out, int count, cudaStream_t s);
 // a4 + a5  glev[count][7][3072] -> ggsw std (nullable) and ggsw Fourier (nullable)
 void launch_scheme_switch(const DeviceKeys &K, const uint64_t *glev, uint64_t *ggsw_std, double *ggsw_f, int count,
                           cudaStream_t s);

@@ -1004,6 +1004,81 @@ int cbs_lwe_decrypt_bits(const uint64_t *sk, int n, const uint64_t *lwe, uint64_
     return CBS_OK;
 }
 
+// The GLWE twin of cbs_lwe_decrypt_bits: coefficient j of GLWE g is bit g * 1024 + j.
+// phase[j] = body[j] - sum_c sum_k s_c[k] m_c[j - k], negated where j - k wraps (X^1024 = -1); only the non-zero key
+// words take part, so a binary key costs about 1024 additions per bit.
+int cbs_glwe_decrypt_bits(const uint64_t *glwe_sk, const uint64_t *glwe, uint64_t nglwe, uint64_t nbits, uint64_t *bits_out)
+{
+    if (!glwe_sk || !glwe || !bits_out || nbits > nglwe * 1024) return CBS_ERR_ARG;
+    std::vector<int> nz[2];
+    for (int c = 0; c < 2; c++)
+        for (int k = 0; k < 1024; k++)
+            if (glwe_sk[c * 1024 + k]) nz[c].push_back(k);
+    const uint64_t delta = 1ull << 63;
+    for (uint64_t b = 0; b < nbits; b++) {
+        const uint64_t *g = glwe + (b / 1024) * 3072;
+        const int j = (int)(b % 1024);
+        uint64_t phase = g[2048 + j];
+        for (int c = 0; c < 2; c++)
+            for (int k : nz[c]) {
+                const uint64_t m = j >= k ? g[c * 1024 + j - k] : 0ull - g[c * 1024 + j - k + 1024];
+                phase -= m * glwe_sk[c * 1024 + k];
+            }
+        const uint64_t rounding = (phase & (delta >> 1)) << 1;
+        bits_out[b] = (phase + rounding) / delta;
+    }
+    return CBS_OK;
+}
+
+// GlweCiphertextList<Vec<u64>> {data, glwe_size = 3, polynomial_size = 1024, modulus}: the shape trans_key.bin holds its
+// first-round LUTs in (all_rd_keys_walk), here for the output of cbs_pack_lwes
+int cbs_glwe_list_save(const char *path, const uint64_t *data, uint64_t nglwe)
+{
+    if (!path || (!data && nglwe)) return CBS_ERR_ARG;
+    Writer w;
+    w.vec(data, nglwe * 3072);
+    w.u64(3);
+    w.u64(1024);
+    w.modulus();
+    std::string p(path);
+    size_t slash = p.find_last_of('/');
+    if (slash != std::string::npos) mkdirs(p.substr(0, slash));
+    if (!w.save(p)) {
+        set_error("cannot write " + p);
+        return CBS_ERR_IO;
+    }
+    return CBS_OK;
+}
+
+int cbs_glwe_list_load(const char *path, uint64_t **data, uint64_t *nglwe)
+{
+    Reader r;
+    if (!path || !data || !nglwe || !r.load(path)) {
+        set_error(std::string("cannot read ") + (path ? path : "(null)"));
+        return CBS_ERR_IO;
+    }
+    uint64_t n = r.u64();
+    // n comes from the file: bound it by the bytes present (40 trailer bytes: sizes and modulus) before using it
+    if (!r.ok || r.buf.size() < r.off + 40 || n != (r.buf.size() - r.off - 40) / 8 || (r.buf.size() - r.off - 40) % 8 || n % 3072) {
+        set_error(std::string(path) + ": not a GlweCiphertextList<u64> of GLWE(2, 1024)");
+        return CBS_ERR_FORMAT;
+    }
+    uint64_t *p = (uint64_t *)malloc(8 * (n ? n : 1));
+    memcpy(p, r.buf.data() + r.off, 8 * n);
+    r.off += 8 * n;
+    r.expect(3);
+    r.expect(1024);
+    r.modulus();
+    if (!r.done()) {
+        free(p);
+        set_error(std::string(path) + ": malformed GlweCiphertextList trailer (need glwe_size 3, polynomial_size 1024)");
+        return CBS_ERR_FORMAT;
+    }
+    *data = p;
+    *nglwe = n / 3072;
+    return CBS_OK;
+}
+
 // bincode Vec<u64> (the intermediate/decoded_result*.txt files of the client stages)
 int cbs_u64_vec_save(const char *path, const uint64_t *data, uint64_t n)
 {
