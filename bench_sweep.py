@@ -10,6 +10,7 @@ CUDA-event times, max over ranks, and rank 0 prints.
   python bench_sweep.py --cbs-only / --aes-only
   torchrun --nproc_per_node 8 bench_sweep.py --config5 1024 --config5-dev 1024   # configs[4], host-buffer and HBM-resident
   python bench_sweep.py --pack 8 64 1024     # LWE-to-GLWE packing of the CTR transcipher output (1 GPU)
+  python bench_sweep.py --seeded-keys 8 64   # seeded transciphering keys against reference-format keys (1 GPU)
 Each CBS point = LWE keyswitch-free circuit bootstrap (blind rotation -> GLEV extraction + trace ->
 scheme switch to a Fourier GGSW), inputs resident in HBM, CUDA events on the launching stream, 3
 warm-up + 5 timed launches; the first batch sizes are verified by decrypting the GGSW rows.
@@ -42,6 +43,9 @@ def main():
     ap.add_argument("--pack", type=int, nargs="*", default=None, metavar="BLOCKS",
                     help="LWE-to-GLWE packing only: transcipher BLOCKS (default 8 64 1024) CTR blocks in HBM, time "
                          "cbs_pack_lwes_dev and the download of the packed GLWEs against that of the LWE rows (1 GPU)")
+    ap.add_argument("--seeded-keys", type=int, nargs="*", default=None, metavar="BLOCKS",
+                    help="seeded transciphering keys only: bytes, upload time and ECB / CTR blocks/s at BLOCKS (default 8 64) "
+                         "with the seeded key against the reference-format key, both forms alternating in one process (1 GPU)")
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     import numpy as np
@@ -108,6 +112,11 @@ def main():
     if args.pack is not None:
         assert world == 1, "--pack runs on one GPU"
         pack_bench(args.pack or [8, 64, 1024], ks, ctx, stream, local, emit)
+        args.aes_only = args.cbs_only = True  # nothing else
+        args.aes_blocks = []
+    if args.seeded_keys is not None:
+        assert world == 1, "--seeded-keys runs on one GPU"
+        seeded_keys_bench(args.seeded_keys or [8, 64], ks, ctx, stream, local, emit)
         args.aes_only = args.cbs_only = True  # nothing else
         args.aes_blocks = []
     if args.config5:
@@ -347,6 +356,115 @@ def config5_dev(nb, ks, ctx, world, rank, local, dist, emit, sync_all, max_over_
                       "ranks; mini-workloads are checked against the values stage 7 actually produced"})
 
 
+def card_info(local):
+    import subprocess
+    try:
+        return subprocess.run(["nvidia-smi", f"--id={local}", "--query-gpu=name,power.limit,clocks.max.sm",
+                               "--format=csv,noheader"], capture_output=True, text=True, timeout=30).stdout.strip()
+    except (OSError, subprocess.TimeoutExpired):
+        return "nvidia-smi unavailable"
+
+
+def seeded_keys_bench(blocks, ks, ctx, stream, local, emit):
+    """Seeded transciphering keys (every LUT encrypted; 32-byte seed + bodies, masks expanded on the GPU) against the
+    reference-format keys (first-round LUTs encrypted, the rest trivial), per direction, in one process:
+      * bytes a client sends: the three AllRdKeys arrays against the seed and the bodies;
+      * upload time: cbs_*trans_key_upload of the full arrays against cbs_*trans_key_seeded_upload, from pinned host buffers,
+        CUDA events on the context stream around each (synchronous) call, 2 warm-up calls, then the mean of 5 calls per form,
+        the two forms alternating;
+      * transcipher throughput through the _dev calls with each key form at each block count (1 warm-up, then the mean of
+        3 calls under CUDA events, forms alternating);
+      * verification in the same run: both outputs decrypt to the plaintext, and the rows after the seeded upload are the
+        rows after uploading the host-expanded key (cbs_*trans_key_seeded_expand), bit for bit.
+    The card's name, power limit and max SM clock are read in the same run."""
+    import numpy as np
+    import torch
+    import aes_clear
+    import ref_io
+    import temp_fhe_transciphering_b200 as cbs
+    card = card_info(local)
+    key, iv = aes_clear.harness_aes_key(None), aes_clear.harness_iv(None)
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+
+    def events_ms(fn, reps):
+        torch.cuda.synchronize()
+        e0.record(stream)
+        for _ in range(reps):
+            fn()
+        e1.record(stream)
+        torch.cuda.synchronize()
+        return e0.elapsed_time(e1) / reps
+
+    def pinned(a):
+        t = torch.empty(a.size, dtype=torch.int64, pin_memory=True)
+        t.numpy().view(np.uint64)[:] = a.reshape(-1)
+        return t.numpy().view(np.uint64).reshape(a.shape)
+
+    for mode in ("ecb", "ctr"):
+        if mode == "ecb":
+            full = [pinned(a) for a in ks.gen_transciphering_keys(key, 31337)]
+            ms, bodies = ks.gen_seeded_transciphering_keys(key, 31338)
+            expanded = cbs.expand_seeded_trans_key(ms, bodies)
+            up_full, up_seeded = ctx.upload_trans_key, ctx.upload_seeded_trans_key
+        else:
+            full = [pinned(a) for a in ks.gen_forward_transciphering_keys(key, 31337)]
+            ms, bodies = ks.gen_seeded_forward_transciphering_keys(key, 31338)
+            expanded = cbs.expand_seeded_fwd_trans_key(ms, bodies)
+            up_full, up_seeded = ctx.upload_fwd_trans_key, ctx.upload_seeded_fwd_trans_key
+        bodies = pinned(bodies)
+        t_full, t_seeded = [], []
+        for rep in range(7):
+            a = events_ms(lambda: up_full(*full), 1)
+            b = events_ms(lambda: up_seeded(ms, bodies), 1)
+            if rep >= 2:
+                t_full.append(a)
+                t_seeded.append(b)
+        emit({"bench": "seeded_trans_key_upload", "mode": mode, "glwes": int(bodies.shape[0]),
+              "reference_format_bytes": int(sum(a.nbytes for a in full)), "seeded_bytes": 32 + int(bodies.nbytes),
+              "upload_reference_format_ms": float(np.mean(t_full)), "upload_seeded_ms": float(np.mean(t_seeded)),
+              "card": card, "n_gpus": 1})
+        for nb in blocks:
+            pt = bytes(np.random.default_rng(nb).integers(0, 256, 16 * nb, dtype=np.uint8))
+            if mode == "ecb":
+                d_in = [torch.frombuffer(bytearray(aes_clear.ecb_encrypt(key, pt)), dtype=torch.uint8).cuda()]
+            else:
+                counters = b"".join(((int.from_bytes(iv, "big") + b) % (1 << 128)).to_bytes(16, "big") for b in range(nb))
+                d_in = [torch.frombuffer(bytearray(counters), dtype=torch.uint8).cuda(),
+                        torch.frombuffer(bytearray(aes_clear.ctr_crypt(key, iv, pt)), dtype=torch.uint8).cuda()]
+            rows = {f: torch.empty((nb, 128, 2049), dtype=torch.int64, device="cuda") for f in ("full", "seeded", "expanded")}
+
+            def run(form):
+                out = rows[form].data_ptr()
+                if mode == "ecb":
+                    ctx.transcipher_dev(d_in[0].data_ptr(), nb, out)
+                else:
+                    ctx.ctr_transcipher_dev(d_in[0].data_ptr(), d_in[1].data_ptr(), nb, out)
+
+            ms_run = {"full": [], "seeded": []}
+            for rep in range(4):
+                for form, upload in (("full", lambda: up_full(*full)), ("seeded", lambda: up_seeded(ms, bodies))):
+                    upload()
+                    t = events_ms(lambda: run(form), 1)
+                    if rep:
+                        ms_run[form].append(t)
+            up_full(*expanded)
+            run("expanded")
+            torch.cuda.synchronize()
+            want = np.unpackbits(np.frombuffer(pt, dtype=np.uint8))
+            wrong = {}
+            for form in ("full", "seeded"):
+                bits = ref_io.decode_bit(ref_io.lwe_phase(rows[form].cpu().numpy().view(np.uint64).reshape(-1, 2049), ks.glwe_sk))
+                wrong[form] = sorted(set((np.flatnonzero(bits != want) // 128).tolist()))
+            same = bool(torch.equal(rows["seeded"], rows["expanded"]))
+            emit({"bench": "seeded_trans_key_transcipher", "mode": mode, "blocks": nb,
+                  "reference_format_ms": float(np.mean(ms_run["full"])), "seeded_ms": float(np.mean(ms_run["seeded"])),
+                  "reference_format_blocks_per_s": nb / (np.mean(ms_run["full"]) * 1e-3),
+                  "seeded_blocks_per_s": nb / (np.mean(ms_run["seeded"]) * 1e-3),
+                  "seeded_rows_equal_host_expanded": same, "blocks_wrong_reference_format": wrong["full"],
+                  "blocks_wrong_seeded": wrong["seeded"], "verified": bool(same and not wrong["full"] and not wrong["seeded"]),
+                  "card": card, "n_gpus": 1})
+
+
 def pack_bench(blocks, ks, ctx, stream, local, emit):
     """LWE-to-GLWE packing of the device-resident CTR transcipher output.  Per block count: the blocks are transciphered in
     HBM, cbs_pack_lwes_dev is timed with CUDA events on the launching stream (2 warm-up calls, then the mean of 5 calls; at
@@ -354,17 +472,12 @@ def pack_bench(blocks, ks, ctx, stream, local, emit):
     GLWEs is timed against the download of the LWE rows it replaces (pinned host buffers, best of 3 each).  Verified by
     decrypting both: every packed bit must equal the bit of its row.  The card's name, power limit and max SM clock are
     read in the same run."""
-    import subprocess
     import numpy as np
     import torch
     import aes_clear
     import ref_io
     import temp_fhe_transciphering_b200 as cbs
-    try:
-        card = subprocess.run(["nvidia-smi", f"--id={local}", "--query-gpu=name,power.limit,clocks.max.sm",
-                               "--format=csv,noheader"], capture_output=True, text=True, timeout=30).stdout.strip()
-    except (OSError, subprocess.TimeoutExpired):
-        card = "nvidia-smi unavailable"
+    card = card_info(local)
     key, iv = aes_clear.harness_aes_key(None), aes_clear.harness_iv(None)
     ctx.upload_fwd_trans_key(*ks.gen_forward_transciphering_keys(key, 424242))
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)

@@ -113,6 +113,45 @@ int cbs_fwd_trans_key_generate_os_entropy(const cbs_keyset *ks, const uint8_t ae
                                           uint64_t *kf_last);
 int cbs_fwd_trans_key_load(const char *path, uint64_t *kf_first, uint64_t *kf_mid, uint64_t *kf_last);
 int cbs_fwd_trans_key_save(const char *path, const uint64_t *kf_first, const uint64_t *kf_mid, const uint64_t *kf_last);
+
+/* Seeded transciphering keys: every LUT encrypted, masks expanded from a public seed.
+ *   WARNING: the generators above write the middle and last LUTs as trivial GLWE, as the reference does: zero mask, keyed
+ *   table in the body, so the top bit of body coefficient i of a LUT is its table bit and anyone holding the key reads the
+ *   round keys rk1..rk10 - and from any one of them the AES key.  The seeded keys below encrypt every LUT.
+ *   Layout.  GLWE g counts through the direction's AllRdKeys order: first-round LUTs [nmult][16][2], middle [8][nmult][16][2],
+ *   last [16][2]; nmult = 4 for the inverse (ECB) key, 3 for the forward (CTR) key: G = 1184 / 896 GLWE.  A seeded key is
+ *   mask_seed (32 bytes) + bodies[G][1024] u64 (CBS_TRANS_KEY_SEEDED_WORDS / CBS_FWD_TRANS_KEY_SEEDED_WORDS words, 9.7 / 7.3 MB
+ *   against 29.1 / 22.0 MB for the full key).  Mask word w (0..2047) of GLWE g is the RFC 8439 ChaCha20 block with key =
+ *   mask_seed as 8 little-endian u32, counter = w / 8, nonce = (g, dir, 0x6b73616d "mask"), dir = 0 inverse / 1 forward:
+ *   the u64 out[2i] | out[2i+1] << 32, i = w % 8, after the feed-forward.  Expanded GLWE g = [mask(g)][bodies[g]], word for word
+ *   the AllRdKeys layout, so an expanded key goes to every call that takes k10_9/k8_1/k0 (or kf_*).
+ *   Security rests on ChaCha20 as a PRF, as tfhe-rs's seeded ciphertexts rest on their CSPRNG.
+ *   *_seeded_generate: the same keyed tables as cbs_trans_key_generate / cbs_fwd_trans_key_generate, every LUT a fresh
+ *   encryption body = sum mask_c * S_c + e + pt with the noise from the secret stream; the mask seed is an output: from
+ *   getrandom(2), apart from the noise key (_os_entropy), or derived from `seed` (deterministic test variant, NOT secure).
+ *   *_seeded_expand: the host form of the device expansion: mask_seed + bodies -> the three AllRdKeys arrays.
+ *   *_seeded_save / _load: "CBSSEED1", u64 direction, the 32-byte seed, u64 word count, the bodies (56 + 8192 G bytes); load
+ *   returns CBS_ERR_FORMAT for another magic, the other direction, another count, a truncated file or trailing bytes.
+ *   Null arguments return CBS_ERR_ARG (load: CBS_ERR_IO). */
+#define CBS_SEED_BYTES                 32u
+#define CBS_TRANS_KEY_SEEDED_WORDS     (1184u * 1024u)
+#define CBS_FWD_TRANS_KEY_SEEDED_WORDS (896u * 1024u)
+int cbs_trans_key_seeded_generate(const cbs_keyset *ks, const uint8_t aes_key[16], uint64_t seed, uint8_t mask_seed_out[32],
+                                  uint64_t *bodies);
+int cbs_trans_key_seeded_generate_os_entropy(const cbs_keyset *ks, const uint8_t aes_key[16], uint8_t mask_seed_out[32],
+                                             uint64_t *bodies);
+int cbs_fwd_trans_key_seeded_generate(const cbs_keyset *ks, const uint8_t aes_key[16], uint64_t seed, uint8_t mask_seed_out[32],
+                                      uint64_t *bodies);
+int cbs_fwd_trans_key_seeded_generate_os_entropy(const cbs_keyset *ks, const uint8_t aes_key[16], uint8_t mask_seed_out[32],
+                                                 uint64_t *bodies);
+int cbs_trans_key_seeded_expand(const uint8_t mask_seed[32], const uint64_t *bodies, uint64_t *k10_9, uint64_t *k8_1, uint64_t *k0);
+int cbs_fwd_trans_key_seeded_expand(const uint8_t mask_seed[32], const uint64_t *bodies, uint64_t *kf_first, uint64_t *kf_mid,
+                                    uint64_t *kf_last);
+int cbs_trans_key_seeded_save(const char *path, const uint8_t mask_seed[32], const uint64_t *bodies);
+int cbs_trans_key_seeded_load(const char *path, uint8_t mask_seed[32], uint64_t *bodies);
+int cbs_fwd_trans_key_seeded_save(const char *path, const uint8_t mask_seed[32], const uint64_t *bodies);
+int cbs_fwd_trans_key_seeded_load(const char *path, uint8_t mask_seed[32], uint64_t *bodies);
+
 /* LweCiphertextList<Vec<u64>> result.bin */
 int cbs_lwe_list_load(const char *path, uint64_t **data /* malloc'd, free with cbs_free */, uint64_t *count,
                       uint64_t *lwe_words);
@@ -227,6 +266,12 @@ int cbs_aes128_transcipher_dev(cbs_ctx *ctx, const uint8_t *d_ct, int nblocks, u
 int cbs_fwd_trans_key_upload(cbs_ctx *ctx, const uint64_t *kf_first, const uint64_t *kf_mid, const uint64_t *kf_last);
 /* d_ctr = the nblocks counter blocks (16 bytes each), d_ct = the AES-CTR ciphertext bytes */
 int cbs_aes128_ctr_transcipher_dev(cbs_ctx *ctx, const uint8_t *d_ctr, const uint8_t *d_ct, int nblocks, uint64_t *d_out);
+/* Seeded keys (above) -> the device: the bodies are copied into the LUT buffers and the masks expanded there from the seed
+ * (k_expand_lut_masks), so only the 9.7 / 7.3 MB of bodies cross the bus; the device key is then word for word the
+ * *_seeded_expand arrays, and the *_transcipher_dev calls run with it unchanged.  Synchronous like cbs_trans_key_upload (the
+ * host buffers are free on return); a later upload of either form of the same direction replaces it. */
+int cbs_trans_key_seeded_upload(cbs_ctx *ctx, const uint8_t mask_seed[32], const uint64_t *bodies);
+int cbs_fwd_trans_key_seeded_upload(cbs_ctx *ctx, const uint8_t mask_seed[32], const uint64_t *bodies);
 
 /* Stage 8 on device buffers: the same computations and results as cbs_max_u16, cbs_max_u16_lut, cbs_sum_u16 and
  * cbs_inner_product_u16, bit for bit.

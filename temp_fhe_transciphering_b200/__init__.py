@@ -32,6 +32,8 @@ K0_WORDS = 16 * 2 * 3072
 KF_FIRST_WORDS = 3 * 16 * 2 * 3072
 KF_MID_WORDS = 8 * 3 * 16 * 2 * 3072
 KF_LAST_WORDS = 16 * 2 * 3072
+TRANS_KEY_SEEDED_GLWES = 1184  # seeded keys: one 1024-word body per LUT GLWE, AllRdKeys order (include/cbs_b200.h)
+FWD_TRANS_KEY_SEEDED_GLWES = 896
 
 
 class CbsError(RuntimeError):
@@ -205,6 +207,26 @@ class KeySet:
         _check(lib().cbs_fwd_trans_key_generate(self._h, pk, ctypes.c_uint64(seed), p1, p2, p3), "cbs_fwd_trans_key_generate")
         return a, b, c
 
+    def gen_seeded_transciphering_keys(self, aes_key, seed=None):
+        """The transciphering key with EVERY LUT encrypted, in seeded form -> (mask_seed: 32 bytes, bodies [1184][1024]).
+        gen_transciphering_keys writes rounds 8..0 as trivial LUTs whose bodies show the round keys; this one does not.
+        seed = None: noise key and mask seed from getrandom(2); an integer: the deterministic, not secure test generator."""
+        return self._gen_seeded("cbs_trans_key_seeded_generate", TRANS_KEY_SEEDED_GLWES, aes_key, seed)
+
+    def gen_seeded_forward_transciphering_keys(self, aes_key, seed=None):
+        """The forward (CTR) twin of gen_seeded_transciphering_keys -> (mask_seed, bodies [896][1024])."""
+        return self._gen_seeded("cbs_fwd_trans_key_seeded_generate", FWD_TRANS_KEY_SEEDED_GLWES, aes_key, seed)
+
+    def _gen_seeded(self, fn, nglwe, aes_key, seed):
+        bodies, pb = _out((nglwe, 1024))
+        ms = (ctypes.c_uint8 * 32)()
+        _, pk = _u8(aes_key)
+        if seed is None:
+            _check(getattr(lib(), fn + "_os_entropy")(self._h, pk, ms, pb), fn + "_os_entropy")
+        else:
+            _check(getattr(lib(), fn)(self._h, pk, ctypes.c_uint64(seed), ms, pb), fn)
+        return bytes(ms), bodies
+
     def encrypt_bits_big(self, bits, seed):
         bits = np.ascontiguousarray(bits, dtype=np.uint8)
         out, po = _out((bits.size, LWE_BIG))
@@ -249,6 +271,67 @@ def save_fwd_trans_key(path, kf_first, kf_mid, kf_last):
     b, p2 = _u64(kf_mid)
     c, p3 = _u64(kf_last)
     _check(lib().cbs_fwd_trans_key_save(str(path).encode(), p1, p2, p3), "cbs_fwd_trans_key_save")
+
+
+def _seed(mask_seed):
+    if len(mask_seed) != 32:
+        raise ValueError("a mask seed is 32 bytes")
+    return (ctypes.c_uint8 * 32).from_buffer_copy(bytes(mask_seed))
+
+
+def _bodies(bodies, nglwe):
+    b, pb = _u64(bodies)
+    if b.size != nglwe * 1024:
+        raise ValueError(f"seeded key bodies must hold {nglwe} x 1024 words, got {b.size}")
+    return b, pb
+
+
+def expand_seeded_trans_key(mask_seed, bodies):
+    """Seeded inverse key -> (k10_9, k8_1, k0) with the masks regenerated from mask_seed: the arrays every reference-format
+    call takes (upload_trans_key, aes_to_lwe_transciphering, save_trans_key)."""
+    a, p1 = _out((4, 16, 2, GLWE_WORDS))
+    b, p2 = _out((8, 4, 16, 2, GLWE_WORDS))
+    c, p3 = _out((16, 2, GLWE_WORDS))
+    _, pb = _bodies(bodies, TRANS_KEY_SEEDED_GLWES)
+    _check(lib().cbs_trans_key_seeded_expand(_seed(mask_seed), pb, p1, p2, p3), "cbs_trans_key_seeded_expand")
+    return a, b, c
+
+
+def expand_seeded_fwd_trans_key(mask_seed, bodies):
+    """Seeded forward key -> (kf_first, kf_mid, kf_last)."""
+    a, p1 = _out((3, 16, 2, GLWE_WORDS))
+    b, p2 = _out((8, 3, 16, 2, GLWE_WORDS))
+    c, p3 = _out((16, 2, GLWE_WORDS))
+    _, pb = _bodies(bodies, FWD_TRANS_KEY_SEEDED_GLWES)
+    _check(lib().cbs_fwd_trans_key_seeded_expand(_seed(mask_seed), pb, p1, p2, p3), "cbs_fwd_trans_key_seeded_expand")
+    return a, b, c
+
+
+def _load_seeded(fn, nglwe, path):
+    bodies, pb = _out((nglwe, 1024))
+    ms = (ctypes.c_uint8 * 32)()
+    _check(getattr(lib(), fn)(str(path).encode(), ms, pb), fn)
+    return bytes(ms), bodies
+
+
+def load_seeded_trans_key(path):
+    """seeded inverse key file ("CBSSEED1") -> (mask_seed, bodies [1184][1024])."""
+    return _load_seeded("cbs_trans_key_seeded_load", TRANS_KEY_SEEDED_GLWES, path)
+
+
+def save_seeded_trans_key(path, mask_seed, bodies):
+    _, pb = _bodies(bodies, TRANS_KEY_SEEDED_GLWES)
+    _check(lib().cbs_trans_key_seeded_save(str(path).encode(), _seed(mask_seed), pb), "cbs_trans_key_seeded_save")
+
+
+def load_seeded_fwd_trans_key(path):
+    """seeded forward key file -> (mask_seed, bodies [896][1024])."""
+    return _load_seeded("cbs_fwd_trans_key_seeded_load", FWD_TRANS_KEY_SEEDED_GLWES, path)
+
+
+def save_seeded_fwd_trans_key(path, mask_seed, bodies):
+    _, pb = _bodies(bodies, FWD_TRANS_KEY_SEEDED_GLWES)
+    _check(lib().cbs_fwd_trans_key_seeded_save(str(path).encode(), _seed(mask_seed), pb), "cbs_fwd_trans_key_seeded_save")
 
 
 def load_lwe_list(path):
@@ -495,6 +578,16 @@ class Context:
         """forward-direction (CTR) transciphering key -> device, once; then ctr_transcipher_dev can be called repeatedly."""
         (a, pa), (b, pb), (c, pc) = _u64(kf_first), _u64(kf_mid), _u64(kf_last)
         _check(lib().cbs_fwd_trans_key_upload(self._h, pa, pb, pc), "cbs_fwd_trans_key_upload")
+
+    def upload_seeded_trans_key(self, mask_seed, bodies):
+        """seeded inverse key -> device: the bodies are copied, the masks expanded on the GPU (k_expand_lut_masks)."""
+        _, pb = _bodies(bodies, TRANS_KEY_SEEDED_GLWES)
+        _check(lib().cbs_trans_key_seeded_upload(self._h, _seed(mask_seed), pb), "cbs_trans_key_seeded_upload")
+
+    def upload_seeded_fwd_trans_key(self, mask_seed, bodies):
+        """seeded forward (CTR) key -> device, as upload_seeded_trans_key."""
+        _, pb = _bodies(bodies, FWD_TRANS_KEY_SEEDED_GLWES)
+        _check(lib().cbs_fwd_trans_key_seeded_upload(self._h, _seed(mask_seed), pb), "cbs_fwd_trans_key_seeded_upload")
 
     def ctr_transcipher_dev(self, d_ctr_ptr, d_ct_ptr, nblocks, d_out_ptr):
         """device-resident CTR transciphering: d_ctr = the public 16-byte counter blocks, d_ct = the AES-CTR ciphertext."""

@@ -370,7 +370,7 @@ int dev_aes(cbs_ctx *ctx, AesDir dir, const uint8_t *d_in, const uint8_t *d_ct, 
 // compute stream; the middle and last LUTs, first read by the ladders of the first middle round (one keyswitch + blind rotation,
 // >= 2.4 ms, into the call), go with the check on the copy stream, and ev_keys marks their end.  The caller then sets
 // keys_in_flight for dev_aes_part and orders the compute stream after ev_keys before it releases the host buffers.
-int aes_key_upload(cbs_ctx *ctx, AesDir dir, const uint64_t *first, const uint64_t *mid, const uint64_t *last, bool overlap)
+int aes_key_alloc(cbs_ctx *ctx, AesDir dir)
 {
     const cbs_host::AesDirDesc &d = kAesDirs[dir];
     cbs_ctx::AesKeys &key = ctx->aes[dir];
@@ -378,6 +378,26 @@ int aes_key_upload(cbs_ctx *ctx, AesDir dir, const uint64_t *first, const uint64
     if (!key.first) CUDA_TRY(cudaMalloc(&key.first, (size_t)d.first_words * 8));
     if (!key.mid) CUDA_TRY(cudaMalloc(&key.mid, (size_t)d.mid_words * 8));
     if (!key.last) CUDA_TRY(cudaMalloc(&key.last, (size_t)d.last_words * 8));
+    return CBS_OK;
+}
+
+// the device flag of direction `dir`: 1 if a mask word of its middle or last LUTs is non-zero, queued on `cs`
+int aes_key_check_masks(cbs_ctx *ctx, AesDir dir, cudaStream_t cs)
+{
+    const cbs_host::AesDirDesc &d = kAesDirs[dir];
+    const cbs_ctx::AesKeys &key = ctx->aes[dir];
+    int *flag = ctx->d_masks_nonzero + dir;
+    CUDA_TRY(cudaMemsetAsync(flag, 0, sizeof(int), cs));
+    launch_masks_nonzero(key.mid, 8 * d.nmult * 16 * 2, flag, cs);
+    launch_masks_nonzero(key.last, 16 * 2, flag, cs);
+    return CBS_OK;
+}
+
+int aes_key_upload(cbs_ctx *ctx, AesDir dir, const uint64_t *first, const uint64_t *mid, const uint64_t *last, bool overlap)
+{
+    const cbs_host::AesDirDesc &d = kAesDirs[dir];
+    cbs_ctx::AesKeys &key = ctx->aes[dir];
+    TRY(aes_key_alloc(ctx, dir));
     cudaStream_t cs = ctx->stream;
     if (overlap) {
         if (!ctx->copy_stream) {
@@ -390,15 +410,40 @@ int aes_key_upload(cbs_ctx *ctx, AesDir dir, const uint64_t *first, const uint64
         CUDA_TRY(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_copy_after, 0));
         cs = ctx->copy_stream;
     }
-    int *flag = ctx->d_masks_nonzero + dir;
     CUDA_TRY(cudaMemcpyAsync(key.mid, mid, (size_t)d.mid_words * 8, cudaMemcpyHostToDevice, cs));
     CUDA_TRY(cudaMemcpyAsync(key.last, last, (size_t)d.last_words * 8, cudaMemcpyHostToDevice, cs));
-    CUDA_TRY(cudaMemsetAsync(flag, 0, sizeof(int), cs));
-    launch_masks_nonzero(key.mid, 8 * d.nmult * 16 * 2, flag, cs);
-    launch_masks_nonzero(key.last, 16 * 2, flag, cs);
+    TRY(aes_key_check_masks(ctx, dir, cs));
     if (overlap) CUDA_TRY(cudaEventRecord(ctx->ev_keys, cs));
     TRY(upload(ctx, key.first, first, (size_t)d.first_words * 8));
     if (!overlap) CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    key.uploaded = true;
+    return CBS_OK;
+}
+
+// Seeded key (include/cbs_b200.h) of direction `dir`: the bodies go into words 2048..3071 of every LUT GLWE (three strided
+// copies, one per key buffer), k_expand_lut_masks writes words 0..2047, and the same mask check as aes_key_upload follows (the
+// expanded masks are not zero, so the LUT ladders run their full first CMux).  On the compute stream, synchronised.
+int aes_key_seeded_upload(cbs_ctx *ctx, AesDir dir, const uint8_t mask_seed[32], const uint64_t *bodies)
+{
+    const cbs_host::AesDirDesc &d = kAesDirs[dir];
+    cbs_ctx::AesKeys &key = ctx->aes[dir];
+    TRY(aes_key_alloc(ctx, dir));
+    uint64_t *const dst[3] = {key.first, key.mid, key.last};
+    const uint32_t words[3] = {d.first_words, d.mid_words, d.last_words};
+    const uint64_t *src = bodies;
+    for (int i = 0; i < 3; i++) {
+        const size_t n = words[i] / kGlweWords;
+        CUDA_TRY(cudaMemcpy2DAsync(dst[i] + 2048, kGlweWords * 8, src, 1024 * 8, 1024 * 8, n, cudaMemcpyHostToDevice, ctx->stream));
+        src += n * 1024;
+    }
+    LutMaskSeed seed;
+    memcpy(seed.w, mask_seed, sizeof seed.w);
+    const int nfirst = d.first_words / kGlweWords, nglwe = (d.first_words + d.mid_words + d.last_words) / kGlweWords;
+    launch_expand_lut_masks(seed, dir, nfirst, nglwe, key.first, key.mid, key.last, ctx->stream);
+    ctx->launches++;
+    TRY(check_launch("k_expand_lut_masks"));
+    TRY(aes_key_check_masks(ctx, dir, ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     key.uploaded = true;
     return CBS_OK;
 }
@@ -932,6 +977,20 @@ int cbs_fwd_trans_key_upload(cbs_ctx *ctx, const uint64_t *kf_first, const uint6
     ENTER(ctx);
     if (!kf_first || !kf_mid || !kf_last) return set_error("cbs_fwd_trans_key_upload: null argument"), CBS_ERR_ARG;
     return aes_key_upload(ctx, kAesFwd, kf_first, kf_mid, kf_last, false);
+}
+
+int cbs_trans_key_seeded_upload(cbs_ctx *ctx, const uint8_t mask_seed[32], const uint64_t *bodies)
+{
+    ENTER(ctx);
+    if (!mask_seed || !bodies) return set_error("cbs_trans_key_seeded_upload: null argument"), CBS_ERR_ARG;
+    return aes_key_seeded_upload(ctx, kAesInv, mask_seed, bodies);
+}
+
+int cbs_fwd_trans_key_seeded_upload(cbs_ctx *ctx, const uint8_t mask_seed[32], const uint64_t *bodies)
+{
+    ENTER(ctx);
+    if (!mask_seed || !bodies) return set_error("cbs_fwd_trans_key_seeded_upload: null argument"), CBS_ERR_ARG;
+    return aes_key_seeded_upload(ctx, kAesFwd, mask_seed, bodies);
 }
 
 int cbs_aes128_ctr_transcipher_dev(cbs_ctx *ctx, const uint8_t *d_ctr, const uint8_t *d_ct, int nblocks, uint64_t *d_out)

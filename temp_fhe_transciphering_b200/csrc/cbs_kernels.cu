@@ -9,6 +9,7 @@
 // Groups synchronise with named barriers (bar.sync id, 64), never with __syncthreads, so the groups
 // of a CTA drift freely and hide each other's shared-memory and barrier latency.
 #include "cbs_kernels.cuh"
+#include "chacha20.h"
 #include "digits.cuh"
 #include "fft512.cuh"
 #include <algorithm>
@@ -2180,6 +2181,30 @@ void launch_masks_nonzero(const uint64_t *luts, int count, int *flag, cudaStream
 {
     if (count <= 0) return;
     k_masks_nonzero<<<count < 592 ? count : 592, 256, 0, s>>>(luts, count, flag);
+}
+
+// Mask polynomials of a seeded transciphering key (include/cbs_b200.h): CTA g = GLWE g of the direction's AllRdKeys order,
+// thread t = ChaCha20 block t of its mask (words 8t .. 8t + 7), written as four 16-byte stores.  The first nfirst GLWE go to
+// `first`, the next 8 nfirst to `mid`, the rest to `last`.
+__global__ void __launch_bounds__(256) k_expand_lut_masks(LutMaskSeed seed, uint32_t dir, int nfirst, uint64_t *__restrict__ first,
+                                                          uint64_t *__restrict__ mid, uint64_t *__restrict__ last)
+{
+    const int g = blockIdx.x, t = threadIdx.x;
+    uint64_t w[8];
+    cbs_chacha::mask_block(seed.w, dir, (uint32_t)g, (uint32_t)t, w);
+    uint64_t *glwe = g < nfirst ? first + (size_t)g * kGlweWords
+                     : g < 9 * nfirst ? mid + (size_t)(g - nfirst) * kGlweWords
+                                      : last + (size_t)(g - 9 * nfirst) * kGlweWords;
+    ulonglong2 *dst = reinterpret_cast<ulonglong2 *>(glwe + 8 * t);
+#pragma unroll
+    for (int i = 0; i < 4; i++) dst[i] = make_ulonglong2(w[2 * i], w[2 * i + 1]);
+}
+
+void launch_expand_lut_masks(const LutMaskSeed &seed, int dir, int nfirst, int nglwe, uint64_t *first, uint64_t *mid,
+                             uint64_t *last, cudaStream_t s)
+{
+    if (nglwe <= 0) return;
+    k_expand_lut_masks<<<nglwe, cbs_chacha::kMaskBlocksPerGlwe, 0, s>>>(seed, (uint32_t)dir, nfirst, first, mid, last);
 }
 
 int launch_lut8(const DeviceKeys &K, const double *ggsw_f, const uint64_t *luts, const int *lut_index,

@@ -70,6 +70,14 @@ int launch_lut8(const DeviceKeys &K, const double *ggsw_f, const uint64_t *luts,
                 const int *out_index, uint64_t *out, int njobs, int accs_per_byte, const int *masks_nonzero, cudaStream_t s);
 // *flag |= 1 if any mask word of the `count` GLWE accumulators at `luts` is non-zero (device-side "are these LUTs trivial?")
 void launch_masks_nonzero(const uint64_t *luts, int count, int *flag, cudaStream_t s);
+// mask polynomials (words 0..2047) of the nglwe LUT GLWE of a seeded transciphering key of direction dir from its 32-byte
+//     mask seed (chacha20.h mask_block): GLWE g < nfirst at first[g], then mid[g - nfirst], then last[g - 9 nfirst]; the body
+//     words are left as they are
+struct LutMaskSeed {
+    uint32_t w[8];  // the seed as 8 little-endian words
+};
+void launch_expand_lut_masks(const LutMaskSeed &seed, int dir, int nfirst, int nglwe, uint64_t *first, uint64_t *mid,
+                             uint64_t *last, cudaStream_t s);
 
 // a7 with gathered selectors (inner-product circuit): job j runs the ladder over the GGSWs ggsw_f[sel[j*8 + i]]
 //     (i = 0..7, -1 = constant-0 selector) on accumulator luts[lut_index[j]], 4 LWE(2048) out at out[out_index[j] + q]

@@ -22,11 +22,14 @@ struct AesDirDesc {
     uint8_t mults[4];                          // their values, in key (AllRdKeys tuple) order
     uint32_t first_words, mid_words, last_words;
     uint64_t seed_base;                        // first-round LUT `id` is encrypted with the Rng stream seed_base + id
+    uint64_t seeded_noise_base;                // seeded keys: the noise of LUT g comes from the Rng stream seeded_noise_base + g
 };
 inline constexpr AesDirDesc kAesDirs[2] = {
-    {4, {9, 11, 13, 14}, CBS_K10_9_WORDS, CBS_K8_1_WORDS, CBS_K0_WORDS, 9000},  // data_struct.rs:76-81
-    {3, {1, 2, 3, 0}, CBS_KF_FIRST_WORDS, CBS_KF_MID_WORDS, CBS_KF_LAST_WORDS, 11000},
+    {4, {9, 11, 13, 14}, CBS_K10_9_WORDS, CBS_K8_1_WORDS, CBS_K0_WORDS, 9000, 1ull << 40},  // data_struct.rs:76-81
+    {3, {1, 2, 3, 0}, CBS_KF_FIRST_WORDS, CBS_KF_MID_WORDS, CBS_KF_LAST_WORDS, 11000, (1ull << 40) + (1u << 20)},
 };
+// the seeded generators' deterministic test variant draws the mask seed from this stream of its seed
+inline constexpr uint64_t kMaskSeedStream = (1ull << 40) + (2u << 20);
 }  // namespace cbs_host
 
 // Host-side key material in the standard domain (flat layouts of include/cbs_b200.h).

@@ -8,6 +8,7 @@
 // cbs_lib/src/glwe_keyswitch.rs:183-218 (GLWE keyswitch key = GLEV of -S_in),
 // src/data_struct.rs:30-269 + src/aes_manager.rs:163-432 (AllRdKeys tables).
 #include "cbs_b200.h"
+#include "chacha20.h"
 #include "host_common.h"
 #include "ip_plan.h"
 
@@ -219,6 +220,18 @@ static double fourier_to_limb(const double *in, uint64_t *limb, double max_value
 //   * RngSource::os_entropy(): ChaCha20 (RFC 8439 block function) keyed with 256 bits from getrandom(2), stream id as
 //     nonce - what the stage executables use when no seed is given, like the reference's own client
 //     (client_key_generation.rs:91-96 new_seeder(); harness/run_submission.py:74-77: keys differ on every run).
+static bool os_random(void *dst, size_t bytes)
+{
+    size_t got = 0;
+    unsigned char *p = static_cast<unsigned char *>(dst);
+    while (got < bytes) {
+        ssize_t n = getrandom(p + got, bytes - got, 0);
+        if (n <= 0) return false;
+        got += (size_t)n;
+    }
+    return true;
+}
+
 struct RngSource {
     bool secure = false;
     uint64_t seed = 0;
@@ -227,14 +240,7 @@ struct RngSource {
     static bool os_entropy(RngSource &out)
     {
         out.secure = true;
-        size_t got = 0;
-        unsigned char *p = reinterpret_cast<unsigned char *>(out.key);
-        while (got < sizeof out.key) {
-            ssize_t n = getrandom(p + got, sizeof out.key - got, 0);
-            if (n <= 0) return false;
-            got += (size_t)n;
-        }
-        return true;
+        return os_random(out.key, sizeof out.key);
     }
 };
 
@@ -266,26 +272,11 @@ struct Rng {
         }
     }
     static uint64_t rotl(uint64_t x, int k) { return (x << k) | (x >> (64 - k)); }
-    static uint32_t rotl32(uint32_t x, int k) { return (x << k) | (x >> (32 - k)); }
     void chacha_block()
     {
         uint32_t x[16];
-        memcpy(x, cc, sizeof x);
-#define CBS_QR(a, b, c, d)                                                                       \
-    x[a] += x[b], x[d] = rotl32(x[d] ^ x[a], 16), x[c] += x[d], x[b] = rotl32(x[b] ^ x[c], 12), \
-        x[a] += x[b], x[d] = rotl32(x[d] ^ x[a], 8), x[c] += x[d], x[b] = rotl32(x[b] ^ x[c], 7)
-        for (int r = 0; r < 10; r++) {
-            CBS_QR(0, 4, 8, 12);
-            CBS_QR(1, 5, 9, 13);
-            CBS_QR(2, 6, 10, 14);
-            CBS_QR(3, 7, 11, 15);
-            CBS_QR(0, 5, 10, 15);
-            CBS_QR(1, 6, 11, 12);
-            CBS_QR(2, 7, 8, 13);
-            CBS_QR(3, 4, 9, 14);
-        }
-#undef CBS_QR
-        for (int i = 0; i < 8; i++) buf[i] = (uint64_t)(x[2 * i] + cc[2 * i]) | ((uint64_t)(x[2 * i + 1] + cc[2 * i + 1]) << 32);
+        cbs_chacha::block(cc, x);
+        for (int i = 0; i < 8; i++) buf[i] = (uint64_t)x[2 * i] | ((uint64_t)x[2 * i + 1] << 32);
         if (++cc[12] == 0) cc[15]++;  // 2^32 blocks of 64 bytes per (stream, cc[15]): far beyond any use here
         have = 8;
     }
@@ -327,11 +318,13 @@ static void add_mul_binary(uint64_t *body, const uint64_t *a, const uint64_t *s,
     }
 }
 
-// fresh GLWE encryption: ct = (a_0..a_{k-1}, sum a_c * s_c + e + pt)
+// fresh GLWE encryption: ct = (a_0..a_{k-1}, sum a_c * s_c + e + pt); the mask a is drawn from rng, or, with
+// mask_given, is what ct already holds (the seeded keys' public mask stream; the noise still comes from rng)
 static void glwe_encrypt(uint64_t *ct, const uint64_t *pt /*N or null*/, const uint64_t *sk, int k, int N, double std,
-                         Rng &rng)
+                         Rng &rng, bool mask_given = false)
 {
-    for (int i = 0; i < k * N; i++) ct[i] = rng.next();
+    if (!mask_given)
+        for (int i = 0; i < k * N; i++) ct[i] = rng.next();
     uint64_t *body = ct + (size_t)k * N;
     for (int j = 0; j < N; j++) body[j] = rng.noise(std) + (pt ? pt[j] : 0ull);
     for (int c = 0; c < k; c++) add_mul_binary(body, ct + (size_t)c * N, sk + (size_t)c * N, N);
@@ -448,10 +441,37 @@ static void lut_plaintext(uint64_t *pt, const uint8_t table[256], int acc_idx, u
 
 using namespace cbs_host;
 
+// The keyed tables of direction `dir` in AllRdKeys order: [0] the first round, [1 + i] middle block i, [9] the last round.
+// Inverse get_10_9_round_lut / get_round_lut / get_0_round_lut (aes_manager.rs:338-432), forward S(x ^ rk0) / S(x ^ rk_i) /
+// the last round (cbs_lib/src/aes_ref.rs:334-380).  Middle block i is keyed with round key i + 1.
+static void aes_key_tables(AesDir dir, const uint8_t aes_key[16], uint8_t tab[10][16][256])
+{
+    const bool inv = dir == kAesInv;
+    AesTables aes(aes_key);
+    inv ? aes.lut_10_9(tab[0]) : aes.lut_fwd(0, tab[0]);
+    for (int i = 0; i < 8; i++) inv ? aes.lut_round(i + 1, tab[1 + i]) : aes.lut_fwd(i + 1, tab[1 + i]);
+    inv ? aes.lut_round(0, tab[9]) : aes.lut_fwd_last(tab[9]);
+}
+
+// GLWE g of the direction's AllRdKeys order (first [nmult][16][2], middle [8][nmult][16][2], last [16][2], G GLWE in all): its
+// plaintext, and where it sits in the three key arrays
+static void aes_key_lut_plaintext(const AesDirDesc &d, const uint8_t tab[10][16][256], int g, uint64_t *pt)
+{
+    const int F = d.nmult * 32, round = g < F ? 0 : g < 9 * F ? 1 + (g - F) / F : 9;
+    const int id = round == 0 ? g : round < 9 ? (g - F) % F : g - 9 * F;
+    const int a = id & 1, b = (id >> 1) & 15, m = id >> 5;
+    lut_plaintext(pt, tab[round][b], a, round == 9 ? 0 : d.mults[m]);
+}
+template <typename P>
+static P aes_key_glwe(const AesDirDesc &d, int g, P first, P mid, P last)
+{
+    const int F = d.nmult * 32;
+    return g < F ? first + (size_t)g * 3072 : g < 9 * F ? mid + (size_t)(g - F) * 3072 : last + (size_t)(g - 9 * F) * 3072;
+}
+static int aes_key_nglwe(const AesDirDesc &d) { return d.nmult * 32 * 9 + 32; }
+
 // Transciphering key of direction `dir` (host_common.h kAesDirs): the first-round LUTs encrypted, one Rng stream per LUT; the
 // middle and last rounds as trivial GLWE (zero mask, the table in the body), as src/data_struct.rs:140-151,258-263 writes them.
-// Keyed tables: inverse get_10_9_round_lut / get_round_lut / get_0_round_lut (aes_manager.rs:338-432), forward
-// S(x ^ rk0) / S(x ^ rk_i) / the last round (cbs_lib/src/aes_ref.rs:334-380).  Middle block i is keyed with round key i + 1.
 static int aes_key_generate(AesDir dir, const char *fn, const cbs_keyset *ks, const uint8_t aes_key[16], const RngSource &src,
                             uint64_t *first, uint64_t *mid, uint64_t *last)
 {
@@ -460,30 +480,148 @@ static int aes_key_generate(AesDir dir, const char *fn, const cbs_keyset *ks, co
         return CBS_ERR_ARG;
     }
     const AesDirDesc &d = kAesDirs[dir];
-    const bool inv = dir == kAesInv;
-    AesTables aes(aes_key);
-    uint8_t tab[16][256];
-    inv ? aes.lut_10_9(tab) : aes.lut_fwd(0, tab);
+    uint8_t tab[10][16][256];
+    aes_key_tables(dir, aes_key, tab);
     const uint64_t *S = ks->glwe_sk.data();
-    parallel_for(d.nmult * 16 * 2, [&](int id) {
-        const int a = id & 1, b = (id >> 1) & 15, m = id >> 5;
+    const int F = d.nmult * 16 * 2;
+    parallel_for(F, [&](int id) {
         Rng rng(src, d.seed_base + (uint64_t)id);
         std::vector<uint64_t> pt(1024);
-        lut_plaintext(pt.data(), tab[b], a, d.mults[m]);
+        aes_key_lut_plaintext(d, tab, id, pt.data());
         glwe_encrypt(first + (size_t)id * 3072, pt.data(), S, 2, 1024, kStdGlwe, rng);
     });
     memset(mid, 0, sizeof(uint64_t) * d.mid_words);
-    for (int i = 0; i < 8; i++) {
-        inv ? aes.lut_round(i + 1, tab) : aes.lut_fwd(i + 1, tab);
-        for (int m = 0; m < d.nmult; m++)
-            for (int b = 0; b < 16; b++)
-                for (int a = 0; a < 2; a++)
-                    lut_plaintext(mid + ((((size_t)i * d.nmult + m) * 16 + b) * 2 + a) * 3072 + 2048, tab[b], a, d.mults[m]);
-    }
     memset(last, 0, sizeof(uint64_t) * d.last_words);
-    inv ? aes.lut_round(0, tab) : aes.lut_fwd_last(tab);
-    for (int b = 0; b < 16; b++)
-        for (int a = 0; a < 2; a++) lut_plaintext(last + ((size_t)b * 2 + a) * 3072 + 2048, tab[b], a, 0);
+    for (int g = F; g < aes_key_nglwe(d); g++) aes_key_lut_plaintext(d, tab, g, aes_key_glwe(d, g, first, mid, last) + 2048);
+    return CBS_OK;
+}
+
+// Seeded keys (include/cbs_b200.h): every LUT of the direction encrypted, its mask the public ChaCha20 stream of the mask seed
+// (chacha20.h), its noise from the secret stream seeded_noise_base + g of `src`.  The mask seed is `mask_seed` as given.
+static int aes_key_seeded_generate(AesDir dir, const char *fn, const cbs_keyset *ks, const uint8_t aes_key[16], const RngSource &src,
+                                   const uint8_t mask_seed[32], uint64_t *bodies)
+{
+    const AesDirDesc &d = kAesDirs[dir];
+    uint8_t tab[10][16][256];
+    aes_key_tables(dir, aes_key, tab);
+    uint32_t key[8];
+    memcpy(key, mask_seed, 32);
+    const uint64_t *S = ks->glwe_sk.data();
+    parallel_for(aes_key_nglwe(d), [&](int g) {
+        Rng rng(src, d.seeded_noise_base + (uint64_t)g);
+        std::vector<uint64_t> pt(1024), ct(3072);
+        aes_key_lut_plaintext(d, tab, g, pt.data());
+        for (int blk = 0; blk < cbs_chacha::kMaskBlocksPerGlwe; blk++) cbs_chacha::mask_block(key, dir, g, blk, ct.data() + 8 * blk);
+        glwe_encrypt(ct.data(), pt.data(), S, 2, 1024, kStdGlwe, rng, true);
+        memcpy(bodies + (size_t)g * 1024, ct.data() + 2048, 1024 * 8);
+    });
+    return CBS_OK;
+}
+
+static bool seeded_args_ok(const char *fn, const cbs_keyset *ks, const uint8_t *aes_key, const uint8_t *mask_seed_out,
+                           const uint64_t *bodies)
+{
+    if (!ks || ks->glwe_sk.empty() || !aes_key || !mask_seed_out || !bodies) {
+        set_error(std::string(fn) + ": needs a keyset with the GLWE secret key and non-null buffers");
+        return false;
+    }
+    return true;
+}
+
+// test variant: noise and mask seed both from the deterministic generator of `seed`, the seed on its own stream
+static int aes_key_seeded_generate_seed(AesDir dir, const char *fn, const cbs_keyset *ks, const uint8_t aes_key[16], uint64_t seed,
+                                        uint8_t mask_seed_out[32], uint64_t *bodies)
+{
+    if (!seeded_args_ok(fn, ks, aes_key, mask_seed_out, bodies)) return CBS_ERR_ARG;
+    const RngSource src(seed);
+    Rng rng(src, kMaskSeedStream);
+    for (int i = 0; i < 4; i++) {
+        const uint64_t w = rng.next();
+        memcpy(mask_seed_out + 8 * i, &w, 8);
+    }
+    return aes_key_seeded_generate(dir, fn, ks, aes_key, src, mask_seed_out, bodies);
+}
+
+// the noise key and the mask seed from two separate getrandom(2) draws
+static int aes_key_seeded_generate_os_entropy(AesDir dir, const char *fn, const cbs_keyset *ks, const uint8_t aes_key[16],
+                                              uint8_t mask_seed_out[32], uint64_t *bodies)
+{
+    if (!seeded_args_ok(fn, ks, aes_key, mask_seed_out, bodies)) return CBS_ERR_ARG;
+    RngSource src(0);
+    if (!RngSource::os_entropy(src) || !os_random(mask_seed_out, 32)) {
+        set_error("getrandom failed");
+        return CBS_ERR_IO;
+    }
+    return aes_key_seeded_generate(dir, fn, ks, aes_key, src, mask_seed_out, bodies);
+}
+
+// host restatement of k_expand_lut_masks: the seeded key as the direction's three AllRdKeys arrays
+static int aes_key_seeded_expand(AesDir dir, const char *fn, const uint8_t mask_seed[32], const uint64_t *bodies, uint64_t *first,
+                                 uint64_t *mid, uint64_t *last)
+{
+    if (!mask_seed || !bodies || !first || !mid || !last) {
+        set_error(std::string(fn) + ": null argument");
+        return CBS_ERR_ARG;
+    }
+    const AesDirDesc &d = kAesDirs[dir];
+    uint32_t key[8];
+    memcpy(key, mask_seed, 32);
+    parallel_for(aes_key_nglwe(d), [&](int g) {
+        uint64_t *ct = aes_key_glwe(d, g, first, mid, last);
+        for (int blk = 0; blk < cbs_chacha::kMaskBlocksPerGlwe; blk++) cbs_chacha::mask_block(key, dir, g, blk, ct + 8 * blk);
+        memcpy(ct + 2048, bodies + (size_t)g * 1024, 1024 * 8);
+    });
+    return CBS_OK;
+}
+
+// "CBSSEED1", u64 direction, the 32-byte mask seed, u64 body word count, the bodies
+static const char kSeededMagic[8] = {'C', 'B', 'S', 'S', 'E', 'E', 'D', '1'};
+
+static int aes_key_seeded_save(AesDir dir, const char *fn, const char *path, const uint8_t mask_seed[32], const uint64_t *bodies)
+{
+    if (!path || !mask_seed || !bodies) {
+        set_error(std::string(fn) + ": null argument");
+        return CBS_ERR_ARG;
+    }
+    const uint64_t words = (uint64_t)aes_key_nglwe(kAesDirs[dir]) * 1024;
+    Writer w;
+    w.buf.reserve(56 + 8 * words);
+    w.buf.insert(w.buf.end(), kSeededMagic, kSeededMagic + 8);
+    w.u64((uint64_t)dir);
+    w.buf.insert(w.buf.end(), mask_seed, mask_seed + 32);
+    w.vec(bodies, words);
+    std::string p(path);
+    size_t slash = p.find_last_of('/');
+    if (slash != std::string::npos) mkdirs(p.substr(0, slash));
+    if (!w.save(p)) {
+        set_error("cannot write " + p);
+        return CBS_ERR_IO;
+    }
+    return CBS_OK;
+}
+
+static int aes_key_seeded_load(AesDir dir, const char *path, uint8_t mask_seed[32], uint64_t *bodies)
+{
+    Reader r;
+    if (!path || !mask_seed || !bodies || !r.load(path)) {
+        set_error(std::string("cannot read ") + (path ? path : "(null)"));
+        return CBS_ERR_IO;
+    }
+    const uint64_t words = (uint64_t)aes_key_nglwe(kAesDirs[dir]) * 1024;
+    bool ok = r.buf.size() == 56 + 8 * words && memcmp(r.buf.data(), kSeededMagic, 8) == 0;
+    if (ok) {
+        r.off = 8;
+        ok = r.u64() == (uint64_t)dir;
+        r.off = 48;
+        ok = ok && r.u64() == words;
+    }
+    if (!ok) {
+        set_error(std::string(path) + (dir == kAesInv ? ": not a seeded inverse (ECB) transciphering key"
+                                                      : ": not a seeded forward (CTR) transciphering key"));
+        return CBS_ERR_FORMAT;
+    }
+    memcpy(mask_seed, r.buf.data() + 16, 32);
+    memcpy(bodies, r.buf.data() + 56, 8 * words);
     return CBS_OK;
 }
 
@@ -940,6 +1078,61 @@ int cbs_fwd_trans_key_save(const char *path, const uint64_t *kf_first, const uin
 int cbs_fwd_trans_key_load(const char *path, uint64_t *kf_first, uint64_t *kf_mid, uint64_t *kf_last)
 {
     return aes_key_load(kAesFwd, "not a forward (CTR) transciphering key for AES_TIGHT", path, kf_first, kf_mid, kf_last);
+}
+
+int cbs_trans_key_seeded_generate(const cbs_keyset *ks, const uint8_t aes_key[16], uint64_t seed, uint8_t mask_seed_out[32],
+                                  uint64_t *bodies)
+{
+    return aes_key_seeded_generate_seed(kAesInv, "cbs_trans_key_seeded_generate", ks, aes_key, seed, mask_seed_out, bodies);
+}
+
+int cbs_trans_key_seeded_generate_os_entropy(const cbs_keyset *ks, const uint8_t aes_key[16], uint8_t mask_seed_out[32],
+                                             uint64_t *bodies)
+{
+    return aes_key_seeded_generate_os_entropy(kAesInv, "cbs_trans_key_seeded_generate", ks, aes_key, mask_seed_out, bodies);
+}
+
+int cbs_fwd_trans_key_seeded_generate(const cbs_keyset *ks, const uint8_t aes_key[16], uint64_t seed, uint8_t mask_seed_out[32],
+                                      uint64_t *bodies)
+{
+    return aes_key_seeded_generate_seed(kAesFwd, "cbs_fwd_trans_key_seeded_generate", ks, aes_key, seed, mask_seed_out, bodies);
+}
+
+int cbs_fwd_trans_key_seeded_generate_os_entropy(const cbs_keyset *ks, const uint8_t aes_key[16], uint8_t mask_seed_out[32],
+                                                 uint64_t *bodies)
+{
+    return aes_key_seeded_generate_os_entropy(kAesFwd, "cbs_fwd_trans_key_seeded_generate", ks, aes_key, mask_seed_out, bodies);
+}
+
+int cbs_trans_key_seeded_expand(const uint8_t mask_seed[32], const uint64_t *bodies, uint64_t *k10_9, uint64_t *k8_1, uint64_t *k0)
+{
+    return aes_key_seeded_expand(kAesInv, "cbs_trans_key_seeded_expand", mask_seed, bodies, k10_9, k8_1, k0);
+}
+
+int cbs_fwd_trans_key_seeded_expand(const uint8_t mask_seed[32], const uint64_t *bodies, uint64_t *kf_first, uint64_t *kf_mid,
+                                    uint64_t *kf_last)
+{
+    return aes_key_seeded_expand(kAesFwd, "cbs_fwd_trans_key_seeded_expand", mask_seed, bodies, kf_first, kf_mid, kf_last);
+}
+
+int cbs_trans_key_seeded_save(const char *path, const uint8_t mask_seed[32], const uint64_t *bodies)
+{
+    return aes_key_seeded_save(kAesInv, "cbs_trans_key_seeded_save", path, mask_seed, bodies);
+}
+
+int cbs_trans_key_seeded_load(const char *path, uint8_t mask_seed[32], uint64_t *bodies)
+{
+    return aes_key_seeded_load(kAesInv, path, mask_seed, bodies);
+}
+
+int cbs_fwd_trans_key_seeded_save(const char *path, const uint8_t mask_seed[32], const uint64_t *bodies)
+{
+    return aes_key_seeded_save(kAesFwd, "cbs_fwd_trans_key_seeded_save", path, mask_seed, bodies);
+}
+
+int cbs_fwd_trans_key_seeded_load(const char *path, uint8_t mask_seed[32], uint64_t *bodies)
+{
+    return aes_key_seeded_load(kAesFwd, path, mask_seed, bodies);
 }
 
 int cbs_lwe_list_load(const char *path, uint64_t **data, uint64_t *count, uint64_t *lwe_words)
