@@ -11,6 +11,7 @@ CUDA-event times, max over ranks, and rank 0 prints.
   torchrun --nproc_per_node 8 bench_sweep.py --config5 1024 --config5-dev 1024   # configs[4], host-buffer and HBM-resident
   python bench_sweep.py --pack 8 64 1024     # LWE-to-GLWE packing of the CTR transcipher output (1 GPU)
   python bench_sweep.py --seeded-keys 8 64   # seeded transciphering keys against reference-format keys (1 GPU)
+  python bench_sweep.py --slots 64x1 16x4 8x8   # S senders x b blocks, each with its own AES key: per-sender calls vs key slots
 Each CBS point = LWE keyswitch-free circuit bootstrap (blind rotation -> GLEV extraction + trace ->
 scheme switch to a Fourier GGSW), inputs resident in HBM, CUDA events on the launching stream, 3
 warm-up + 5 timed launches; the first batch sizes are verified by decrypting the GGSW rows.
@@ -46,6 +47,10 @@ def main():
     ap.add_argument("--seeded-keys", type=int, nargs="*", default=None, metavar="BLOCKS",
                     help="seeded transciphering keys only: bytes, upload time and ECB / CTR blocks/s at BLOCKS (default 8 64) "
                          "with the seeded key against the reference-format key, both forms alternating in one process (1 GPU)")
+    ap.add_argument("--slots", nargs="*", default=None, metavar="SxB",
+                    help="key slots only: S senders with B blocks each (default 64x1 16x4 8x8), distinct AES keys and seeded "
+                         "keys; route A uploads each sender's key and transciphers its blocks alone, route B transciphers all "
+                         "S*B blocks in one call over resident key slots; ECB and CTR blocks/s, verified (1 GPU)")
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     import numpy as np
@@ -117,6 +122,12 @@ def main():
     if args.seeded_keys is not None:
         assert world == 1, "--seeded-keys runs on one GPU"
         seeded_keys_bench(args.seeded_keys or [8, 64], ks, ctx, stream, local, emit)
+        args.aes_only = args.cbs_only = True  # nothing else
+        args.aes_blocks = []
+    if args.slots is not None:
+        assert world == 1, "--slots runs on one GPU"
+        shapes = [tuple(int(x) for x in v.lower().split("x")) for v in (args.slots or ["64x1", "16x4", "8x8"])]
+        slots_bench(shapes, ks, ctx, stream, local, emit)
         args.aes_only = args.cbs_only = True  # nothing else
         args.aes_blocks = []
     if args.config5:
@@ -463,6 +474,106 @@ def seeded_keys_bench(blocks, ks, ctx, stream, local, emit):
                   "seeded_rows_equal_host_expanded": same, "blocks_wrong_reference_format": wrong["full"],
                   "blocks_wrong_seeded": wrong["seeded"], "verified": bool(same and not wrong["full"] and not wrong["seeded"]),
                   "card": card, "n_gpus": 1})
+
+
+def slots_bench(shapes, ks, ctx, stream, local, emit):
+    """Many senders, each with its own AES key, for (S senders, b blocks each) in `shapes`, per direction:
+      * route A, what one key per context allows: for every sender, cbs_*trans_key_seeded_upload of its key, then the _dev
+        call on its b blocks;
+      * route B: the S seeded keys uploaded into key slots once (timed on their own: the mean per slot upload), then one
+        cbs_aes128_*transcipher_slots_dev call over all S*b blocks, the senders interleaved (block k*S + s is sender s's k-th);
+      * blocks/s from CUDA events around each route, ending in a device synchronise: 1 warm-up pass, then the mean of 3 passes,
+        the routes alternating;
+      * verification in the same run: every block of both routes decrypts to its sender's plaintext, and whether the two
+        routes' rows are bit-identical (route A's parts of one or two blocks take the team blind-rotation kernel by default,
+        route B's the v4 kernel; the line records CBS_BR_LOWLAT).
+    The card's name, power limit and max SM clock are read in the same run."""
+    import numpy as np
+    import torch
+    import aes_clear
+    import ref_io
+    card = card_info(local)
+    lowlat = os.environ.get("CBS_BR_LOWLAT", "1")
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+
+    def events_ms(fn):
+        torch.cuda.synchronize()
+        e0.record(stream)
+        fn()
+        e1.record(stream)
+        torch.cuda.synchronize()
+        return e0.elapsed_time(e1)
+
+    def dev(b):
+        return torch.frombuffer(bytearray(b), dtype=torch.uint8).cuda()
+
+    def counters(iv, n):
+        return b"".join(((int.from_bytes(iv, "big") + k) % (1 << 128)).to_bytes(16, "big") for k in range(n))
+
+    nsend = max(S for S, _ in shapes)
+    aes_keys = [aes_clear.harness_aes_key(f"sender-{s}") for s in range(nsend)]
+    ivs = [aes_clear.harness_iv(f"sender-{s}") for s in range(nsend)]
+    for mode in ("ecb", "ctr"):
+        gen = ks.gen_seeded_transciphering_keys if mode == "ecb" else ks.gen_seeded_forward_transciphering_keys
+        keys = [gen(aes_keys[s], 7000 + s) for s in range(nsend)]
+        if mode == "ecb":
+            ctx.reserve_trans_key_slots(nsend)
+            up_single, up_slot = ctx.upload_seeded_trans_key, ctx.upload_seeded_trans_key_slot
+        else:
+            ctx.reserve_fwd_trans_key_slots(nsend)
+            up_single, up_slot = ctx.upload_seeded_fwd_trans_key, ctx.upload_seeded_fwd_trans_key_slot
+        for S, b in shapes:
+            nb = S * b
+            order = [(s, k) for k in range(b) for s in range(S)]  # route B block i = sender order[i][0]'s block order[i][1]
+            pts = [bytes(np.random.default_rng([S, b, s]).integers(0, 256, 16 * b, dtype=np.uint8)) for s in range(S)]
+            if mode == "ecb":
+                ins = [(dev(aes_clear.ecb_encrypt(aes_keys[s], pts[s])),) for s in range(S)]
+            else:
+                ins = [(dev(counters(ivs[s], b)), dev(aes_clear.ctr_crypt(aes_keys[s], ivs[s], pts[s]))) for s in range(S)]
+            # route B's interleaved inputs, gathered from the senders' device buffers
+            d_inter = [torch.stack([ins[s][j].view(b, 16)[k] for s, k in order]).reshape(-1) for j in range(len(ins[0]))]
+            slots = np.array([s for s, _ in order], dtype=np.int32)
+            out_a = torch.empty((S, b, 128, 2049), dtype=torch.int64, device="cuda")
+            out_b = torch.empty((nb, 128, 2049), dtype=torch.int64, device="cuda")
+
+            def route_a():
+                for s in range(S):
+                    up_single(*keys[s])
+                    if mode == "ecb":
+                        ctx.transcipher_dev(ins[s][0].data_ptr(), b, out_a[s].data_ptr())
+                    else:
+                        ctx.ctr_transcipher_dev(ins[s][0].data_ptr(), ins[s][1].data_ptr(), b, out_a[s].data_ptr())
+
+            def route_b():
+                if mode == "ecb":
+                    ctx.transcipher_slots_dev(d_inter[0].data_ptr(), slots, nb, out_b.data_ptr())
+                else:
+                    ctx.ctr_transcipher_slots_dev(d_inter[0].data_ptr(), d_inter[1].data_ptr(), slots, nb, out_b.data_ptr())
+
+            t_up = events_ms(lambda: [up_slot(s, *keys[s]) for s in range(S)]) / S
+            ms = {"a": [], "b": []}
+            for rep in range(4):
+                for name, fn in (("a", route_a), ("b", route_b)):
+                    t = events_ms(fn)
+                    if rep:
+                        ms[name].append(t)
+            rows_a = out_a.cpu().numpy().view(np.uint64)
+            rows_b = out_b.cpu().numpy().view(np.uint64)
+            # route B's rows back in sender order
+            back = np.empty_like(rows_a)
+            for i, (s, k) in enumerate(order):
+                back[s, k] = rows_b[i]
+            wrong = {}
+            for name, rows in (("a", rows_a), ("b", back)):
+                bits = ref_io.decode_bit(ref_io.lwe_phase(rows.reshape(-1, 2049), ks.glwe_sk)).reshape(S, b * 128)
+                wrong[name] = [s for s in range(S) if not np.array_equal(bits[s], np.unpackbits(np.frombuffer(pts[s], np.uint8)))]
+            same = bool(np.array_equal(rows_a, back))
+            ta, tb = float(np.mean(ms["a"])), float(np.mean(ms["b"]))
+            emit({"bench": "key_slots", "mode": mode, "senders": S, "blocks_per_sender": b, "blocks": nb,
+                  "route_a_ms": ta, "route_b_ms": tb, "route_a_blocks_per_s": nb / (ta * 1e-3),
+                  "route_b_blocks_per_s": nb / (tb * 1e-3), "slot_upload_ms": t_up,
+                  "senders_wrong_route_a": wrong["a"], "senders_wrong_route_b": wrong["b"], "rows_bit_identical": same,
+                  "cbs_br_lowlat": lowlat, "verified": not wrong["a"] and not wrong["b"], "card": card, "n_gpus": 1})
 
 
 def pack_bench(blocks, ks, ctx, stream, local, emit):

@@ -273,6 +273,38 @@ int cbs_aes128_ctr_transcipher_dev(cbs_ctx *ctx, const uint8_t *d_ctr, const uin
 int cbs_trans_key_seeded_upload(cbs_ctx *ctx, const uint8_t mask_seed[32], const uint64_t *bodies);
 int cbs_fwd_trans_key_seeded_upload(cbs_ctx *ctx, const uint8_t mask_seed[32], const uint64_t *bodies);
 
+/* Key slots: many transciphering keys resident at once (one per AES sender), and one call over blocks of many keys.
+ *   Each direction has a pool of slots; a slot holds one key in the expanded AllRdKeys layout (29.1 MB inverse, 22.0 MB
+ *   forward).  Every slot is under the context's one FHE keyset: slots separate AES senders, not FHE clients.
+ *   *_slots_reserve: the pool gets nslots contiguous slots.  A later reserve with a larger count grows it and keeps every
+ *   uploaded slot (device-to-device copy on the context's stream; the old buffers are freed stream-ordered).  The same count
+ *   does nothing; a smaller count or nslots <= 0 returns CBS_ERR_ARG; a failed allocation returns CBS_ERR_NOMEM and leaves
+ *   the pool as it was.
+ *   *_slot_upload / *_seeded_slot_upload: put a key of either form into a reserved slot (slot < 0 or >= the reserved count:
+ *   CBS_ERR_ARG), replacing what it held.  Synchronous like cbs_trans_key_upload, and ordered after earlier work of the
+ *   context that may still read the slot.  Slots and the single key of cbs_trans_key_upload and its twins are independent:
+ *   neither kind of upload changes what the other kind of call computes.
+ *   *_transcipher_slots_dev: block b is transciphered under slot slots[b].  slots is a HOST array [nblocks]; d_ct (ECB), d_ctr
+ *   and d_ct (CTR) and d_out [nblocks][128] big LWE are as in the single-key _dev calls, and block b's rows are bit for bit
+ *   the rows the single-key call gives for that block under that key.  The slot array is checked before anything is queued:
+ *   a slot < 0, >= the reserved count, or never uploaded in the call's direction, nblocks <= 0 or a null pointer returns
+ *   CBS_ERR_ARG.  Queued on the context's stream, never synchronises; the slot array is copied before the call returns, so
+ *   the queued work reads no host memory.
+ *   *_transcipher_slots: host buffers (ct, ctr = the nblocks counter blocks [nblocks][16], out [nblocks][128] big LWE);
+ *   synchronous: the inputs go up, the _dev call runs, the rows come down. */
+int cbs_trans_key_slots_reserve(cbs_ctx *ctx, int nslots);
+int cbs_fwd_trans_key_slots_reserve(cbs_ctx *ctx, int nslots);
+int cbs_trans_key_slot_upload(cbs_ctx *ctx, int slot, const uint64_t *k10_9, const uint64_t *k8_1, const uint64_t *k0);
+int cbs_fwd_trans_key_slot_upload(cbs_ctx *ctx, int slot, const uint64_t *kf_first, const uint64_t *kf_mid, const uint64_t *kf_last);
+int cbs_trans_key_seeded_slot_upload(cbs_ctx *ctx, int slot, const uint8_t mask_seed[32], const uint64_t *bodies);
+int cbs_fwd_trans_key_seeded_slot_upload(cbs_ctx *ctx, int slot, const uint8_t mask_seed[32], const uint64_t *bodies);
+int cbs_aes128_transcipher_slots_dev(cbs_ctx *ctx, const uint8_t *d_ct, const int32_t *slots, int nblocks, uint64_t *d_out);
+int cbs_aes128_ctr_transcipher_slots_dev(cbs_ctx *ctx, const uint8_t *d_ctr, const uint8_t *d_ct, const int32_t *slots,
+                                         int nblocks, uint64_t *d_out);
+int cbs_aes128_transcipher_slots(cbs_ctx *ctx, const uint8_t *ct, const int32_t *slots, int nblocks, uint64_t *out);
+int cbs_aes128_ctr_transcipher_slots(cbs_ctx *ctx, const uint8_t *ctr, const uint8_t *ct, const int32_t *slots, int nblocks,
+                                     uint64_t *out);
+
 /* Stage 8 on device buffers: the same computations and results as cbs_max_u16, cbs_max_u16_lut, cbs_sum_u16 and
  * cbs_inner_product_u16, bit for bit.
  *   Layout: d_in [nvals][16] big LWE (MSB first), d_out [16] big LWE.  The transcipher output [nblocks][128] big LWE is

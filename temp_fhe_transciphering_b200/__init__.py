@@ -113,6 +113,13 @@ def _u8(b):
     return a, a.ctypes.data_as(ctypes.POINTER(ctypes.c_uint8))
 
 
+def _slots(slots, nblocks):
+    a = np.ascontiguousarray(slots, dtype=np.int32).reshape(-1)
+    if a.size != nblocks:
+        raise ValueError(f"{a.size} slots for {nblocks} blocks")
+    return a, a.ctypes.data_as(ctypes.POINTER(ctypes.c_int32))
+
+
 class KeySet:
     """Host-side evaluation (and optionally secret) keys in the standard domain.
 
@@ -588,6 +595,67 @@ class Context:
         """seeded forward (CTR) key -> device, as upload_seeded_trans_key."""
         _, pb = _bodies(bodies, FWD_TRANS_KEY_SEEDED_GLWES)
         _check(lib().cbs_fwd_trans_key_seeded_upload(self._h, _seed(mask_seed), pb), "cbs_fwd_trans_key_seeded_upload")
+
+    # key slots: many transciphering keys resident at once, block b of a call under slot slots[b] (include/cbs_b200.h)
+    def reserve_trans_key_slots(self, nslots):
+        """grow the inverse (ECB) key pool to nslots slots (29.1 MB each); uploaded slots are kept."""
+        _check(lib().cbs_trans_key_slots_reserve(self._h, int(nslots)), "cbs_trans_key_slots_reserve")
+
+    def reserve_fwd_trans_key_slots(self, nslots):
+        """grow the forward (CTR) key pool to nslots slots (22.0 MB each)."""
+        _check(lib().cbs_fwd_trans_key_slots_reserve(self._h, int(nslots)), "cbs_fwd_trans_key_slots_reserve")
+
+    def upload_trans_key_slot(self, slot, k10_9, k8_1, k0):
+        (a, p1), (b, p2), (d, p3) = _u64(k10_9), _u64(k8_1), _u64(k0)
+        _check(lib().cbs_trans_key_slot_upload(self._h, int(slot), p1, p2, p3), "cbs_trans_key_slot_upload")
+
+    def upload_fwd_trans_key_slot(self, slot, kf_first, kf_mid, kf_last):
+        (a, p1), (b, p2), (d, p3) = _u64(kf_first), _u64(kf_mid), _u64(kf_last)
+        _check(lib().cbs_fwd_trans_key_slot_upload(self._h, int(slot), p1, p2, p3), "cbs_fwd_trans_key_slot_upload")
+
+    def upload_seeded_trans_key_slot(self, slot, mask_seed, bodies):
+        _, pb = _bodies(bodies, TRANS_KEY_SEEDED_GLWES)
+        _check(lib().cbs_trans_key_seeded_slot_upload(self._h, int(slot), _seed(mask_seed), pb), "cbs_trans_key_seeded_slot_upload")
+
+    def upload_seeded_fwd_trans_key_slot(self, slot, mask_seed, bodies):
+        _, pb = _bodies(bodies, FWD_TRANS_KEY_SEEDED_GLWES)
+        _check(lib().cbs_fwd_trans_key_seeded_slot_upload(self._h, int(slot), _seed(mask_seed), pb),
+               "cbs_fwd_trans_key_seeded_slot_upload")
+
+    def transcipher_slots_dev(self, d_ct_ptr, slots, nblocks, d_out_ptr):
+        """device-resident ECB transciphering, block b under key slot slots[b] (a host sequence of nblocks ints)."""
+        s, ps = _slots(slots, nblocks)
+        _check(lib().cbs_aes128_transcipher_slots_dev(self._h, ctypes.c_void_p(d_ct_ptr), ps, int(nblocks),
+                                                      ctypes.c_void_p(d_out_ptr)), "cbs_aes128_transcipher_slots_dev")
+
+    def ctr_transcipher_slots_dev(self, d_ctr_ptr, d_ct_ptr, slots, nblocks, d_out_ptr):
+        """device-resident CTR transciphering, block b under key slot slots[b]; d_ctr = the public counter blocks."""
+        s, ps = _slots(slots, nblocks)
+        _check(lib().cbs_aes128_ctr_transcipher_slots_dev(self._h, ctypes.c_void_p(d_ctr_ptr), ctypes.c_void_p(d_ct_ptr), ps,
+                                                          int(nblocks), ctypes.c_void_p(d_out_ptr)),
+               "cbs_aes128_ctr_transcipher_slots_dev")
+
+    def transcipher_slots(self, ct, slots):
+        """ECB ciphertext blocks, block b under slot slots[b] -> [nblocks][128][2049] (MSB first inside each byte)."""
+        c, pc = _u8(ct)
+        nblocks = c.size // 16
+        s, ps = _slots(slots, nblocks)
+        out, po = _out((nblocks, 128, LWE_BIG))
+        _check(lib().cbs_aes128_transcipher_slots(self._h, pc, ps, nblocks, po), "cbs_aes128_transcipher_slots")
+        return out
+
+    def ctr_transcipher_slots(self, ctr, ct, slots):
+        """CTR: ctr = the nblocks 16-byte counter blocks (each sender its own IV), ct = the AES-CTR ciphertext, block b under
+        slot slots[b] -> [nblocks][128][2049] plaintext bits."""
+        c, pc = _u8(ct)
+        nblocks = c.size // 16
+        k, pk = _u8(ctr)
+        if k.size != c.size:
+            raise ValueError(f"{k.size // 16} counter blocks for {nblocks} ciphertext blocks")
+        s, ps = _slots(slots, nblocks)
+        out, po = _out((nblocks, 128, LWE_BIG))
+        _check(lib().cbs_aes128_ctr_transcipher_slots(self._h, pk, pc, ps, nblocks, po), "cbs_aes128_ctr_transcipher_slots")
+        return out
 
     def ctr_transcipher_dev(self, d_ctr_ptr, d_ct_ptr, nblocks, d_out_ptr):
         """device-resident CTR transciphering: d_ctr = the public 16-byte counter blocks, d_ct = the AES-CTR ciphertext."""

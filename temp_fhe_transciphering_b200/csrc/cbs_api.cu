@@ -71,6 +71,15 @@ struct cbs_ctx {
     // [dir]: 0 = every mask word of the direction's middle and last LUTs is zero (always true for AllRdKeys written by the
     // reference, src/data_struct.rs:145-151,258-263); set by k_masks_nonzero at upload, enables the first-CMux shortcut
     int *d_masks_nonzero = nullptr;
+    // key slots per direction (cbs_trans_key_slots_reserve): `n` transciphering keys side by side, first [n][nmult][16][2],
+    // mid [n][8][nmult][16][2], last [n][16][2] GLWE (each slot in the single-key buffers' layout), flags[n] = that slot's
+    // k_masks_nonzero result; a slot is read only once `uploaded[slot]` is set
+    struct KeySlots {
+        uint64_t *first = nullptr, *mid = nullptr, *last = nullptr;
+        int *flags = nullptr;
+        int n = 0;
+        std::vector<bool> uploaded;
+    } slots[2];
     std::map<std::string, DevBuf> ws;
     int chunk_blocks = 64;
     // circuit bootstraps per sub-batch of a stage-8 LUT-circuit layer (bounds the Fourier GGSW workspace to 4.2 GB at
@@ -284,12 +293,21 @@ int job_tables(cbs_ctx *ctx, int nb, int nmult, int **lut, int **out)
 // server_encrypted_aes_decryption.rs:89-189): rounds 10 + 9 on the public ciphertext blocks d_in, rounds 8..1, the last
 // round and the per-byte bit reversal.  Forward (CTR, aes_he.rs:285-474): round 1 on the public counter blocks d_in,
 // rounds 2..9, the last round, then XOR with the public CTR ciphertext d_ct.
-int dev_aes_part(cbs_ctx *ctx, AesDir dir, const uint8_t *d_in, const uint8_t *d_ct, int nb, uint64_t *d_out)
+//
+// The key a call reads.  One key: the direction's buffers, flags = its device trivial-LUT flag, slots = nullptr.  Key slots: the
+// direction's slot pool, flags = its per-slot flags, slots = the device slot table of the blocks (in dev_aes_part: of the part's
+// first block); the part then builds its LUT index tables and its trivial-LUT flag on the device (k_slot_lut_index).
+struct AesKeyView {
+    const uint64_t *first, *mid, *last;
+    const int *flags;
+    const int *slots;
+};
+
+int dev_aes_part(cbs_ctx *ctx, AesDir dir, const AesKeyView &key, const uint8_t *d_in, const uint8_t *d_ct, int nb, uint64_t *d_out)
 {
     const int nmult = kAesDirs[dir].nmult, B = nb * 128;
     const bool inv = dir == kAesInv;
-    const cbs_ctx::AesKeys &key = ctx->aes[dir];
-    const int *masks_nonzero = ctx->d_masks_nonzero + dir;
+    const int *masks_nonzero = key.flags;
     uint64_t *d_t, *d_st, *d_ks;
     double *d_ggsw_f;
     int *lut_m, *out_m, *lut_1, *out_1;
@@ -299,9 +317,20 @@ int dev_aes_part(cbs_ctx *ctx, AesDir dir, const uint8_t *d_in, const uint8_t *d
     TRY(ws_typed(ctx, "ggsw_f", (size_t)B * kGgswWords, &d_ggsw_f));
     TRY(job_tables(ctx, nb, nmult, &lut_m, &out_m));
     TRY(job_tables(ctx, nb, 1, &lut_1, &out_1));
+    if (key.slots) {
+        // the out-index tables are the single key's; the LUT indices and the trivial-LUT flag follow the blocks' slots
+        int *flag;
+        TRY(ws_typed(ctx, "slot_lut_m", (size_t)nb * 16 * nmult * 2, &lut_m));
+        TRY(ws_typed(ctx, "slot_lut_1", (size_t)nb * 16 * 2, &lut_1));
+        TRY(ws_typed(ctx, "slot_flag", 1, &flag));
+        launch_slot_lut_index(key.slots, nb, nmult, key.flags, lut_m, lut_1, flag, S(ctx));
+        ctx->launches++;
+        TRY(check_launch("k_slot_lut_index"));
+        masks_nonzero = flag;
+    }
     auto linear = [&]() { inv ? launch_inv_linear(d_t, d_st, nb, S(ctx)) : launch_fwd_linear(d_t, d_st, nb, S(ctx)); };
     // first round(s): the input block is public, so the keyed LUTs are "rotated" by sample extraction
-    launch_known_rotate(d_in, key.first, d_t, nb, nmult, inv, S(ctx));
+    launch_known_rotate(d_in, key.first, d_t, nb, nmult, inv, key.slots, S(ctx));
     linear();
     ctx->launches += 2;
     TRY(check_launch("first rounds"));
@@ -347,21 +376,62 @@ int run_in_lanes(cbs_ctx *ctx, int nb, Fn part)
 }
 
 // nblocks blocks in chunks of chunk_blocks, each split into lanes; d_ct is nullptr for the inverse direction
-int dev_aes(cbs_ctx *ctx, AesDir dir, const uint8_t *d_in, const uint8_t *d_ct, int nblocks, uint64_t *d_out)
+int dev_aes(cbs_ctx *ctx, AesDir dir, const AesKeyView &key, const uint8_t *d_in, const uint8_t *d_ct, int nblocks, uint64_t *d_out)
 {
-    if (!ctx->aes[dir].uploaded) {
-        set_error(dir == kAesInv ? "transciphering key not uploaded (cbs_trans_key_upload)"
-                                 : "forward transciphering key not uploaded (cbs_fwd_trans_key_upload)");
-        return CBS_ERR_ARG;
-    }
     for (int c0 = 0; c0 < nblocks; c0 += ctx->chunk_blocks) {
         auto part = [&](int b0, int n) {
             const size_t b = (size_t)c0 + b0;
-            return dev_aes_part(ctx, dir, d_in + b * 16, d_ct ? d_ct + b * 16 : nullptr, n, d_out + b * 128 * kLweBig);
+            AesKeyView k = key;
+            if (k.slots) k.slots += b;
+            return dev_aes_part(ctx, dir, k, d_in + b * 16, d_ct ? d_ct + b * 16 : nullptr, n, d_out + b * 128 * kLweBig);
         };
         TRY(run_in_lanes(ctx, std::min(ctx->chunk_blocks, nblocks - c0), part));
     }
     return CBS_OK;
+}
+
+// dev_aes under the direction's single key (cbs_trans_key_upload and its twins)
+int dev_aes_single(cbs_ctx *ctx, AesDir dir, const uint8_t *d_in, const uint8_t *d_ct, int nblocks, uint64_t *d_out)
+{
+    const cbs_ctx::AesKeys &k = ctx->aes[dir];
+    if (!k.uploaded) {
+        set_error(dir == kAesInv ? "transciphering key not uploaded (cbs_trans_key_upload)"
+                                 : "forward transciphering key not uploaded (cbs_fwd_trans_key_upload)");
+        return CBS_ERR_ARG;
+    }
+    return dev_aes(ctx, dir, {k.first, k.mid, k.last, ctx->d_masks_nonzero + dir, nullptr}, d_in, d_ct, nblocks, d_out);
+}
+
+// Every block's slot must be reserved and uploaded in direction `dir`: checked on the host before anything is queued, so no
+// unchecked slot value reaches a kernel.  The checked table is returned in `table` for the device copy.
+int check_slots(const cbs_ctx *ctx, AesDir dir, const int32_t *slots, int nblocks, const char *what, std::vector<int> *table)
+{
+    const cbs_ctx::KeySlots &P = ctx->slots[dir];
+    table->resize(nblocks);
+    for (int b = 0; b < nblocks; b++) {
+        const int s = slots[b];
+        if (s < 0 || s >= P.n || !P.uploaded[s]) {
+            set_error(std::string(what) + ": block " + std::to_string(b) + " names slot " + std::to_string(s) +
+                      (s < 0 || s >= P.n ? ", outside the " + std::to_string(P.n) + " reserved slots" : ", which holds no key"));
+            return CBS_ERR_ARG;
+        }
+        (*table)[b] = s;
+    }
+    return CBS_OK;
+}
+
+// dev_aes under key slots: block b under slot slots[b] (host array).  The table goes to the device from a pageable host copy,
+// and cudaMemcpyAsync returns once pageable memory is staged, so the queued work reads no host memory after the return.
+int dev_aes_slots(cbs_ctx *ctx, AesDir dir, const uint8_t *d_in, const uint8_t *d_ct, const int32_t *slots, int nblocks,
+                  uint64_t *d_out, const char *what)
+{
+    std::vector<int> table;
+    TRY(check_slots(ctx, dir, slots, nblocks, what, &table));
+    int *d_slots;
+    TRY(ws_typed(ctx, "slot_table", (size_t)nblocks, &d_slots));
+    CUDA_TRY(cudaMemcpyAsync(d_slots, table.data(), sizeof(int) * nblocks, cudaMemcpyHostToDevice, ctx->stream));
+    const cbs_ctx::KeySlots &P = ctx->slots[dir];
+    return dev_aes(ctx, dir, {P.first, P.mid, P.last, P.flags, d_slots}, d_in, d_ct, nblocks, d_out);
 }
 
 // Uploads direction `dir`'s transciphering key and answers "are its middle and last LUTs trivial?" on the device, right behind
@@ -381,23 +451,40 @@ int aes_key_alloc(cbs_ctx *ctx, AesDir dir)
     return CBS_OK;
 }
 
-// the device flag of direction `dir`: 1 if a mask word of its middle or last LUTs is non-zero, queued on `cs`
-int aes_key_check_masks(cbs_ctx *ctx, AesDir dir, cudaStream_t cs)
+// Where an upload writes one key of direction `dir`: the direction's single-key buffers and flag, or one key slot's parts
+struct AesKeyDst {
+    uint64_t *first, *mid, *last;
+    int *flag;
+};
+
+AesKeyDst single_key_dst(cbs_ctx *ctx, AesDir dir)
+{
+    cbs_ctx::AesKeys &k = ctx->aes[dir];
+    return {k.first, k.mid, k.last, ctx->d_masks_nonzero + dir};
+}
+
+AesKeyDst slot_dst(cbs_ctx *ctx, AesDir dir, int slot)
 {
     const cbs_host::AesDirDesc &d = kAesDirs[dir];
-    const cbs_ctx::AesKeys &key = ctx->aes[dir];
-    int *flag = ctx->d_masks_nonzero + dir;
-    CUDA_TRY(cudaMemsetAsync(flag, 0, sizeof(int), cs));
-    launch_masks_nonzero(key.mid, 8 * d.nmult * 16 * 2, flag, cs);
-    launch_masks_nonzero(key.last, 16 * 2, flag, cs);
+    cbs_ctx::KeySlots &P = ctx->slots[dir];
+    return {P.first + (size_t)slot * d.first_words, P.mid + (size_t)slot * d.mid_words, P.last + (size_t)slot * d.last_words,
+            P.flags + slot};
+}
+
+// the key's device flag: 1 if a mask word of its middle or last LUTs is non-zero, queued on `cs`
+int aes_key_check_masks(AesDir dir, const AesKeyDst &key, cudaStream_t cs)
+{
+    const cbs_host::AesDirDesc &d = kAesDirs[dir];
+    CUDA_TRY(cudaMemsetAsync(key.flag, 0, sizeof(int), cs));
+    launch_masks_nonzero(key.mid, 8 * d.nmult * 16 * 2, key.flag, cs);
+    launch_masks_nonzero(key.last, 16 * 2, key.flag, cs);
     return CBS_OK;
 }
 
-int aes_key_upload(cbs_ctx *ctx, AesDir dir, const uint64_t *first, const uint64_t *mid, const uint64_t *last, bool overlap)
+int aes_key_write(cbs_ctx *ctx, AesDir dir, const AesKeyDst &key, const uint64_t *first, const uint64_t *mid, const uint64_t *last,
+                  bool overlap)
 {
     const cbs_host::AesDirDesc &d = kAesDirs[dir];
-    cbs_ctx::AesKeys &key = ctx->aes[dir];
-    TRY(aes_key_alloc(ctx, dir));
     cudaStream_t cs = ctx->stream;
     if (overlap) {
         if (!ctx->copy_stream) {
@@ -412,22 +499,27 @@ int aes_key_upload(cbs_ctx *ctx, AesDir dir, const uint64_t *first, const uint64
     }
     CUDA_TRY(cudaMemcpyAsync(key.mid, mid, (size_t)d.mid_words * 8, cudaMemcpyHostToDevice, cs));
     CUDA_TRY(cudaMemcpyAsync(key.last, last, (size_t)d.last_words * 8, cudaMemcpyHostToDevice, cs));
-    TRY(aes_key_check_masks(ctx, dir, cs));
+    TRY(aes_key_check_masks(dir, key, cs));
     if (overlap) CUDA_TRY(cudaEventRecord(ctx->ev_keys, cs));
     TRY(upload(ctx, key.first, first, (size_t)d.first_words * 8));
     if (!overlap) CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-    key.uploaded = true;
+    return CBS_OK;
+}
+
+int aes_key_upload(cbs_ctx *ctx, AesDir dir, const uint64_t *first, const uint64_t *mid, const uint64_t *last, bool overlap)
+{
+    TRY(aes_key_alloc(ctx, dir));
+    TRY(aes_key_write(ctx, dir, single_key_dst(ctx, dir), first, mid, last, overlap));
+    ctx->aes[dir].uploaded = true;
     return CBS_OK;
 }
 
 // Seeded key (include/cbs_b200.h) of direction `dir`: the bodies go into words 2048..3071 of every LUT GLWE (three strided
 // copies, one per key buffer), k_expand_lut_masks writes words 0..2047, and the same mask check as aes_key_upload follows (the
 // expanded masks are not zero, so the LUT ladders run their full first CMux).  On the compute stream, synchronised.
-int aes_key_seeded_upload(cbs_ctx *ctx, AesDir dir, const uint8_t mask_seed[32], const uint64_t *bodies)
+int aes_key_seeded_write(cbs_ctx *ctx, AesDir dir, const AesKeyDst &key, const uint8_t mask_seed[32], const uint64_t *bodies)
 {
     const cbs_host::AesDirDesc &d = kAesDirs[dir];
-    cbs_ctx::AesKeys &key = ctx->aes[dir];
-    TRY(aes_key_alloc(ctx, dir));
     uint64_t *const dst[3] = {key.first, key.mid, key.last};
     const uint32_t words[3] = {d.first_words, d.mid_words, d.last_words};
     const uint64_t *src = bodies;
@@ -442,9 +534,16 @@ int aes_key_seeded_upload(cbs_ctx *ctx, AesDir dir, const uint8_t mask_seed[32],
     launch_expand_lut_masks(seed, dir, nfirst, nglwe, key.first, key.mid, key.last, ctx->stream);
     ctx->launches++;
     TRY(check_launch("k_expand_lut_masks"));
-    TRY(aes_key_check_masks(ctx, dir, ctx->stream));
+    TRY(aes_key_check_masks(dir, key, ctx->stream));
     CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-    key.uploaded = true;
+    return CBS_OK;
+}
+
+int aes_key_seeded_upload(cbs_ctx *ctx, AesDir dir, const uint8_t mask_seed[32], const uint64_t *bodies)
+{
+    TRY(aes_key_alloc(ctx, dir));
+    TRY(aes_key_seeded_write(ctx, dir, single_key_dst(ctx, dir), mask_seed, bodies));
+    ctx->aes[dir].uploaded = true;
     return CBS_OK;
 }
 
@@ -463,12 +562,99 @@ int aes_transcipher_host(cbs_ctx *ctx, AesDir dir, const uint8_t *in, const uint
         TRY(ws_typed(ctx, "io_result", (size_t)nblocks * 128 * kLweBig, &d_out));
         TRY(upload(ctx, d_in, in, (size_t)nblocks * 16));
         if (ct) TRY(upload(ctx, d_ct, ct, (size_t)nblocks * 16));
-        return dev_aes(ctx, dir, d_in, d_ct, nblocks, d_out);
+        return dev_aes_single(ctx, dir, d_in, d_ct, nblocks, d_out);
     };
     const int rc = run();
     // whatever happened, the compute stream is ordered after the key copy before the call returns (host buffers, later calls)
     cudaStreamWaitEvent(ctx->stream, ctx->ev_keys, 0);
     ctx->keys_in_flight = false;
+    if (rc != CBS_OK) {
+        cudaStreamSynchronize(ctx->stream);
+        return rc;
+    }
+    return download(ctx, out, d_out, (size_t)nblocks * 128 * kLweBig * 8);
+}
+
+// ---- key slots (include/cbs_b200.h) ----
+
+// Grows direction `dir`'s pool to nslots slots: new buffers from the stream-ordered allocator, the uploaded slots copied over
+// device to device and the old buffers freed, all on the compute stream behind earlier work that may read them.  An allocation
+// failure frees what was allocated and leaves the old pool as it was.
+int key_slots_reserve(cbs_ctx *ctx, AesDir dir, int nslots, const char *what)
+{
+    cbs_ctx::KeySlots &P = ctx->slots[dir];
+    if (nslots <= 0 || nslots < P.n) {
+        set_error(std::string(what) + ": " + std::to_string(nslots) + " slots requested, " + std::to_string(P.n) +
+                  " reserved (a pool only grows)");
+        return CBS_ERR_ARG;
+    }
+    if (nslots == P.n) return CBS_OK;
+    const cbs_host::AesDirDesc &d = kAesDirs[dir];
+    const size_t slot_bytes[4] = {(size_t)d.first_words * 8, (size_t)d.mid_words * 8, (size_t)d.last_words * 8, sizeof(int)};
+    void **old[4] = {(void **)&P.first, (void **)&P.mid, (void **)&P.last, (void **)&P.flags};
+    void *grown[4] = {};
+    for (int i = 0; i < 4; i++) {
+        const cudaError_t e = cudaMallocAsync(&grown[i], slot_bytes[i] * nslots, ctx->stream);
+        if (e != cudaSuccess) {
+            cudaGetLastError();
+            for (int j = 0; j < i; j++) cudaFreeAsync(grown[j], ctx->stream);
+            set_error(std::string(what) + ": cannot allocate " + std::to_string(nslots) + " slots: " + cudaGetErrorString(e));
+            return CBS_ERR_NOMEM;
+        }
+    }
+    for (int i = 0; i < 4; i++) {
+        if (P.n) CUDA_TRY(cudaMemcpyAsync(grown[i], *old[i], slot_bytes[i] * P.n, cudaMemcpyDeviceToDevice, ctx->stream));
+        if (*old[i]) CUDA_TRY(cudaFreeAsync(*old[i], ctx->stream));
+        *old[i] = grown[i];
+    }
+    P.n = nslots;
+    P.uploaded.resize(nslots, false);
+    return CBS_OK;
+}
+
+// a slot upload replaces the slot's key: it is not readable until the upload has completed
+int key_slot_begin(cbs_ctx *ctx, AesDir dir, int slot, const char *what)
+{
+    cbs_ctx::KeySlots &P = ctx->slots[dir];
+    if (slot < 0 || slot >= P.n) {
+        set_error(std::string(what) + ": slot " + std::to_string(slot) + " outside the " + std::to_string(P.n) + " reserved slots");
+        return CBS_ERR_ARG;
+    }
+    P.uploaded[slot] = false;
+    return CBS_OK;
+}
+
+int key_slot_upload(cbs_ctx *ctx, AesDir dir, int slot, const uint64_t *first, const uint64_t *mid, const uint64_t *last,
+                    const char *what)
+{
+    TRY(key_slot_begin(ctx, dir, slot, what));
+    TRY(aes_key_write(ctx, dir, slot_dst(ctx, dir, slot), first, mid, last, false));
+    ctx->slots[dir].uploaded[slot] = true;
+    return CBS_OK;
+}
+
+int key_slot_seeded_upload(cbs_ctx *ctx, AesDir dir, int slot, const uint8_t mask_seed[32], const uint64_t *bodies, const char *what)
+{
+    TRY(key_slot_begin(ctx, dir, slot, what));
+    TRY(aes_key_seeded_write(ctx, dir, slot_dst(ctx, dir, slot), mask_seed, bodies));
+    ctx->slots[dir].uploaded[slot] = true;
+    return CBS_OK;
+}
+
+// Host-buffer transciphering under key slots: the inputs go up, dev_aes_slots runs, the rows come down.  Synchronous.
+int aes_transcipher_slots_host(cbs_ctx *ctx, AesDir dir, const uint8_t *in, const uint8_t *ct, const int32_t *slots, int nblocks,
+                               uint64_t *out, const char *what)
+{
+    std::vector<int> table;
+    TRY(check_slots(ctx, dir, slots, nblocks, what, &table));
+    uint8_t *d_in, *d_ct = nullptr;
+    uint64_t *d_out;
+    TRY(ws_typed(ctx, ct ? "io_ctr" : "io_ct", (size_t)nblocks * 16, &d_in));
+    if (ct) TRY(ws_typed(ctx, "io_ct", (size_t)nblocks * 16, &d_ct));
+    TRY(ws_typed(ctx, "io_result", (size_t)nblocks * 128 * kLweBig, &d_out));
+    TRY(upload(ctx, d_in, in, (size_t)nblocks * 16));
+    if (ct) TRY(upload(ctx, d_ct, ct, (size_t)nblocks * 16));
+    const int rc = dev_aes_slots(ctx, dir, d_in, d_ct, table.data(), nblocks, d_out, what);
     if (rc != CBS_OK) {
         cudaStreamSynchronize(ctx->stream);
         return rc;
@@ -674,6 +860,9 @@ void cbs_ctx_destroy(cbs_ctx *ctx)
     if (ctx->d_plan_luts) cudaFree(ctx->d_plan_luts);
     for (const cbs_ctx::AesKeys &key : ctx->aes)
         for (uint64_t *p : {key.first, key.mid, key.last})
+            if (p) cudaFree(p);
+    for (const cbs_ctx::KeySlots &P : ctx->slots)
+        for (void *p : {(void *)P.first, (void *)P.mid, (void *)P.last, (void *)P.flags})
             if (p) cudaFree(p);
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
     if (ctx->ev_keys) cudaEventDestroy(ctx->ev_keys);
@@ -927,7 +1116,7 @@ int cbs_aes_first_rounds(cbs_ctx *ctx, const uint8_t *ct, int nblocks, const uin
     TRY(ws_typed(ctx, "st", (size_t)nblocks * 128 * kLweBig, &d_st));
     TRY(upload(ctx, d_ct, ct, (size_t)nblocks * 16));
     TRY(upload(ctx, d_k, k10_9, (size_t)CBS_K10_9_WORDS * 8));
-    launch_known_rotate(d_ct, d_k, d_t4, nblocks, 4, 1, ctx->stream);
+    launch_known_rotate(d_ct, d_k, d_t4, nblocks, 4, 1, nullptr, ctx->stream);
     launch_inv_linear(d_t4, d_st, nblocks, ctx->stream);
     ctx->launches += 2;
     TRY(check_launch("first rounds"));
@@ -960,7 +1149,7 @@ int cbs_aes128_transcipher_dev(cbs_ctx *ctx, const uint8_t *d_ct, int nblocks, u
 {
     ENTER(ctx);
     if (nblocks <= 0 || !d_ct || !d_out) return set_error("cbs_aes128_transcipher_dev: bad argument"), CBS_ERR_ARG;
-    return dev_aes(ctx, kAesInv, d_ct, nullptr, nblocks, d_out);
+    return dev_aes_single(ctx, kAesInv, d_ct, nullptr, nblocks, d_out);
 }
 
 int cbs_aes128_transcipher(cbs_ctx *ctx, const uint8_t *ct, int nblocks, const uint64_t *k10_9, const uint64_t *k8_1,
@@ -997,7 +1186,7 @@ int cbs_aes128_ctr_transcipher_dev(cbs_ctx *ctx, const uint8_t *d_ctr, const uin
 {
     ENTER(ctx);
     if (nblocks <= 0 || !d_ctr || !d_ct || !d_out) return set_error("cbs_aes128_ctr_transcipher_dev: bad argument"), CBS_ERR_ARG;
-    return dev_aes(ctx, kAesFwd, d_ctr, d_ct, nblocks, d_out);
+    return dev_aes_single(ctx, kAesFwd, d_ctr, d_ct, nblocks, d_out);
 }
 
 int cbs_aes128_ctr_transcipher(cbs_ctx *ctx, const uint8_t *ct, int nblocks, const uint8_t iv[16], const uint64_t *kf_first,
@@ -1017,6 +1206,77 @@ int cbs_aes128_ctr_transcipher(cbs_ctx *ctx, const uint8_t *ct, int nblocks, con
             if (++cur[i] != 0) break;
     }
     return aes_transcipher_host(ctx, kAesFwd, ctr.data(), ct, nblocks, kf_first, kf_mid, kf_last, out);
+}
+
+int cbs_trans_key_slots_reserve(cbs_ctx *ctx, int nslots)
+{
+    ENTER(ctx);
+    return key_slots_reserve(ctx, kAesInv, nslots, "cbs_trans_key_slots_reserve");
+}
+
+int cbs_fwd_trans_key_slots_reserve(cbs_ctx *ctx, int nslots)
+{
+    ENTER(ctx);
+    return key_slots_reserve(ctx, kAesFwd, nslots, "cbs_fwd_trans_key_slots_reserve");
+}
+
+int cbs_trans_key_slot_upload(cbs_ctx *ctx, int slot, const uint64_t *k10_9, const uint64_t *k8_1, const uint64_t *k0)
+{
+    ENTER(ctx);
+    if (!k10_9 || !k8_1 || !k0) return set_error("cbs_trans_key_slot_upload: null argument"), CBS_ERR_ARG;
+    return key_slot_upload(ctx, kAesInv, slot, k10_9, k8_1, k0, "cbs_trans_key_slot_upload");
+}
+
+int cbs_fwd_trans_key_slot_upload(cbs_ctx *ctx, int slot, const uint64_t *kf_first, const uint64_t *kf_mid, const uint64_t *kf_last)
+{
+    ENTER(ctx);
+    if (!kf_first || !kf_mid || !kf_last) return set_error("cbs_fwd_trans_key_slot_upload: null argument"), CBS_ERR_ARG;
+    return key_slot_upload(ctx, kAesFwd, slot, kf_first, kf_mid, kf_last, "cbs_fwd_trans_key_slot_upload");
+}
+
+int cbs_trans_key_seeded_slot_upload(cbs_ctx *ctx, int slot, const uint8_t mask_seed[32], const uint64_t *bodies)
+{
+    ENTER(ctx);
+    if (!mask_seed || !bodies) return set_error("cbs_trans_key_seeded_slot_upload: null argument"), CBS_ERR_ARG;
+    return key_slot_seeded_upload(ctx, kAesInv, slot, mask_seed, bodies, "cbs_trans_key_seeded_slot_upload");
+}
+
+int cbs_fwd_trans_key_seeded_slot_upload(cbs_ctx *ctx, int slot, const uint8_t mask_seed[32], const uint64_t *bodies)
+{
+    ENTER(ctx);
+    if (!mask_seed || !bodies) return set_error("cbs_fwd_trans_key_seeded_slot_upload: null argument"), CBS_ERR_ARG;
+    return key_slot_seeded_upload(ctx, kAesFwd, slot, mask_seed, bodies, "cbs_fwd_trans_key_seeded_slot_upload");
+}
+
+int cbs_aes128_transcipher_slots_dev(cbs_ctx *ctx, const uint8_t *d_ct, const int32_t *slots, int nblocks, uint64_t *d_out)
+{
+    ENTER(ctx);
+    if (nblocks <= 0 || !d_ct || !slots || !d_out) return set_error("cbs_aes128_transcipher_slots_dev: bad argument"), CBS_ERR_ARG;
+    return dev_aes_slots(ctx, kAesInv, d_ct, nullptr, slots, nblocks, d_out, "cbs_aes128_transcipher_slots_dev");
+}
+
+int cbs_aes128_ctr_transcipher_slots_dev(cbs_ctx *ctx, const uint8_t *d_ctr, const uint8_t *d_ct, const int32_t *slots, int nblocks,
+                                         uint64_t *d_out)
+{
+    ENTER(ctx);
+    if (nblocks <= 0 || !d_ctr || !d_ct || !slots || !d_out)
+        return set_error("cbs_aes128_ctr_transcipher_slots_dev: bad argument"), CBS_ERR_ARG;
+    return dev_aes_slots(ctx, kAesFwd, d_ctr, d_ct, slots, nblocks, d_out, "cbs_aes128_ctr_transcipher_slots_dev");
+}
+
+int cbs_aes128_transcipher_slots(cbs_ctx *ctx, const uint8_t *ct, const int32_t *slots, int nblocks, uint64_t *out)
+{
+    ENTER(ctx);
+    if (nblocks <= 0 || !ct || !slots || !out) return set_error("cbs_aes128_transcipher_slots: bad argument"), CBS_ERR_ARG;
+    return aes_transcipher_slots_host(ctx, kAesInv, ct, nullptr, slots, nblocks, out, "cbs_aes128_transcipher_slots");
+}
+
+int cbs_aes128_ctr_transcipher_slots(cbs_ctx *ctx, const uint8_t *ctr, const uint8_t *ct, const int32_t *slots, int nblocks,
+                                     uint64_t *out)
+{
+    ENTER(ctx);
+    if (nblocks <= 0 || !ctr || !ct || !slots || !out) return set_error("cbs_aes128_ctr_transcipher_slots: bad argument"), CBS_ERR_ARG;
+    return aes_transcipher_slots_host(ctx, kAesFwd, ctr, ct, slots, nblocks, out, "cbs_aes128_ctr_transcipher_slots");
 }
 
 }  // extern "C"

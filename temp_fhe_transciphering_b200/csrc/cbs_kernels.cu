@@ -2237,8 +2237,9 @@ int launch_lut8(const DeviceKeys &K, const double *ggsw_f, const uint64_t *luts,
 // a8: known_rotate_keyed_lut, cbs_lib/src/aes_he.rs:64-93 (rounds 10 + 9: the AES ciphertext byte is
 // public, so the keyed LUT is "rotated" by plain sample extraction at lut_idx*256 + byte).
 // t4 layout [4 mult][nblocks][128][2049]; k10_9 layout [4][16][2][3072]; ct = raw AES ciphertext bytes.
+// slot != nullptr: luts is a key-slot pool [S][nmult][16][2] and block blk reads slot slot[blk].
 __global__ void k_known_rotate(const uint8_t *__restrict__ ct, const uint64_t *__restrict__ luts,
-                               uint64_t *__restrict__ tm, int nblocks, int inv_shift)
+                               uint64_t *__restrict__ tm, int nblocks, int inv_shift, const int *__restrict__ slot)
 {
     const int lweid = blockIdx.x;  // (m, blk, i)
     const int i = lweid % 128, blk = (lweid / 128) % nblocks, m = lweid / (128 * nblocks);
@@ -2248,6 +2249,7 @@ __global__ void k_known_rotate(const uint8_t *__restrict__ ct, const uint64_t *_
     const int row = byte & 3, col = byte >> 2;
     const int src = inv_shift ? 4 * ((col - row + 4) & 3) + row : byte;
     const int T = (bit & 3) * 256 + ct[blk * 16 + src];
+    if (slot) luts += (size_t)slot[blk] * (gridDim.x / (128 * nblocks)) * 32 * kGlweWords;
     const uint64_t *glwe = luts + (size_t)((m * 16 + byte) * 2 + (bit >> 2)) * kGlweWords;
     uint64_t *o = tm + (size_t)lweid * kLweBig;
     for (int w = threadIdx.x; w < 2048; w += blockDim.x) {
@@ -2259,10 +2261,42 @@ __global__ void k_known_rotate(const uint8_t *__restrict__ ct, const uint64_t *_
 }
 
 void launch_known_rotate(const uint8_t *ct, const uint64_t *luts, uint64_t *tm, int nblocks, int nmult, int inv_shift,
-                         cudaStream_t s)
+                         const int *slot, cudaStream_t s)
 {
     if (nblocks <= 0) return;
-    k_known_rotate<<<nmult * nblocks * 128, 256, 0, s>>>(ct, luts, tm, nblocks, inv_shift);
+    k_known_rotate<<<nmult * nblocks * 128, 256, 0, s>>>(ct, luts, tm, nblocks, inv_shift, slot);
+}
+
+// Key-slot LUT index tables of one lane part of nb blocks (block b under slot slot[b] of a pool [S][...]): the middle rounds'
+// job (blk, byte, m, a) -> slot * 8 nmult 32 + (m 16 + byte) 2 + a (GLWE from the round's base in mid [S][8][nmult][16][2]),
+// the last round's job (blk, byte, a) -> slot * 32 + byte 2 + a, in the job order of the single-key tables; CTA 0 also writes
+// *flag = OR of slot_flags[slot[b]] (non-zero: some block's LUTs have a non-zero mask, so no block takes the first-CMux
+// shortcut of trivial LUTs).
+__global__ void __launch_bounds__(256) k_slot_lut_index(const int *__restrict__ slot, int nb, int nmult,
+                                                        const int *__restrict__ slot_flags, int *__restrict__ lut_mid,
+                                                        int *__restrict__ lut_last, int *__restrict__ flag)
+{
+    const int n = nb * 16 * nmult * 2;
+    for (int job = blockIdx.x * blockDim.x + threadIdx.x; job < n; job += gridDim.x * blockDim.x) {
+        const int a = job & 1, m = (job >> 1) % nmult, bb = job / (2 * nmult);  // bb = blk * 16 + byte
+        const int s = slot[bb >> 4], byte = bb & 15;
+        lut_mid[job] = s * 8 * nmult * 32 + (m * 16 + byte) * 2 + a;
+        if (m == 0) lut_last[bb * 2 + a] = s * 32 + byte * 2 + a;
+    }
+    if (blockIdx.x == 0) {
+        int any = 0;
+        for (int b = threadIdx.x; b < nb; b += blockDim.x) any |= slot_flags[slot[b]];
+        any = __syncthreads_or(any != 0);
+        if (threadIdx.x == 0) *flag = any != 0;
+    }
+}
+
+void launch_slot_lut_index(const int *slot, int nb, int nmult, const int *slot_flags, int *lut_mid, int *lut_last, int *flag,
+                           cudaStream_t s)
+{
+    if (nb <= 0) return;
+    const int n = nb * 16 * nmult * 2, blocks = (n + 255) / 256;
+    k_slot_lut_index<<<blocks < 148 ? blocks : 148, 256, 0, s>>>(slot, nb, nmult, slot_flags, lut_mid, lut_last, flag);
 }
 
 // forward linear layer: he_shift_rows (cbs_lib/src/aes_he.rs:348-366) on the x1, x2, x3 lists followed by

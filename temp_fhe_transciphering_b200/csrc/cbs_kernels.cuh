@@ -92,9 +92,16 @@ void launch_lwe_add_rows(uint64_t *pool, const int *triples, int count, cudaStre
 void launch_glev_to_lwe(const uint64_t *glev, const int *pairs, uint64_t *pool, int count, cudaStream_t s);
 
 // a8  rounds 10+9: sample extraction from the encrypted keyed LUTs (ct = raw AES ciphertext bytes; the cleartext inv_shift_rows is applied inside)
-//     luts = [nmult][16][2] GLWE, tm = [nmult][nblocks][128][2049]; inv_shift = 1 for the inverse direction
+//     luts = [nmult][16][2] GLWE, tm = [nmult][nblocks][128][2049]; inv_shift = 1 for the inverse direction.
+//     slot = nullptr: one key; else a device [nblocks] slot table, luts a key-slot pool [S][nmult][16][2] and block b reads
+//     the LUTs of slot slot[b]
 void launch_known_rotate(const uint8_t *ct, const uint64_t *luts, uint64_t *tm, int nblocks, int nmult, int inv_shift,
-                         cudaStream_t s);
+                         const int *slot, cudaStream_t s);
+// key-slot LUT index tables of nb blocks under slots slot[nb] (device): lut_mid[nb*16*nmult*2] for the middle rounds (GLWE
+//     indices into mid + round * nmult*32 of a pool mid [S][8][nmult][16][2]), lut_last[nb*16*2] into last [S][16][2], both in
+//     the job order of the single-key tables; *flag = OR of slot_flags[slot[b]] (the k_lut8_v2 trivial-LUT flag of the blocks)
+void launch_slot_lut_index(const int *slot, int nb, int nmult, const int *slot_flags, int *lut_mid, int *lut_last, int *flag,
+                           cudaStream_t s);
 // forward direction (CTR): ShiftRows + MixColumns-precomp over t3 = [3 (x1,x2,x3)][nblocks][128][2049]
 void launch_fwd_linear(const uint64_t *t3, uint64_t *st, int nblocks, cudaStream_t s);
 // last-round ShiftRows permutation + XOR with the public ciphertext bits + MSB-first order
