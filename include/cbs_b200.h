@@ -213,6 +213,21 @@ int cbs_circuit_bootstrap(cbs_ctx *ctx, const uint64_t *in_small, uint64_t *ggsw
  * bits (LSB first), nluts LUTs per byte, each LUT = 2 GLWE accumulators;
  * out[nbytes][nluts][8] big LWE, bit 4*a + t of accumulator a. */
 int cbs_lut8_eval(cbs_ctx *ctx, const uint64_t *ggsw_bits, int nbytes, const uint64_t *luts, int nluts, uint64_t *out);
+/* max_of_two, src/bin/server_encrypted_compute.rs:34-98: the CMux ladder of one tree level of cbs_max_u16, on given inputs.
+ * ggsw[nvals][16] standard-domain GGSW of the values' bits (MSB first), op[nvals][16] GLWE data operands (cbs_max_u16 takes
+ * them from the bootstraps' level-1 GLEV, doubled); pair p = (a_idx[p], b_idx[p]) -> out[npairs][16] big LWE, output bit j
+ * of pair p computed with e starting from operand a's bit j (DESIGN.md section 4a).  npairs = 0 returns CBS_OK; negative
+ * counts, null pointers and a pair index outside [0, nvals) return CBS_ERR_ARG before anything is queued. */
+int cbs_max_of_two(cbs_ctx *ctx, const uint64_t *ggsw, const uint64_t *op, int nvals, const int32_t *a_idx, const int32_t *b_idx,
+                   int npairs, uint64_t *out);
+/* The gathered LUT ladder of the stage-8 LUT circuits (csrc/host/ip_plan.h) on given inputs.  ggsw[nbits] standard-domain
+ * GGSW; job j runs the accumulator luts[lut_index[j]] (luts[nluts] GLWE) through the selectors sel[j][0..7] (selector i
+ * rotates by 2^i; -1 = the constant-0 selector, its CMux is skipped) and writes the 4 extractions at 0, 256, 512, 768 to rows
+ * out_index[j] .. out_index[j] + 3 of out[nout] big LWE; every other row of out is zero.  njobs = 0 returns CBS_OK; negative
+ * counts, null pointers, a selector outside [-1, nbits), a lut_index outside [0, nluts) and an output window outside
+ * [0, nout) or overlapping another job's return CBS_ERR_ARG before anything is queued. */
+int cbs_lut8_gather_eval(cbs_ctx *ctx, const uint64_t *ggsw, int nbits, const int32_t *sel, const uint64_t *luts, int nluts,
+                         const int32_t *lut_index, const int32_t *out_index, int njobs, uint64_t *out, int nout);
 /* known_rotate_keyed_lut x4 + he_inv_mix_columns_precomp + he_inv_shift_rows
  * (cbs_lib/src/aes_he.rs:64, server_encrypted_aes_decryption.rs:89-128): first two rounds */
 int cbs_aes_first_rounds(cbs_ctx *ctx, const uint8_t *ct, int nblocks, const uint64_t *k10_9, uint64_t *state_out);

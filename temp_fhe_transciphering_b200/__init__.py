@@ -113,6 +113,11 @@ def _u8(b):
     return a, a.ctypes.data_as(ctypes.POINTER(ctypes.c_uint8))
 
 
+def _i32(a):
+    a = np.ascontiguousarray(a, dtype=np.int32).reshape(-1)
+    return a, a.ctypes.data_as(ctypes.POINTER(ctypes.c_int32))
+
+
 def _slots(slots, nblocks):
     a = np.ascontiguousarray(slots, dtype=np.int32).reshape(-1)
     if a.size != nblocks:
@@ -481,6 +486,32 @@ class Context:
         nluts = l.shape[1]
         out, po = _out((nbytes, nluts, 8, LWE_BIG))
         _check(lib().cbs_lut8_eval(self._h, pg, nbytes, pl, nluts, po), "cbs_lut8_eval")
+        return out
+
+    def max_of_two(self, ggsw, op, a_idx, b_idx):
+        """max_of_two, src/bin/server_encrypted_compute.rs:34-98, one ladder per pair (a_idx[p], b_idx[p]): ggsw
+        [nvals][16][GGSW] (standard domain, MSB first), op [nvals][16][GLWE] data operands -> [npairs][16][2049]."""
+        g, pg = _u64(np.reshape(ggsw, (-1, 16, GGSW_WORDS)))
+        o, po = _u64(np.reshape(op, (g.shape[0], 16, GLWE_WORDS)))
+        (a, pa), (b, pb) = _i32(a_idx), _i32(b_idx)
+        if a.size != b.size:
+            raise ValueError(f"{a.size} a indices for {b.size} b indices")
+        out, pout = _out((a.size, 16, LWE_BIG))
+        _check(lib().cbs_max_of_two(self._h, pg, po, g.shape[0], pa, pb, a.size, pout), "cbs_max_of_two")
+        return out
+
+    def evaluate_gathered_luts(self, ggsw, sel, luts, lut_index, out_index, nout):
+        """the gathered LUT ladder of the stage-8 circuits: ggsw [nbits][GGSW], sel [njobs][8] (-1: constant-0 selector),
+        luts [nluts][GLWE] -> out [nout][2049]; job j writes rows out_index[j] .. + 3, the other rows are zero."""
+        g, pg = _u64(np.reshape(ggsw, (-1, GGSW_WORDS)))
+        l, pl = _u64(np.reshape(luts, (-1, GLWE_WORDS)))
+        s, ps = _i32(sel)
+        (li, pli), (oi, poi) = _i32(lut_index), _i32(out_index)
+        if s.size != 8 * li.size or oi.size != li.size:
+            raise ValueError(f"sel of {s.size} entries, {li.size} LUT indices and {oi.size} output indices")
+        out, pout = _out((nout, LWE_BIG))
+        _check(lib().cbs_lut8_gather_eval(self._h, pg, g.shape[0], ps, pl, l.shape[0], pli, poi, li.size, pout, int(nout)),
+               "cbs_lut8_gather_eval")
         return out
 
     def aes_first_rounds(self, ct, k10_9):

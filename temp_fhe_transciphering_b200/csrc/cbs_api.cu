@@ -10,6 +10,7 @@
 #include "fft_tables.h"
 #include "host/host_common.h"
 
+#include <algorithm>
 #include <climits>
 #include <cmath>
 #include <cstdio>
@@ -1101,6 +1102,87 @@ int cbs_lut8_eval(cbs_ctx *ctx, const uint64_t *ggsw_bits, int nbytes, const uin
     ctx->launches++;
     TRY(dev_lut8(ctx, d_ggsw_f, d_luts, d_li, d_oi, d_out, njobs, apb, nullptr));
     return download(ctx, out, d_out, (size_t)njobs * 4 * kLweBig * 8);
+}
+
+int cbs_max_of_two(cbs_ctx *ctx, const uint64_t *ggsw, const uint64_t *op, int nvals, const int32_t *a_idx, const int32_t *b_idx,
+                   int npairs, uint64_t *out)
+{
+    ENTER(ctx);
+    // counts bounded so that nvals * 16 * 63 Fourier polynomials and npairs * 16 groups stay ints
+    bool ok = nvals >= 0 && npairs >= 0 && nvals <= (INT_MAX >> 10) && npairs <= (INT_MAX >> 5) &&
+              (!npairs || (ggsw && op && a_idx && b_idx && out));
+    for (int p = 0; ok && p < npairs; p++) ok = a_idx[p] >= 0 && a_idx[p] < nvals && b_idx[p] >= 0 && b_idx[p] < nvals;
+    if (!ok) return set_error("cbs_max_of_two: bad argument (negative count, null pointer or pair index outside [0, nvals))"), CBS_ERR_ARG;
+    if (!npairs) return CBS_OK;
+    const int nbits = nvals * 16;
+    uint64_t *d_ggsw, *d_op, *d_out;
+    double *d_ggsw_f;
+    int *d_a, *d_b;
+    TRY(ws_typed(ctx, "ggsw_std", (size_t)nbits * kGgswWords, &d_ggsw));
+    TRY(ws_typed(ctx, "ggsw_f", (size_t)nbits * kGgswWords, &d_ggsw_f));
+    TRY(ws_typed(ctx, "io_luts", (size_t)nbits * kGlweWords, &d_op));
+    TRY(ws_typed(ctx, "io_out", (size_t)npairs * 16 * kLweBig, &d_out));
+    TRY(ws_typed(ctx, "io_li", (size_t)npairs, &d_a));
+    TRY(ws_typed(ctx, "io_oi", (size_t)npairs, &d_b));
+    TRY(upload(ctx, d_ggsw, ggsw, (size_t)nbits * kGgswWords * 8));
+    TRY(upload(ctx, d_op, op, (size_t)nbits * kGlweWords * 8));
+    TRY(upload(ctx, d_a, a_idx, sizeof(int) * npairs));
+    TRY(upload(ctx, d_b, b_idx, sizeof(int) * npairs));
+    launch_ggsw_to_fourier(ctx->K, d_ggsw, d_ggsw_f, nbits, ctx->stream);
+    ctx->launches++;
+    launch_max_ladder(ctx->K, d_ggsw_f, d_op, d_a, d_b, d_out, npairs, ctx->stream);
+    ctx->launches++;
+    TRY(check_launch("k_max_ladder"));
+    return download(ctx, out, d_out, (size_t)npairs * 16 * kLweBig * 8);
+}
+
+int cbs_lut8_gather_eval(cbs_ctx *ctx, const uint64_t *ggsw, int nbits, const int32_t *sel, const uint64_t *luts, int nluts,
+                         const int32_t *lut_index, const int32_t *out_index, int njobs, uint64_t *out, int nout)
+{
+    ENTER(ctx);
+    bool ok = nbits >= 0 && nluts >= 0 && njobs >= 0 && nout >= 0 && nbits <= (INT_MAX >> 10) && njobs <= (INT_MAX >> 3) &&
+              (!njobs || (sel && luts && lut_index && out_index && out && (ggsw || !nbits)));
+    // output windows [out_index, out_index + 4) inside [0, nout) and pairwise disjoint
+    std::vector<int> starts;
+    starts.reserve(ok ? (size_t)njobs : 0);
+    for (int j = 0; ok && j < njobs; j++) {
+        for (int i = 0; ok && i < 8; i++) ok = sel[(size_t)j * 8 + i] >= -1 && sel[(size_t)j * 8 + i] < nbits;
+        ok = ok && lut_index[j] >= 0 && lut_index[j] < nluts && out_index[j] >= 0 && out_index[j] <= nout - 4;
+        starts.push_back(out_index[j]);
+    }
+    std::sort(starts.begin(), starts.end());
+    for (size_t j = 1; ok && j < starts.size(); j++) ok = starts[j] - starts[j - 1] >= 4;
+    if (!ok)
+        return set_error("cbs_lut8_gather_eval: bad argument (negative count, null pointer, selector outside [-1, nbits), "
+                         "LUT index outside [0, nluts), or an output window outside [0, nout) or overlapping another)"),
+               CBS_ERR_ARG;
+    if (!njobs) return CBS_OK;
+    uint64_t *d_ggsw = nullptr, *d_luts, *d_out;
+    double *d_ggsw_f = nullptr;
+    int *d_sel, *d_li, *d_oi;
+    TRY(ws_typed(ctx, "io_luts", (size_t)nluts * kGlweWords, &d_luts));
+    TRY(ws_typed(ctx, "io_out", (size_t)nout * kLweBig, &d_out));
+    TRY(ws_typed(ctx, "io_sel", (size_t)njobs * 8, &d_sel));
+    TRY(ws_typed(ctx, "io_li", (size_t)njobs, &d_li));
+    TRY(ws_typed(ctx, "io_oi", (size_t)njobs, &d_oi));
+    if (nbits) {
+        TRY(ws_typed(ctx, "ggsw_std", (size_t)nbits * kGgswWords, &d_ggsw));
+        TRY(ws_typed(ctx, "ggsw_f", (size_t)nbits * kGgswWords, &d_ggsw_f));
+        TRY(upload(ctx, d_ggsw, ggsw, (size_t)nbits * kGgswWords * 8));
+    }
+    TRY(upload(ctx, d_luts, luts, (size_t)nluts * kGlweWords * 8));
+    TRY(upload(ctx, d_sel, sel, sizeof(int) * njobs * 8));
+    TRY(upload(ctx, d_li, lut_index, sizeof(int) * njobs));
+    TRY(upload(ctx, d_oi, out_index, sizeof(int) * njobs));
+    CUDA_TRY(cudaMemsetAsync(d_out, 0, (size_t)nout * kLweBig * 8, ctx->stream));
+    if (nbits) {
+        launch_ggsw_to_fourier(ctx->K, d_ggsw, d_ggsw_f, nbits, ctx->stream);
+        ctx->launches++;
+    }
+    launch_lut8_gather(ctx->K, d_ggsw_f, d_sel, d_luts, d_li, d_oi, d_out, njobs, ctx->stream);
+    ctx->launches++;
+    TRY(check_launch("k_lut8_gather"));
+    return download(ctx, out, d_out, (size_t)nout * kLweBig * 8);
 }
 
 int cbs_aes_first_rounds(cbs_ctx *ctx, const uint8_t *ct, int nblocks, const uint64_t *k10_9, uint64_t *state_out)
